@@ -1,6 +1,7 @@
 """bench.py -- the contract benchmark of the temporal MSDeformAttn hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dtype fp32|bf16] [--dist local|uniform]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One STEP = one encoder-layer temporal attention over one clip, forward + backward, at the DeVIS R50 T=6
@@ -25,6 +26,10 @@ Rank 0 prints ONE JSON line:
   also.train_trunk  (every N) trunk training step: fwd + bwd + DDP NCCL gradient all-reduce + clip + AdamW
 Multi-GPU: clips are independent, so each rank works on its own clip (weak scaling, no collective on
 the op path -- SURVEY.md section 8e).
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step returned to its caller: the output and the
+five input gradients, as DIR/<name>.npy (float32; rank 0's clip).  The inputs are seeded, so two builds run with the same
+arguments can be compared output for output; see dump_outputs for the sampling that keeps the files under 64 MB.
 
 `--impl reference` times the reference's CPU implementation of the same unit of work (the oracle's
 PyTorch restatement of ms_deform_attn_core_pytorch + autograd, all host threads): W warm-up and K timed WHOLE
@@ -177,6 +182,26 @@ def ncu_summary(kernel_key, field="dram_bytes_per_launch"):
             return json.load(fh)[kernel_key][field]
     except Exception:
         return None
+
+
+DUMP_MAX_ELEMS = 1 << 21        # per array: the six arrays of a step stay under 64 MB in float32
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every tensor of `arrays` as out_dir/<name>.npy, float64 kept, anything else as float32.  A tensor of more than
+    DUMP_MAX_ELEMS elements is replaced by DUMP_MAX_ELEMS of them, flattened: the flat indices are drawn without replacement
+    from a generator seeded with 0 and sorted, so they depend only on the tensor's size and every run and every build
+    writes the same elements."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, x in arrays.items():
+        x = x.detach()
+        if x.numel() > DUMP_MAX_ELEMS:
+            idx = np.sort(np.random.default_rng(0).choice(x.numel(), DUMP_MAX_ELEMS, replace=False))
+            x = x.reshape(-1)[torch.from_numpy(idx).to(x.device)]
+        x = x.cpu()
+        np.save(os.path.join(out_dir, name + ".npy"), (x.double() if x.dtype == torch.float64 else x.float()).numpy())
 
 
 # ----------------------------------------------------------------------------------------------------
@@ -622,10 +647,12 @@ def run_ours(args, rank, world, local_rank):
     t_region0 = time.perf_counter()
     e0.record()
     for _ in range(args.steps):
-        step()
+        out = step()
     e1.record()
     barrier()
     sampler.window = (t_region0, time.perf_counter())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"out": out, **{"grad_" + k: x.grad for k, x in zip(CLIP_NAMES, leaves)}})
     ms_total = reduce_max(e0.elapsed_time(e1))
     launches = _lib.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
@@ -931,7 +958,13 @@ def main():
                     help="--impl reference: stop timing after this many seconds of wall clock (steps reported honestly)")
     ap.add_argument("--bf16-accumulate", action="store_true",
                     help="with --dtype bf16: accumulate grad_value in bf16 (DEVIS_MSDA_FLAG_BF16_GRAD_VALUE, opt-in)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the output and the input gradients of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed; it does not apply to --impl reference")
     rank, world, local_rank = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
     if args.impl == "reference":
         run_reference(args, rank)

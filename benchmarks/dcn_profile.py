@@ -1,5 +1,5 @@
-import sys, torch
-sys.path.insert(0, "/root/repo")
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from devis_b200.deform_conv import deform_conv2d
 from torch.profiler import ProfilerActivity, profile
 torch.backends.cuda.matmul.allow_tf32 = False

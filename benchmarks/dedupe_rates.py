@@ -1,5 +1,5 @@
-import sys, torch, numpy as np
-sys.path.insert(0,'/root/repo')
+import os, sys, torch, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from devis_b200 import synthetic, clip_geometry
 torch.manual_seed(0)
 def analyse(sigma, label, frames=(2,), heads=(0,3)):

@@ -1,5 +1,5 @@
-import json, sys, statistics, torch
-sys.path.insert(0, '/root/repo')
+import json, os, sys, statistics, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from devis_b200 import TemporalMSDeformAttnEncoder, synthetic, clip_geometry, MultiScaleDeformableAttention as MSDA
 torch.manual_seed(0)
 T, C = 6, 256

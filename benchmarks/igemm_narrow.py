@@ -1,5 +1,6 @@
-import sys, json, statistics, torch
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tests')
+import os, sys, json, statistics, torch
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tests'))
 from conftest import nmax
 from devis_b200 import _lib, deform_conv
 from devis_b200.deform_conv import IGemmDeformConv2dFunction, deform_conv2d

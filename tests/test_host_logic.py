@@ -228,6 +228,25 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert "workload" in line["config"] and "model" not in line["config"]
 
 
+def test_bench_dump_outputs_writes_a_fixed_bounded_sample(tmp_path):
+    """`bench.py --dump-outputs`: small arrays whole (float64 kept, bf16 widened), large ones as the same seeded sample of
+    flat indices in every run, the six arrays of the bench step under 64 MB in all"""
+    import bench
+    n = bench.DUMP_MAX_ELEMS + 1000
+    big = torch.arange(n, dtype=torch.float32)
+    arrays = {"big": big, "f64": torch.randn(3, 4, dtype=torch.float64), "bf16": torch.randn(5).bfloat16()}
+    bench.dump_outputs(str(tmp_path / "a"), arrays)
+    bench.dump_outputs(str(tmp_path / "b"), {"big": big * 2, **{k: v for k, v in arrays.items() if k != "big"}})
+    a, b = np.load(tmp_path / "a" / "big.npy"), np.load(tmp_path / "b" / "big.npy")
+    assert a.dtype == np.float32 and a.shape == (bench.DUMP_MAX_ELEMS,)
+    assert np.all(np.diff(a) > 0) and a[-1] < n and np.array_equal(b, 2 * a)     # distinct sorted indices, same each run
+    f64 = np.load(tmp_path / "a" / "f64.npy")
+    assert f64.dtype == np.float64 and np.array_equal(f64, arrays["f64"].numpy())
+    bf = np.load(tmp_path / "a" / "bf16.npy")
+    assert bf.dtype == np.float32 and np.array_equal(bf, arrays["bf16"].float().numpy())
+    assert 6 * bench.DUMP_MAX_ELEMS * 4 < 64e6
+
+
 def test_weight_gradient_split_rows_equals_one_gemm():
     """deform_conv._wgrad: the batched split-row product (taken for narrow layers with 10^5+ rows) and the single GEMM
     agree; odd row counts exercise the remainder slab."""
