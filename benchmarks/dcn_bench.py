@@ -2,15 +2,19 @@
 this library (devis_b200.deform_conv: hand-written gather/scatter kernels + cuBLAS GEMM) against torchvision's CUDA
 operator (the third-party kernel the reference calls, deformable_segmentation.py:265), forward and forward+backward.
 
-    python benchmarks/dcn_bench.py [--instances 60] [--iters 30] [--json out.json]
+    python benchmarks/dcn_bench.py [--instances 60] [--iters 30] [--json out.json] [--deterministic]
 
 `instances` = trajectories x T reaching the mask head (<= TEST.NUM_OUT unique top-k x T at inference; 300/frame is the
 synthetic stress shape of config 4 -- pass --instances 1800 if memory allows).  Prints one JSON line per layer and a
 total; also the split gather-kernel / GEMM time of this library (C-ABI call on preallocated buffers).
+--deterministic also times this library's forward+backward under torch.use_deterministic_algorithms(True) (64-bit
+fixed-point grad_input), alternating with the default mode in the same process (median of --repeats rounds each).
 """
 import argparse
 import json
 import os
+import statistics
+import subprocess
 import sys
 
 import torch
@@ -49,7 +53,11 @@ def main():
     ap.add_argument("--tf32", action="store_true")
     ap.add_argument("--layers", default=None, help="comma-separated subset of layer names (e.g. lay5,out_lay)")
     ap.add_argument("--no-torchvision", action="store_true")
+    ap.add_argument("--deterministic", action="store_true", help="also time the deterministic backward")
+    ap.add_argument("--repeats", type=int, default=5, help="alternating rounds of --deterministic")
     args = ap.parse_args()
+    if args.deterministic:
+        os.environ.setdefault("CUBLAS_WORKSPACE_CONFIG", ":4096:8")    # before the first cuBLAS call
     torch.backends.cuda.matmul.allow_tf32 = args.tf32
     from devis_b200 import _lib
     from devis_b200.deform_conv import deform_conv2d
@@ -87,7 +95,21 @@ def main():
                     t.grad = None
 
         row["ours_fwd_us"] = _time(lambda: step(deform_conv2d, x, False), args.iters)
-        row["ours_fwd_bwd_us"] = _time(lambda: step(deform_conv2d, x, True), args.iters)
+        if args.deterministic:
+            plain, det = [], []
+            for _ in range(args.repeats):
+                plain.append(_time(lambda: step(deform_conv2d, x, True), args.iters))
+                torch.use_deterministic_algorithms(True)
+                try:
+                    det.append(_time(lambda: step(deform_conv2d, x, True), args.iters))
+                finally:
+                    torch.use_deterministic_algorithms(False)
+            row["ours_fwd_bwd_us"] = statistics.median(plain)
+            row["ours_det_fwd_bwd_us"] = statistics.median(det)
+            row["ours_fwd_bwd_us_range"] = [round(min(plain), 1), round(max(plain), 1)]
+            row["ours_det_fwd_bwd_us_range"] = [round(min(det), 1), round(max(det), 1)]
+        else:
+            row["ours_fwd_bwd_us"] = _time(lambda: step(deform_conv2d, x, True), args.iters)
         if tv_deform_conv2d is not None:
             xc = x.contiguous()      # torchvision wants NCHW
             try:
@@ -140,10 +162,18 @@ def main():
         print(json.dumps({k: (round(v, 1) if isinstance(v, float) else v) for k, v in row.items()}), flush=True)
         del x, cols, gcols, gx
     total = {"layer": "total", "instances": n, "tf32": args.tf32, **{k: round(v, 1) for k, v in tot.items()}}
+    if args.deterministic:
+        total["det_overhead"] = round(tot["ours_det_fwd_bwd_us"] / tot["ours_fwd_bwd_us"], 3)
     print(json.dumps(total), flush=True)
     if args.json:
+        try:
+            smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                                 capture_output=True, text=True, timeout=60).stdout.strip()
+        except (OSError, subprocess.SubprocessError):
+            smi = "unavailable"
         with open(args.json, "w") as f:
-            json.dump({"layers": rows, "total": total, "device": torch.cuda.get_device_name(0)}, f, indent=1)
+            json.dump({"layers": rows, "total": total, "device": torch.cuda.get_device_name(0), "nvidia_smi": smi},
+                      f, indent=1)
 
 
 if __name__ == "__main__":

@@ -282,6 +282,42 @@ def run_train(attn="both", iters=8, height=360, width=640, tf32=False, ddp=None,
     return out
 
 
+def run_train_determinism(height=360, width=640, tf32=False, n_matched=5, steps=2):
+    """Bit-reproducible training with this library's kernels (--train --deterministic, --attn ours): under
+    torch.use_deterministic_algorithms(True) run `steps` training steps (forward, backward, clip_grad_norm, AdamW) from
+    the same seed twice and report whether every parameter ends bit-identical.  If an op outside this library has no
+    deterministic implementation, torch raises and the op is reported instead."""
+    dev = torch.device("cuda")
+    torch.backends.cuda.matmul.allow_tf32 = bool(tf32)
+    torch.backends.cudnn.allow_tf32 = bool(tf32)
+    old = torch.are_deterministic_algorithms_enabled()
+    torch.use_deterministic_algorithms(True)
+    try:
+        finals = []
+        for _ in range(2):
+            torch.manual_seed(0)
+            frames = torch.randn(6, 3, height, width, device=dev)
+            pad = torch.zeros(6, height, width, dtype=torch.bool, device=dev)
+            model = DeVISR50().to(dev).train()
+            for p in model.body.parameters():
+                p.requires_grad_(True)
+            params = [p for p in model.parameters() if p.requires_grad]
+            opt = torch.optim.AdamW(params, lr=1e-5, weight_decay=1e-4)
+            for _ in range(steps):
+                opt.zero_grad(set_to_none=True)
+                model.training_loss(frames, pad, n_matched).backward()
+                torch.nn.utils.clip_grad_norm_(params, 0.1)
+                opt.step()
+            finals.append({k: v.detach().clone() for k, v in model.named_parameters()})
+            del model, opt
+    except RuntimeError as exc:
+        return {"error": str(exc)[:500]}
+    finally:
+        torch.use_deterministic_algorithms(old)
+    differ = [k for k in finals[0] if not torch.equal(finals[0][k], finals[1][k])]
+    return {"steps": steps, "parameters": len(finals[0]), "bit_identical": not differ, "differing": differ[:20]}
+
+
 def run(attn="both", iters=20, num_out=20, breakdown=True, height=360, width=640, tf32=False):
     """tf32: torch.backends.{cuda.matmul,cudnn}.allow_tf32 for everything dense (backbone, projections, FFN, mask-head
     GEMMs; the reference's pinned torch 1.11 had both on by default).  The attention kernels are fp32 either way."""
@@ -326,10 +362,18 @@ if __name__ == "__main__":
     ap.add_argument("--no-breakdown", action="store_true")
     ap.add_argument("--tf32", default="both", choices=["off", "on", "both"])
     ap.add_argument("--train", action="store_true", help="time the training step (config 5) instead of inference (config 3)")
+    ap.add_argument("--deterministic", action="store_true",
+                    help="with --train --attn ours: check that two seeded training runs end bit-identical instead of timing")
     a = ap.parse_args()
+    if a.deterministic and not (a.train and a.attn == "ours"):
+        ap.error("--deterministic needs --train --attn ours")
+    if a.deterministic:
+        os.environ.setdefault("CUBLAS_WORKSPACE_CONFIG", ":4096:8")    # before the first cuBLAS call
     res = {}
     for mode in (["off", "on"] if a.tf32 == "both" else [a.tf32]):
-        if a.train:
+        if a.deterministic:
+            res["tf32_" + mode] = run_train_determinism(tf32=mode == "on")
+        elif a.train:
             res["tf32_" + mode] = run_train(a.attn, max(4, a.iters // 3), tf32=mode == "on")
         else:
             res["tf32_" + mode] = run(a.attn, a.iters, a.num_out, not a.no_breakdown, tf32=mode == "on")

@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # DEVIS_MSDA_LIB selects another build of the same ABI (kernel A/B experiments); the default is the in-tree library
 LIB_PATH = os.environ.get("DEVIS_MSDA_LIB") or os.path.join(_HERE, "libdevis_msda.so")
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 F32, F64, BF16 = 0, 1, 2
 FLAG_DETERMINISTIC, FLAG_NO_GRAD_VALUE, FLAG_BF16_GRAD_VALUE = 1, 2, 4
 # temporal_ref_mode of the fused-prologue entry points (DEVIS_TMSDA_TREF_*)
@@ -44,11 +44,14 @@ SIGNATURES = {
     # include/devis_deform_conv.h
     "devis_dcn_im2col": (_i, [_vp] * 4 + [_i] * 15 + [_vp]),
     "devis_dcn_col2im": (_i, [_vp] * 7 + [_i] * 15 + [_vp]),
+    "devis_dcn_backward_workspace_bytes": (_sz, [_i] * 4 + [_u]),
+    "devis_dcn_col2im_ex": (_i, [_vp] * 7 + [_i] * 15 + [_u, _vp, _sz, _vp]),
     "devis_dcn_fused_form": (_i, [_i] * 5),
     "devis_dcn_packed_weight_elems": (_sz, [_i] * 4),
     "devis_dcn_pack_weight": (_i, [_vp] * 2 + [_i] * 4 + [_vp]),
     "devis_dcn_fused_forward": (_i, [_vp] * 6 + [_i] * 15 + [_vp]),
     "devis_dcn_fused_backward": (_i, [_vp] * 8 + [_i] * 15 + [_vp]),
+    "devis_dcn_fused_backward_ex": (_i, [_vp] * 8 + [_i] * 15 + [_u, _vp, _sz, _vp]),
     "devis_dcn_wgrad_supported": (_i, [_i] * 5),
     "devis_dcn_weight_grad": (_i, [_vp] * 5 + [_i] * 15 + [_vp]),
     "devis_dcn_igemm_supported": (_i, [_i] * 5),

@@ -21,11 +21,40 @@
 //     (red.global.add.v4.f32) -- replacing torchvision's three kernels and its scalar atomics;
 //   * grad_offset / grad_mask are written exactly once (no zero fill); only grad_input is zero-filled by the launcher.
 // groups = 1 and offset_groups = 1 (all DeVIS uses); any kernel size, stride, padding, dilation.
+//
+// Deterministic form (DET = true, float only).  The float scatter of grad_input sums in arrival order, so its last bits
+// change from run to run.  The DET kernels convert every grad_input contribution m * w_corner * gc[c] exactly to a 64-bit
+// fixed-point integer and add it with integer atomics (associative), with the machinery of the attention's deterministic
+// grad_value (msda_common.cuh: DetScale, det_exponent, det_add4, det_finalize_kernel).  The scale is 2^(F - e),
+// F = kDetFracBits, 2^e > 2 * bound, where the bound of every contribution |m * w_corner * gc| (|w_corner| <= 1) is the
+// product of the factors in det.max_bits:
+//   col2im        max|grad_cols| * max|mask|                      (kDcnDetFactorsCol2im)
+//   fused bwd     max|grad_out|  * max|mask| * max|W| * Cout      (kDcnDetFactorsFused; gc = sum_co grad_out[co] * W[co][c][k]
+//                 is never stored: Cout * max|W| bounds sum_co |W| and costs at most log2(Cout) <= 4 bits of resolution)
+// (max|mask| is 1 without a mask).  The accumulators are in channel order, the input's channels-last layout: a lane's
+// four channels are four consecutive 8-byte words (one full 32-byte sector), so no permutation is needed and
+// det_finalize_kernel runs with lpg = 0.  The launcher rejects shapes whose Ho * Wo * kh * kw contributions per element
+// and image could overflow int64 (DEVIS_MSDA_ERR_TOO_LARGE).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "msda_common.cuh"
+
 namespace devis {
+
+constexpr int kDcnDetFactorsCol2im = 2, kDcnDetFactorsFused = 4;
+
+// one fixed-point contribution (sh is a power of two: the product and its conversion are exact)
+__device__ __forceinline__ void dcn_det_add(long long *p, float sh, float v)
+{
+    atomicAdd(reinterpret_cast<unsigned long long *>(p), (unsigned long long)__float2ll_rn(v * sh));
+}
+
+__device__ __forceinline__ float dcn_det_scale(const DetScale &det, int n_factors)
+{
+    return ldexpf(1.f, kDetFracBits - det_exponent(det.max_bits, n_factors));
+}
 
 // one 16-byte vector reduction (SASS REDG.E.ADD.F32x4) instead of four scalar atomics
 __device__ __forceinline__ void dcn_red_add_f4(float *p, float a, float b, float c, float d)
@@ -161,12 +190,13 @@ __device__ __forceinline__ void dcn_red_add(double *p, double v) { atomicAdd(p, 
 // ---------------------------------------------------------------------------------------------------------------------
 // backward: grad_input (scatter), grad_offset, grad_mask from grad_cols, one pass per tap
 // ---------------------------------------------------------------------------------------------------------------------
-template <typename T, int V, int G>
+template <typename T, int V, int G, bool DET = false>
 __global__ void __launch_bounds__(256) dcn_col2im_kernel(const T *__restrict__ input, const T *__restrict__ offset,
                                                          const T *__restrict__ mask, const T *__restrict__ grad_cols,
                                                          T *__restrict__ grad_input, T *__restrict__ grad_offset,
-                                                         T *__restrict__ grad_mask, DcnDims d, int n_base)
+                                                         T *__restrict__ grad_mask, DcnDims d, int n_base, DetScale det)
 {
+    static_assert(!DET || sizeof(T) == 4, "the fixed-point form is float only");
     const int j = threadIdx.x % G;
     int pp = (int)((blockIdx.x * blockDim.x + threadIdx.x) / G);
     const bool live = pp < d.Ho * d.Wo;
@@ -179,6 +209,12 @@ __global__ void __launch_bounds__(256) dcn_col2im_kernel(const T *__restrict__ i
     T *gimg = grad_input ? grad_input + (long long)id.n * d.H * d.W * d.C : nullptr;
     const T *gc = grad_cols + (id.pixel * (d.kh * d.kw) + id.k) * (long long)d.C;
     const T f0 = m * t.w[0], f1 = m * t.w[1], f2 = m * t.w[2], f3 = m * t.w[3];
+    long long *gacc = nullptr;
+    float det_sh = 0.f;
+    if constexpr (DET) {
+        gacc = det.acc + (long long)id.n * d.H * d.W * d.C;
+        det_sh = dcn_det_scale(det, kDcnDetFactorsCol2im);
+    }
     T A0 = 0, A1 = 0, A2 = 0, A3 = 0;
     if (V == 4) {
         const float4 *r0 = reinterpret_cast<const float4 *>(img + (long long)t.row[0] * d.C);
@@ -193,6 +229,14 @@ __global__ void __launch_bounds__(256) dcn_col2im_kernel(const T *__restrict__ i
             A1 += g.x * b.x + g.y * b.y + g.z * b.z + g.w * b.w;
             A2 += g.x * e.x + g.y * e.y + g.z * e.z + g.w * e.w;
             A3 += g.x * f.x + g.y * f.y + g.z * f.z + g.w * f.w;
+            if constexpr (DET) {
+                if (live) {
+                    if (f0 != 0.f) det_add4<1>(gacc + (long long)t.row[0] * d.C + 4 * c, det_sh, f0 * g.x, f0 * g.y, f0 * g.z, f0 * g.w);
+                    if (f1 != 0.f) det_add4<1>(gacc + (long long)t.row[1] * d.C + 4 * c, det_sh, f1 * g.x, f1 * g.y, f1 * g.z, f1 * g.w);
+                    if (f2 != 0.f) det_add4<1>(gacc + (long long)t.row[2] * d.C + 4 * c, det_sh, f2 * g.x, f2 * g.y, f2 * g.z, f2 * g.w);
+                    if (f3 != 0.f) det_add4<1>(gacc + (long long)t.row[3] * d.C + 4 * c, det_sh, f3 * g.x, f3 * g.y, f3 * g.z, f3 * g.w);
+                }
+            }
             if (live && gimg) {
                 float *q = reinterpret_cast<float *>(gimg);
                 if (f0 != 0.f) dcn_red_add_f4(q + (long long)t.row[0] * d.C + 4 * c, f0 * g.x, f0 * g.y, f0 * g.z, f0 * g.w);
@@ -210,6 +254,14 @@ __global__ void __launch_bounds__(256) dcn_col2im_kernel(const T *__restrict__ i
             A1 += g * r1[c];
             A2 += g * r2[c];
             A3 += g * r3[c];
+            if constexpr (DET) {
+                if (live) {
+                    if (f0 != (T)0) dcn_det_add(gacc + (long long)t.row[0] * d.C + c, det_sh, f0 * g);
+                    if (f1 != (T)0) dcn_det_add(gacc + (long long)t.row[1] * d.C + c, det_sh, f1 * g);
+                    if (f2 != (T)0) dcn_det_add(gacc + (long long)t.row[2] * d.C + c, det_sh, f2 * g);
+                    if (f3 != (T)0) dcn_det_add(gacc + (long long)t.row[3] * d.C + c, det_sh, f3 * g);
+                }
+            }
             if (live && gimg) {
                 if (f0 != (T)0) dcn_red_add(gimg + (long long)t.row[0] * d.C + c, f0 * g);
                 if (f1 != (T)0) dcn_red_add(gimg + (long long)t.row[1] * d.C + c, f1 * g);
@@ -429,12 +481,12 @@ __global__ void __launch_bounds__(256, 2) dcn_fused_fwd_kernel(const float *__re
 // forms its slice of the column gradient on the fly, gc[c] = sum_co grad_out[pixel][co] * weight[co][c][k], and uses it
 // exactly like dcn_col2im_kernel uses grad_cols: corner dot products -> grad_offset / grad_mask, 16-byte vector
 // reductions -> grad_input.  The weight gradient (cols^T x grad_out) is computed by the caller from recomputed columns.
-template <int COUT, int G, int PPG>
+template <int COUT, int G, int PPG, bool DET = false>
 __global__ void __launch_bounds__(256, 2) dcn_fused_bwd_kernel(const float *__restrict__ input, const float *__restrict__ offset,
                                                             const float *__restrict__ mask, const float4 *__restrict__ wp,
                                                             const float *__restrict__ grad_out /* (pixels, COUT) */,
                                                             float *__restrict__ grad_input, float *__restrict__ grad_offset,
-                                                            float *__restrict__ grad_mask, DcnDims d, int n_base)
+                                                            float *__restrict__ grad_mask, DetScale det, DcnDims d, int n_base)
 {
     const DcnTile<G, PPG> tile(d, n_base);
     if (!tile.row_live) return;
@@ -443,6 +495,12 @@ __global__ void __launch_bounds__(256, 2) dcn_fused_bwd_kernel(const float *__re
     const long long plane = (long long)d.Ho * d.Wo;
     const float4 *img = reinterpret_cast<const float4 *>(input + (long long)tile.n * d.H * d.W * d.C);
     float *gimg = grad_input ? grad_input + (long long)tile.n * d.H * d.W * d.C : nullptr;
+    long long *gacc = nullptr;
+    float det_sh = 0.f;
+    if constexpr (DET) {
+        gacc = det.acc + (long long)tile.n * d.H * d.W * d.C;
+        det_sh = dcn_det_scale(det, kDcnDetFactorsFused);
+    }
     const float *offset_n = offset + (long long)tile.n * 2 * K * plane;
     const float *mask_n = mask ? mask + (long long)tile.n * K * plane : nullptr;
     float *goff_n = grad_offset + (long long)tile.n * 2 * K * plane;
@@ -504,7 +562,10 @@ __global__ void __launch_bounds__(256, 2) dcn_fused_bwd_kernel(const float *__re
                     const float4 r = corner[i][q];
                     A[i][q] += gc[i].x * r.x + gc[i].y * r.y + gc[i].z * r.z + gc[i].w * r.w;
                     const float f = fw[i][q];
-                    if (gimg && tile.live[i] && f != 0.f)
+                    if constexpr (DET) {
+                        if (tile.live[i] && f != 0.f)
+                            det_add4<1>(gacc + ((long long)t[i].row[q] * C4 + c) * 4, det_sh, f * gc[i].x, f * gc[i].y, f * gc[i].z, f * gc[i].w);
+                    } else if (gimg && tile.live[i] && f != 0.f)
                         dcn_red_add_f4(gimg + ((long long)t[i].row[q] * C4 + c) * 4, f * gc[i].x, f * gc[i].y, f * gc[i].z, f * gc[i].w);
                 }
             }

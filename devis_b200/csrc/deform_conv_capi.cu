@@ -20,6 +20,51 @@ int check_dims(const DcnDims &d, int dtype)
     return DEVIS_MSDA_OK;
 }
 
+// ---- deterministic grad_input (DEVIS_MSDA_FLAG_DETERMINISTIC, deform_conv.cuh "Deterministic form") ---------------------
+// workspace: [int64 accumulators, one per grad_input element][4 x u32 bound factors]
+size_t det_workspace_bytes(long long batch, long long height, long long width, long long channels)
+{
+    return (size_t)(batch * height * width * channels) * sizeof(long long) + 4 * sizeof(unsigned);
+}
+
+// host-side checks of a deterministic call, before any CUDA call
+int check_det(const DcnDims &d, int dtype, const void *workspace, size_t workspace_bytes)
+{
+    if (dtype != DEVIS_MSDA_F32) return DEVIS_MSDA_ERR_UNSUPPORTED;
+    // a tap's live corners are distinct pixels, so one grad_input element receives at most Ho*Wo*kh*kw contributions per
+    // image, each below 2^F in magnitude: their int64 sum cannot overflow while that count stays below 2^(62 - F)
+    if ((double)d.Ho * d.Wo * d.kh * d.kw >= (double)(1LL << (62 - kDetFracBits))) return DEVIS_MSDA_ERR_TOO_LARGE;
+    if (!workspace || workspace_bytes < det_workspace_bytes(d.N, d.H, d.W, d.C)) return DEVIS_MSDA_ERR_WORKSPACE;
+    return DEVIS_MSDA_OK;
+}
+
+// zero the accumulators and the bound factors; factor 0 = max|grad| (n_grad floats), factor 1 = max|mask| (1 without one)
+int det_begin(void *workspace, const DcnDims &d, const void *grad, size_t n_grad, const void *mask, cudaStream_t st,
+              DetScale &det, unsigned *&slots)
+{
+    const size_t n_acc = (size_t)d.N * d.H * d.W * d.C;
+    const cudaError_t e = cudaMemsetAsync(workspace, 0, det_workspace_bytes(d.N, d.H, d.W, d.C), st);
+    if (e != cudaSuccess) return devis_capi_cuda_fail(e);
+    det.acc = reinterpret_cast<long long *>(workspace);
+    slots = reinterpret_cast<unsigned *>(det.acc + n_acc);
+    det.max_bits = slots;
+    const int blocks = devis_capi_helper_blocks();
+    absmax_kernel<false><<<blocks, 256, 0, st>>>(grad, n_grad, slots);
+    int rc = devis_capi_check_launch(DEVIS_MSDA_KERNEL_AUX);
+    if (rc) return rc;
+    if (mask) absmax_kernel<false><<<blocks, 256, 0, st>>>(mask, (size_t)d.N * d.kh * d.kw * d.Ho * d.Wo, slots + 1);
+    else set_word_kernel<<<1, 1, 0, st>>>(slots + 1, 0x3f800000u);
+    return devis_capi_check_launch(DEVIS_MSDA_KERNEL_AUX);
+}
+
+// fixed point -> grad_input (channel order, every element written)
+int det_finish(const DetScale &det, const DcnDims &d, void *grad_input, int n_factors, cudaStream_t st)
+{
+    det_finalize_kernel<<<devis_capi_helper_blocks(), 256, 0, st>>>(det.acc, (float *)grad_input,
+                                                                   (size_t)d.N * d.H * d.W * d.C, det.max_bits, 0, n_factors);
+    return devis_capi_check_launch(DEVIS_MSDA_KERNEL_AUX);
+}
+
 // lanes per tap: a group covers its channels in 16-byte pieces; 8 lanes = one 128-byte line per corner row.
 // Grid: x = output plane (wo fastest), y = kernel position, z = batch item (in slices of at most 65535).
 constexpr int kMaxGridZ = 65535;
@@ -81,42 +126,80 @@ int devis_dcn_im2col(const void *input, const void *offset, const void *mask, vo
                     [&](dim3 b, int n0) { dcn_im2col_kernel<double, 1, 32><<<b, 256, 0, st>>>(in, of, mk, co, d, n0); });
 }
 
+size_t devis_dcn_backward_workspace_bytes(int batch, int height, int width, int channels, unsigned flags)
+{
+    if (!(flags & DEVIS_MSDA_FLAG_DETERMINISTIC) || batch < 0 || height < 0 || width < 0 || channels < 0) return 0;
+    return det_workspace_bytes(batch, height, width, channels);
+}
+
 int devis_dcn_col2im(const void *input, const void *offset, const void *mask, const void *grad_cols, void *grad_input,
                      void *grad_offset, void *grad_mask, int batch, int height, int width, int channels, int out_h,
                      int out_w, int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w, int dil_h,
                      int dil_w, int dtype, void *stream)
 {
+    return devis_dcn_col2im_ex(input, offset, mask, grad_cols, grad_input, grad_offset, grad_mask, batch, height, width,
+                               channels, out_h, out_w, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w,
+                               dtype, 0u, nullptr, 0, stream);
+}
+
+int devis_dcn_col2im_ex(const void *input, const void *offset, const void *mask, const void *grad_cols, void *grad_input,
+                        void *grad_offset, void *grad_mask, int batch, int height, int width, int channels, int out_h,
+                        int out_w, int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w, int dil_h,
+                        int dil_w, int dtype, unsigned flags, void *workspace, size_t workspace_bytes, void *stream)
+{
     const DcnDims d{batch, height, width, channels, out_h, out_w, kernel_h, kernel_w,
                     stride_h, stride_w, pad_h, pad_w, dil_h, dil_w};
-    const int rc = check_dims(d, dtype);
+    int rc = check_dims(d, dtype);
     if (rc) return rc;
+    const bool det_flag = (flags & DEVIS_MSDA_FLAG_DETERMINISTIC) && grad_input;
+    if (det_flag) {
+        rc = check_det(d, dtype, workspace, workspace_bytes);
+        if (rc) return rc;
+    }
     const long long n_taps = (long long)batch * out_h * out_w * kernel_h * kernel_w;
     if (n_taps > 0 && (!input || !offset || !grad_cols || !grad_offset || (mask && !grad_mask)))
         return DEVIS_MSDA_ERR_NULL_POINTER;
     cudaStream_t st = (cudaStream_t)stream;
-    if (grad_input) {   // torchvision: at::zeros_like(input)
+    const bool det = det_flag && n_taps > 0;        // no taps: grad_input is all zeros, filled below
+    if (grad_input && !det) {   // torchvision: at::zeros_like(input)
         const size_t bytes = (size_t)batch * height * width * channels * (dtype == DEVIS_MSDA_F64 ? 8 : 4);
         if (bytes) {
             const cudaError_t e = cudaMemsetAsync(grad_input, 0, bytes, st);
             if (e != cudaSuccess) return devis_capi_cuda_fail(e);
         }
     }
+    if (det) {
+        DetScale ds{};
+        unsigned *slots = nullptr;
+        rc = det_begin(workspace, d, grad_cols, (size_t)n_taps * channels, mask, st, ds, slots);
+        if (rc) return rc;
+        const float *in = (const float *)input, *of = (const float *)offset, *mk = (const float *)mask;
+        const float *gc = (const float *)grad_cols;
+        float *go = (float *)grad_offset, *gm = (float *)grad_mask;
+        rc = dispatch(d, dtype,
+                      [&](dim3 b, int n0) { dcn_col2im_kernel<float, 4, 4, true><<<b, 256, 0, st>>>(in, of, mk, gc, nullptr, go, gm, d, n0, ds); },
+                      [&](dim3 b, int n0) { dcn_col2im_kernel<float, 4, 8, true><<<b, 256, 0, st>>>(in, of, mk, gc, nullptr, go, gm, d, n0, ds); },
+                      [&](dim3 b, int n0) { dcn_col2im_kernel<float, 1, 8, true><<<b, 256, 0, st>>>(in, of, mk, gc, nullptr, go, gm, d, n0, ds); },
+                      [&](dim3 b, int n0) { dcn_col2im_kernel<float, 1, 32, true><<<b, 256, 0, st>>>(in, of, mk, gc, nullptr, go, gm, d, n0, ds); });
+        return rc ? rc : det_finish(ds, d, grad_input, kDcnDetFactorsCol2im, st);
+    }
+    const DetScale nodet{};
     if (dtype == DEVIS_MSDA_F32) {
         const float *in = (const float *)input, *of = (const float *)offset, *mk = (const float *)mask;
         const float *gc = (const float *)grad_cols;
         float *gi = (float *)grad_input, *go = (float *)grad_offset, *gm = (float *)grad_mask;
         return dispatch(d, dtype,
-                        [&](dim3 b, int n0) { dcn_col2im_kernel<float, 4, 4><<<b, 256, 0, st>>>(in, of, mk, gc, gi, go, gm, d, n0); },
-                        [&](dim3 b, int n0) { dcn_col2im_kernel<float, 4, 8><<<b, 256, 0, st>>>(in, of, mk, gc, gi, go, gm, d, n0); },
-                        [&](dim3 b, int n0) { dcn_col2im_kernel<float, 1, 8><<<b, 256, 0, st>>>(in, of, mk, gc, gi, go, gm, d, n0); },
-                        [&](dim3 b, int n0) { dcn_col2im_kernel<float, 1, 32><<<b, 256, 0, st>>>(in, of, mk, gc, gi, go, gm, d, n0); });
+                        [&](dim3 b, int n0) { dcn_col2im_kernel<float, 4, 4><<<b, 256, 0, st>>>(in, of, mk, gc, gi, go, gm, d, n0, nodet); },
+                        [&](dim3 b, int n0) { dcn_col2im_kernel<float, 4, 8><<<b, 256, 0, st>>>(in, of, mk, gc, gi, go, gm, d, n0, nodet); },
+                        [&](dim3 b, int n0) { dcn_col2im_kernel<float, 1, 8><<<b, 256, 0, st>>>(in, of, mk, gc, gi, go, gm, d, n0, nodet); },
+                        [&](dim3 b, int n0) { dcn_col2im_kernel<float, 1, 32><<<b, 256, 0, st>>>(in, of, mk, gc, gi, go, gm, d, n0, nodet); });
     }
     const double *in = (const double *)input, *of = (const double *)offset, *mk = (const double *)mask;
     const double *gc = (const double *)grad_cols;
     double *gi = (double *)grad_input, *go = (double *)grad_offset, *gm = (double *)grad_mask;
     return dispatch(d, dtype, [&](dim3, int) {}, [&](dim3, int) {},
-                    [&](dim3 b, int n0) { dcn_col2im_kernel<double, 1, 8><<<b, 256, 0, st>>>(in, of, mk, gc, gi, go, gm, d, n0); },
-                    [&](dim3 b, int n0) { dcn_col2im_kernel<double, 1, 32><<<b, 256, 0, st>>>(in, of, mk, gc, gi, go, gm, d, n0); });
+                    [&](dim3 b, int n0) { dcn_col2im_kernel<double, 1, 8><<<b, 256, 0, st>>>(in, of, mk, gc, gi, go, gm, d, n0, nodet); },
+                    [&](dim3 b, int n0) { dcn_col2im_kernel<double, 1, 32><<<b, 256, 0, st>>>(in, of, mk, gc, gi, go, gm, d, n0, nodet); });
 }
 
 
@@ -331,17 +414,44 @@ int devis_dcn_fused_backward(const void *input, const void *offset, const void *
                              int stride_h, int stride_w, int pad_h, int pad_w, int dil_h, int dil_w, int out_channels,
                              void *stream)
 {
+    return devis_dcn_fused_backward_ex(input, offset, mask, packed_weight, grad_out, grad_input, grad_offset, grad_mask,
+                                       batch, height, width, channels, out_h, out_w, kernel_h, kernel_w, stride_h, stride_w,
+                                       pad_h, pad_w, dil_h, dil_w, out_channels, 0u, nullptr, 0, stream);
+}
+
+}  // extern "C"
+
+// the deterministic data backward, launched through the same DCN_FUSED_CASES switch as the default one
+template <int COUT, int G, int PPG>
+constexpr auto dcn_fused_bwd_det_kernel = dcn_fused_bwd_kernel<COUT, G, PPG, true>;
+
+extern "C" {
+
+int devis_dcn_fused_backward_ex(const void *input, const void *offset, const void *mask, const void *packed_weight,
+                                const void *grad_out, void *grad_input, void *grad_offset, void *grad_mask, int batch,
+                                int height, int width, int channels, int out_h, int out_w, int kernel_h, int kernel_w,
+                                int stride_h, int stride_w, int pad_h, int pad_w, int dil_h, int dil_w, int out_channels,
+                                unsigned flags, void *workspace, size_t workspace_bytes, void *stream)
+{
     const DcnDims d{batch, height, width, channels, out_h, out_w, kernel_h, kernel_w,
                     stride_h, stride_w, pad_h, pad_w, dil_h, dil_w};
-    const int rc = check_dims(d, DEVIS_MSDA_F32);
+    int rc = check_dims(d, DEVIS_MSDA_F32);
     if (rc) return rc;
     const FusedPlan plan = fused_plan(channels, out_channels, kernel_h, kernel_w, DEVIS_MSDA_F32);
     if (!plan.lanes_bwd) return DEVIS_MSDA_ERR_UNSUPPORTED;
+    const bool det_flag = (flags & DEVIS_MSDA_FLAG_DETERMINISTIC) && grad_input;
+    if (det_flag) {
+        rc = check_det(d, DEVIS_MSDA_F32, workspace, workspace_bytes);
+        if (rc) return rc;
+    }
     const long long n_pixels = (long long)batch * out_h * out_w;
     if (n_pixels > 0 && (!input || !offset || !packed_weight || !grad_out || !grad_offset || (mask && !grad_mask)))
         return DEVIS_MSDA_ERR_NULL_POINTER;
+    if (n_pixels > 0 && ((long long)out_h * out_w >= (1LL << 31) || (long long)height * width * channels >= (1LL << 31)))
+        return DEVIS_MSDA_ERR_TOO_LARGE;
     cudaStream_t st = (cudaStream_t)stream;
-    if (grad_input) {
+    const bool det = det_flag && n_pixels > 0;      // no pixels: grad_input is all zeros, filled below
+    if (grad_input && !det) {
         const size_t bytes = (size_t)batch * height * width * channels * 4;
         if (bytes) {
             const cudaError_t e = cudaMemsetAsync(grad_input, 0, bytes, st);
@@ -349,14 +459,30 @@ int devis_dcn_fused_backward(const void *input, const void *offset, const void *
         }
     }
     if (n_pixels == 0) return DEVIS_MSDA_OK;
-    if ((long long)out_h * out_w >= (1LL << 31) || (long long)height * width * channels >= (1LL << 31))
-        return DEVIS_MSDA_ERR_TOO_LARGE;
     const float *in = (const float *)input, *of = (const float *)offset, *mk = (const float *)mask;
     const float4 *wp = (const float4 *)packed_weight;
     const float *go = (const float *)grad_out;
     float *gi = (float *)grad_input, *gof = (float *)grad_offset, *gm = (float *)grad_mask;
-    if (plan.G == 8) { DCN_FUSED_CASES(dcn_fused_bwd_kernel, 8, 1, in, of, mk, wp, go, gi, gof, gm) }
-    else { DCN_FUSED_CASES(dcn_fused_bwd_kernel, 4, 1, in, of, mk, wp, go, gi, gof, gm) }
+    if (det) {
+        DetScale ds{};
+        unsigned *slots = nullptr;
+        rc = det_begin(workspace, d, grad_out, (size_t)n_pixels * out_channels, mask, st, ds, slots);
+        if (rc) return rc;
+        // factors 2, 3: max|W| over the lane-group layout (zero padded: same maximum) and Cout
+        absmax_kernel<false><<<devis_capi_helper_blocks(), 256, 0, st>>>(packed_weight, plan.lanes_elems, slots + 2);
+        rc = devis_capi_check_launch(DEVIS_MSDA_KERNEL_AUX);
+        if (rc) return rc;
+        const float cout_f = (float)out_channels;
+        set_word_kernel<<<1, 1, 0, st>>>(slots + 3, *reinterpret_cast<const unsigned *>(&cout_f));
+        rc = devis_capi_check_launch(DEVIS_MSDA_KERNEL_AUX);
+        if (rc) return rc;
+        if (plan.G == 8) { DCN_FUSED_CASES(dcn_fused_bwd_det_kernel, 8, 1, in, of, mk, wp, go, nullptr, gof, gm, ds) }
+        else { DCN_FUSED_CASES(dcn_fused_bwd_det_kernel, 4, 1, in, of, mk, wp, go, nullptr, gof, gm, ds) }
+        return det_finish(ds, d, grad_input, kDcnDetFactorsFused, st);
+    }
+    const DetScale nodet{};
+    if (plan.G == 8) { DCN_FUSED_CASES(dcn_fused_bwd_kernel, 8, 1, in, of, mk, wp, go, gi, gof, gm, nodet) }
+    else { DCN_FUSED_CASES(dcn_fused_bwd_kernel, 4, 1, in, of, mk, wp, go, gi, gof, gm, nodet) }
     return DEVIS_MSDA_OK;
 }
 

@@ -475,9 +475,12 @@ struct DetScale {
 
 constexpr int kDetFracBits = 36;
 
-__device__ __forceinline__ int det_exponent(const unsigned *max_bits)
+// the bound is the product of n_factors non-negative floats max_bits[0 .. n_factors) (the attention: 2; the deformable
+// convolution, deform_conv.cuh: 4)
+__device__ __forceinline__ int det_exponent(const unsigned *max_bits, int n_factors = 2)
 {
-    const float bound = __uint_as_float(max_bits[0]) * __uint_as_float(max_bits[1]);
+    float bound = __uint_as_float(max_bits[0]);
+    for (int i = 1; i < n_factors; ++i) bound *= __uint_as_float(max_bits[i]);
     int e = 0;
     if (bound > 0.f && bound < 3.0e38f) (void)frexpf(bound, &e);   // bound = f * 2^e, f in [0.5, 1)
     return e + 1;
@@ -514,13 +517,16 @@ __global__ void __launch_bounds__(256) absmax_kernel(const void *x, size_t n, un
     if ((threadIdx.x & 31) == 0) atomicMax(slot, __float_as_uint(m));
 }
 
-__global__ void set_word_kernel(unsigned *slot, unsigned bits) { *slot = bits; }
+// set_word_kernel and det_finalize_kernel are static: each translation unit that includes this header (the attention's
+// and the deformable convolution's) keeps its own copy
+static __global__ void set_word_kernel(unsigned *slot, unsigned bits) { *slot = bits; }
 
-// lpg > 0: the accumulators of every D = 4*lpg channels are in the permuted order of det_add4; lpg == 0: channel order
-__global__ void __launch_bounds__(256) det_finalize_kernel(const long long *acc, float *out, size_t n,
-                                                           const unsigned *max_bits, int lpg)
+// lpg > 0: the accumulators of every D = 4*lpg channels are in the permuted order of det_add4; lpg == 0: channel order.
+// n_factors: as det_exponent
+static __global__ void __launch_bounds__(256) det_finalize_kernel(const long long *acc, float *out, size_t n,
+                                                           const unsigned *max_bits, int lpg, int n_factors = 2)
 {
-    const double back = ldexp(1.0, det_exponent(max_bits) - kDetFracBits);
+    const double back = ldexp(1.0, det_exponent(max_bits, n_factors) - kDetFracBits);
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
         size_t src = i;
         if (lpg) {

@@ -52,15 +52,14 @@ _warned_nondeterministic = False
 
 
 def _alert_not_deterministic():
-    """grad_input is scattered with float ``red.global.add`` (fused backward and devis_dcn_col2im alike): the sum order,
-    hence the last bits, change from run to run -- unlike the attention op, the deformable convolution has no
-    fixed-point mode.  Under ``torch.use_deterministic_algorithms(True)`` say so, the way ATen's non-deterministic
-    kernels do (error, or a warning in warn_only mode); only the WEIGHT gradient is rerouted to a deterministic GEMM."""
+    """float64 grad_input is scattered with float atomics: the sum order, hence the last bits, change from run to run
+    (the fixed-point form of _grad_input_flags is float32 only).  Under ``torch.use_deterministic_algorithms(True)`` say
+    so, the way ATen's non-deterministic kernels do (error, or a warning in warn_only mode)."""
     global _warned_nondeterministic
     if not torch.are_deterministic_algorithms_enabled():
         return
-    msg = ("devis_b200.deform_conv2d backward does not have a deterministic implementation for grad_input (float atomic "
-           "scatter), but you set 'torch.use_deterministic_algorithms(True)'")
+    msg = ("devis_b200.deform_conv2d backward does not have a deterministic implementation for float64 grad_input "
+           "(float atomic scatter), but you set 'torch.use_deterministic_algorithms(True)'")
     if torch.is_deterministic_algorithms_warn_only_enabled():
         if not _warned_nondeterministic:
             warnings.warn(msg, stacklevel=3)
@@ -68,6 +67,34 @@ def _alert_not_deterministic():
         return
     raise RuntimeError(msg + ". You can turn off determinism just for this operation, or use warn_only=True.")
 _COLS_CHUNK_BYTES = 256 << 20          # recomputed columns per weight-gradient chunk
+_DET_ACC_CHUNK_BYTES = 256 << 20       # 64-bit grad_input accumulators per deterministic data-backward call
+
+
+def _grad_input_flags(dtype):
+    """backward flags of the grad_input scatter.  Under ``torch.use_deterministic_algorithms(True)`` float32 takes the
+    64-bit fixed-point form (DEVIS_MSDA_FLAG_DETERMINISTIC: bit-identical run to run); float64 has none (2^-36 of the
+    largest contribution is coarser than float64 accumulation) and raises torch's alert instead."""
+    if not torch.are_deterministic_algorithms_enabled():
+        return 0
+    if dtype == torch.float32:
+        return _lib.FLAG_DETERMINISTIC
+    _alert_not_deterministic()
+    return 0
+
+
+def _data_chunk(n, h, w, c, flags, per):
+    """batch items per data-backward call: ``per`` (the caller's bound), and with the fixed-point form at most
+    _DET_ACC_CHUNK_BYTES of accumulators (8 B per input element; 6.6 GB for 1800 instances of a 32-channel 90 x 160 map).
+    Each call has its own fixed-point scale, which depends on the shapes and the values only."""
+    if flags:
+        per = min(per, _DET_ACC_CHUNK_BYTES // max(1, h * w * c * 8))
+    return max(1, min(n, per))
+
+
+def _workspace(lib, per, h, w, c, flags, device):
+    """(workspace, bytes) of a data-backward call over ``per`` batch items"""
+    nbytes = int(lib.devis_dcn_backward_workspace_bytes(per, h, w, c, flags))
+    return (torch.empty(nbytes, dtype=torch.uint8, device=device), nbytes) if nbytes else (None, 0)
 
 
 def _wgrad(g2, cols):
@@ -160,27 +187,35 @@ class FusedDeformConv2dFunction(Function):
         stream = torch.cuda.current_stream().cuda_stream
         with torch.cuda.device(x.device):
             if need_in or need_off or (need_m and mask is not None):
-                if need_in:
-                    _alert_not_deterministic()
+                flags = _grad_input_flags(x.dtype) if need_in else 0
                 gx = torch.empty_like(x) if need_in else None
                 grad_off = torch.empty_like(offset)
                 grad_m = torch.empty_like(mask) if mask is not None else None
                 if ctx.form & 2:
-                    _lib.check(lib.devis_dcn_fused_backward(_ptr(x), _ptr(offset), _ptr(mask), _ptr(packed), _ptr(g), _ptr(gx),
-                                                            _ptr(grad_off), _ptr(grad_m), *ctx.dims, cout, stream))
+                    per = _data_chunk(n, h, w, c, flags, n)
+                    ws, ws_bytes = _workspace(lib, per, h, w, c, flags, x.device)
+                    for n0 in range(0, n, per):
+                        n1 = min(n, n0 + per)
+                        _lib.check(lib.devis_dcn_fused_backward_ex(
+                            _ptr(x[n0:n1]), _ptr(offset[n0:n1]), _ptr(mask[n0:n1]) if mask is not None else None,
+                            _ptr(packed), _ptr(g[n0:n1]), _ptr(gx[n0:n1]) if need_in else None, _ptr(grad_off[n0:n1]),
+                            _ptr(grad_m[n0:n1]) if mask is not None else None, n1 - n0, *ctx.dims[1:], cout, flags,
+                            _ptr(ws), ws_bytes, stream))
                 else:
                     # wider layers: column gradient by GEMM (a bounded chunk of the batch at a time) + scatter kernel
                     w2 = ctx.weight.permute(0, 2, 3, 1).reshape(cout, k * c)
-                    per = max(1, min(n, _COLS_CHUNK_BYTES // max(1, ho * wo * k * c * 4)))
+                    per = _data_chunk(n, h, w, c, flags, _COLS_CHUNK_BYTES // max(1, ho * wo * k * c * 4))
+                    ws, ws_bytes = _workspace(lib, per, h, w, c, flags, x.device)
                     g2 = g.view(n * ho * wo, cout)
                     for n0 in range(0, n, per):
                         n1 = min(n, n0 + per)
                         grad_cols = g2[n0 * ho * wo:n1 * ho * wo] @ w2
-                        _lib.check(lib.devis_dcn_col2im(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
-                                                        _ptr(mask[n0:n1]) if mask is not None else None, _ptr(grad_cols),
-                                                        _ptr(gx[n0:n1]) if need_in else None, _ptr(grad_off[n0:n1]),
-                                                        _ptr(grad_m[n0:n1]) if mask is not None else None, n1 - n0,
-                                                        *ctx.dims[1:], _DTYPES[x.dtype], stream))
+                        _lib.check(lib.devis_dcn_col2im_ex(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
+                                                           _ptr(mask[n0:n1]) if mask is not None else None, _ptr(grad_cols),
+                                                           _ptr(gx[n0:n1]) if need_in else None, _ptr(grad_off[n0:n1]),
+                                                           _ptr(grad_m[n0:n1]) if mask is not None else None, n1 - n0,
+                                                           *ctx.dims[1:], _DTYPES[x.dtype], flags, _ptr(ws), ws_bytes,
+                                                           stream))
                 grad_in = gx.permute(0, 3, 1, 2) if need_in else None
             if need_w and x.dtype == torch.float32 and not torch.are_deterministic_algorithms_enabled() \
                     and lib.devis_dcn_wgrad_supported(c, cout, kh, kw, _DTYPES[x.dtype]):
@@ -252,15 +287,24 @@ class DeformConv2dFunction(Function):
             grad_b = g2.sum(0)
         if need_in or need_off or (need_m and mask is not None):
             grad_cols = g2 @ w2
-            if need_in:
-                _alert_not_deterministic()
+            flags = _grad_input_flags(x.dtype) if need_in else 0
             gx = torch.empty_like(x) if need_in else None
             grad_off = torch.empty_like(offset)
             grad_m = torch.empty_like(mask) if mask is not None else None
+            lib = _lib.load()
             with torch.cuda.device(x.device):
-                _lib.check(_lib.load().devis_dcn_col2im(_ptr(x), _ptr(offset), _ptr(mask), _ptr(grad_cols), _ptr(gx),
-                                                        _ptr(grad_off), _ptr(grad_m), *ctx.dims, _DTYPES[x.dtype],
-                                                        torch.cuda.current_stream().cuda_stream))
+                stream = torch.cuda.current_stream().cuda_stream
+                per = _data_chunk(n, h, w, c, flags, n)
+                ws, ws_bytes = _workspace(lib, per, h, w, c, flags, x.device)
+                for n0 in range(0, n, per):
+                    n1 = min(n, n0 + per)
+                    _lib.check(lib.devis_dcn_col2im_ex(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
+                                                       _ptr(mask[n0:n1]) if mask is not None else None,
+                                                       _ptr(grad_cols[n0 * ho * wo:n1 * ho * wo]),
+                                                       _ptr(gx[n0:n1]) if need_in else None, _ptr(grad_off[n0:n1]),
+                                                       _ptr(grad_m[n0:n1]) if mask is not None else None, n1 - n0,
+                                                       *ctx.dims[1:], _DTYPES[x.dtype], flags, _ptr(ws), ws_bytes,
+                                                       stream))
             grad_in = gx.permute(0, 3, 1, 2) if need_in else None
         return grad_in, grad_off, grad_w, grad_b, grad_m, None, None, None
 
@@ -350,20 +394,21 @@ class IGemmDeformConv2dFunction(Function):
             if need_b and ctx.has_bias:
                 grad_b = g2.sum(0)
             if need_in or need_off or (need_m and mask is not None):
-                if need_in:
-                    _alert_not_deterministic()
+                flags = _grad_input_flags(x.dtype) if need_in else 0
                 gx = torch.empty_like(x) if need_in else None
                 grad_off = torch.empty_like(offset)
                 grad_m = torch.empty_like(mask) if mask is not None else None
-                per = max(1, min(n, _COLS_CHUNK_BYTES // max(1, ho * wo * k * c * 4)))
+                per = _data_chunk(n, h, w, c, flags, _COLS_CHUNK_BYTES // max(1, ho * wo * k * c * 4))
+                ws, ws_bytes = _workspace(lib, per, h, w, c, flags, x.device)
                 for n0 in range(0, n, per):
                     n1 = min(n, n0 + per)
                     grad_cols = g2[n0 * ho * wo:n1 * ho * wo] @ w2
-                    _lib.check(lib.devis_dcn_col2im(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
-                                                    _ptr(mask[n0:n1]) if mask is not None else None, _ptr(grad_cols),
-                                                    _ptr(gx[n0:n1]) if need_in else None, _ptr(grad_off[n0:n1]),
-                                                    _ptr(grad_m[n0:n1]) if mask is not None else None, n1 - n0,
-                                                    *ctx.dims[1:], _DTYPES[x.dtype], stream))
+                    _lib.check(lib.devis_dcn_col2im_ex(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
+                                                       _ptr(mask[n0:n1]) if mask is not None else None, _ptr(grad_cols),
+                                                       _ptr(gx[n0:n1]) if need_in else None, _ptr(grad_off[n0:n1]),
+                                                       _ptr(grad_m[n0:n1]) if mask is not None else None, n1 - n0,
+                                                       *ctx.dims[1:], _DTYPES[x.dtype], flags, _ptr(ws), ws_bytes,
+                                                       stream))
                 grad_in = gx.permute(0, 3, 1, 2) if need_in else None
         return grad_in, grad_off, grad_w, grad_b, grad_m, None, None, None
 

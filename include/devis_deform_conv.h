@@ -42,6 +42,26 @@ int devis_dcn_col2im(const void *input_nhwc, const void *offset, const void *mas
                      int channels, int out_h, int out_w, int kernel_h, int kernel_w, int stride_h, int stride_w,
                      int pad_h, int pad_w, int dil_h, int dil_w, int dtype, void *stream);
 
+/* ---- deterministic grad_input -----------------------------------------------------------------------------------------
+ * The default backward scatters grad_input with floating-point atomics: its last bits change from run to run.  The _ex
+ * forms take backward flags (devis_msda.h); with DEVIS_MSDA_FLAG_DETERMINISTIC (float32 only) every grad_input
+ * contribution is converted exactly to 64-bit fixed point and summed with integer atomics, so grad_input is
+ * bit-identical run to run on a device.  Its resolution is 2^-36 of a bound of the largest possible contribution:
+ * max|grad_cols| * max|mask| for col2im, max|grad_out| * max|mask| * out_channels * max|weight| for the fused form
+ * (max|mask| = 1 without a mask); the bound and the scale stay on the device (no synchronisation, graph capture is legal).
+ * grad_offset / grad_mask are written once per element in every mode and are deterministic anyway.
+ * The flag needs a workspace of devis_dcn_backward_workspace_bytes(batch, ...) bytes (8 per grad_input element + 16; 0
+ * without the flag).  Checked on the host before any CUDA call: float64 with the flag -> DEVIS_MSDA_ERR_UNSUPPORTED;
+ * out_h * out_w * kernel_h * kernel_w >= 2^26 (the int64 sum could overflow) -> DEVIS_MSDA_ERR_TOO_LARGE; a missing or
+ * short workspace -> DEVIS_MSDA_ERR_WORKSPACE.  The flag is ignored when grad_input_nhwc is NULL.
+ * devis_dcn_col2im / devis_dcn_fused_backward are the _ex forms with flags = 0. */
+size_t devis_dcn_backward_workspace_bytes(int batch, int height, int width, int channels, unsigned flags);
+int devis_dcn_col2im_ex(const void *input_nhwc, const void *offset, const void *mask, const void *grad_cols,
+                        void *grad_input_nhwc, void *grad_offset, void *grad_mask, int batch, int height, int width,
+                        int channels, int out_h, int out_w, int kernel_h, int kernel_w, int stride_h, int stride_w,
+                        int pad_h, int pad_w, int dil_h, int dil_w, int dtype, unsigned flags, void *workspace,
+                        size_t workspace_bytes, void *stream);
+
 
 /* ---- fused form: gather + contraction with the weights in one kernel; the column matrix is never written ------------
  * For layers with few output channels (the high-resolution half of the mask head) im2col + GEMM is bound by writing and
@@ -73,6 +93,11 @@ int devis_dcn_fused_backward(const void *input_nhwc, const void *offset, const v
                              int batch, int height, int width, int channels, int out_h, int out_w, int kernel_h,
                              int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w, int dil_h, int dil_w,
                              int out_channels, void *stream);
+int devis_dcn_fused_backward_ex(const void *input_nhwc, const void *offset, const void *mask, const void *packed_weight,
+                                const void *grad_out_nhwc, void *grad_input_nhwc, void *grad_offset, void *grad_mask,
+                                int batch, int height, int width, int channels, int out_h, int out_w, int kernel_h,
+                                int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w, int dil_h, int dil_w,
+                                int out_channels, unsigned flags, void *workspace, size_t workspace_bytes, void *stream);
 
 /* devis_dcn_weight_grad: the weight gradient of a narrow layer without a column matrix,
  *   grad_weight[co][k][c] = sum over (n, ho, wo) of mask * bilinear(input[n, .., c]) * grad_out_nhwc[n, ho, wo, co]

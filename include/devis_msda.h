@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define DEVIS_MSDA_ABI_VERSION 2
+#define DEVIS_MSDA_ABI_VERSION 3
 
 /* element types of value / output / grad_output */
 #define DEVIS_MSDA_F32 0  /* value, loc, weights, outputs and all gradients float            */
