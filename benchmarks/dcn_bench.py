@@ -2,13 +2,16 @@
 this library (devis_b200.deform_conv: hand-written gather/scatter kernels + cuBLAS GEMM) against torchvision's CUDA
 operator (the third-party kernel the reference calls, deformable_segmentation.py:265), forward and forward+backward.
 
-    python benchmarks/dcn_bench.py [--instances 60] [--iters 30] [--json out.json] [--deterministic]
+    python benchmarks/dcn_bench.py [--instances 60] [--iters 30] [--json out.json] [--deterministic] [--offset-groups G]
 
 `instances` = trajectories x T reaching the mask head (<= TEST.NUM_OUT unique top-k x T at inference; 300/frame is the
 synthetic stress shape of config 4 -- pass --instances 1800 if memory allows).  Prints one JSON line per layer and a
 total; also the split gather-kernel / GEMM time of this library (C-ABI call on preallocated buffers).
 --deterministic also times this library's forward+backward under torch.use_deterministic_algorithms(True) (64-bit
 fixed-point grad_input), alternating with the default mode in the same process (median of --repeats rounds each).
+--offset-groups G gives both this library and torchvision's operator 2 * G * 9 offset and G * 9 mask channels (every
+mask-head layer's channel count divides by 2, 4 and 8); with G > 1 the tensor-core forward, the constant-bank forward and
+the one-kernel weight gradient do not serve, so those layers run in the im2col form.
 """
 import argparse
 import json
@@ -55,7 +58,11 @@ def main():
     ap.add_argument("--no-torchvision", action="store_true")
     ap.add_argument("--deterministic", action="store_true", help="also time the deterministic backward")
     ap.add_argument("--repeats", type=int, default=5, help="alternating rounds of --deterministic")
+    ap.add_argument("--offset-groups", type=int, default=1)
     args = ap.parse_args()
+    og = args.offset_groups
+    if og < 1:
+        ap.error("--offset-groups must be >= 1")
     if args.deterministic:
         os.environ.setdefault("CUBLAS_WORKSPACE_CONFIG", ":4096:8")    # before the first cuBLAS call
     torch.backends.cuda.matmul.allow_tf32 = args.tf32
@@ -75,11 +82,15 @@ def main():
     for name, cin, cout, h, w in LAYERS:
         if args.layers and name not in args.layers.split(","):
             continue
+        if cin % og:
+            raise SystemExit(f"{name}: {cin} input channels do not divide into {og} offset groups")
         x = rn(n, cin, h, w).contiguous(memory_format=torch.channels_last)
         wt, b = rn(cout, cin, 3, 3) / (3 * cin ** 0.5), rn(cout)
-        off, m = 1.5 * rn(n, 18, h, w), 2 * torch.sigmoid(rn(n, 9, h, w))
+        off, m = 1.5 * rn(n, 18 * og, h, w), 2 * torch.sigmoid(rn(n, 9 * og, h, w))
         gout = rn(n, cout, h, w)
         row = {"layer": name, "instances": n, "cin": cin, "cout": cout, "hw": [h, w]}
+        if og > 1:
+            row["offset_groups"] = og
 
         leaf_sets = {}
 
@@ -126,28 +137,28 @@ def main():
         gx, goff, gm = torch.empty_like(xl), torch.empty_like(off), torch.empty_like(m)
         dims = (n, h, w, cin, h, w, 3, 3, 1, 1, 1, 1, 1, 1)
         st = torch.cuda.current_stream().cuda_stream
-        row["im2col_kernel_us"] = _time(lambda: _lib.check(lib.devis_dcn_im2col(
-            x.data_ptr(), off.data_ptr(), m.data_ptr(), cols.data_ptr(), *dims, _lib.F32, st)), args.iters)
-        row["col2im_kernel_us"] = _time(lambda: _lib.check(lib.devis_dcn_col2im(
+        row["im2col_kernel_us"] = _time(lambda: _lib.check(lib.devis_dcn_im2col_og(
+            x.data_ptr(), off.data_ptr(), m.data_ptr(), cols.data_ptr(), *dims, og, _lib.F32, st)), args.iters)
+        row["col2im_kernel_us"] = _time(lambda: _lib.check(lib.devis_dcn_col2im_og(
             x.data_ptr(), off.data_ptr(), m.data_ptr(), gcols.data_ptr(), gx.data_ptr(), goff.data_ptr(), gm.data_ptr(),
-            *dims, _lib.F32, st)), args.iters)
+            *dims, og, _lib.F32, 0, None, 0, st)), args.iters)
         # fused gather + contraction kernels (layers they serve), same way
-        form = lib.devis_dcn_fused_form(cin, cout, 3, 3, _lib.F32)
+        form = lib.devis_dcn_fused_form_og(cin, cout, 3, 3, og, _lib.F32)
         if form:
-            packed = torch.empty(int(lib.devis_dcn_packed_weight_elems(cin, cout, 3, 3)), device="cuda")
-            _lib.check(lib.devis_dcn_pack_weight(wt.data_ptr(), packed.data_ptr(), cin, cout, 3, 3, st))
+            packed = torch.empty(int(lib.devis_dcn_packed_weight_elems_og(cin, cout, 3, 3, og)), device="cuda")
+            _lib.check(lib.devis_dcn_pack_weight_og(wt.data_ptr(), packed.data_ptr(), cin, cout, 3, 3, og, st))
             out = torch.empty(n, h, w, cout, device="cuda")
             gl = gout.permute(0, 2, 3, 1).contiguous()
         if form & 1:
-            row["fused_fwd_kernel_us"] = _time(lambda: _lib.check(lib.devis_dcn_fused_forward(
-                x.data_ptr(), off.data_ptr(), m.data_ptr(), packed.data_ptr(), b.data_ptr(), out.data_ptr(), *dims, cout,
-                st)), args.iters)
+            row["fused_fwd_kernel_us"] = _time(lambda: _lib.check(lib.devis_dcn_fused_forward_og(
+                x.data_ptr(), off.data_ptr(), m.data_ptr(), packed.data_ptr(), b.data_ptr(), out.data_ptr(), *dims, og,
+                cout, st)), args.iters)
             fb = 4 * (x.numel() + off.numel() + m.numel() + out.numel())
             row["fused_fwd_GBps"] = fb / row["fused_fwd_kernel_us"] / 1e3
         if form & 2:
-            row["fused_bwd_kernel_us"] = _time(lambda: _lib.check(lib.devis_dcn_fused_backward(
+            row["fused_bwd_kernel_us"] = _time(lambda: _lib.check(lib.devis_dcn_fused_backward_og(
                 x.data_ptr(), off.data_ptr(), m.data_ptr(), packed.data_ptr(), gl.data_ptr(), gx.data_ptr(),
-                goff.data_ptr(), gm.data_ptr(), *dims, cout, st)), args.iters)
+                goff.data_ptr(), gm.data_ptr(), *dims, og, cout, 0, None, 0, st)), args.iters)
             bb = 4 * (x.numel() + off.numel() + m.numel() + gl.numel() + gx.numel() + goff.numel() + gm.numel())
             row["fused_bwd_GBps"] = bb / row["fused_bwd_kernel_us"] / 1e3
         # algorithmic bytes of the gather: input + offset + mask read once, columns written once
@@ -161,7 +172,8 @@ def main():
         rows.append(row)
         print(json.dumps({k: (round(v, 1) if isinstance(v, float) else v) for k, v in row.items()}), flush=True)
         del x, cols, gcols, gx
-    total = {"layer": "total", "instances": n, "tf32": args.tf32, **{k: round(v, 1) for k, v in tot.items()}}
+    total = {"layer": "total", "instances": n, "tf32": args.tf32, **({"offset_groups": og} if og > 1 else {}),
+             **{k: round(v, 1) for k, v in tot.items()}}
     if args.deterministic:
         total["det_overhead"] = round(tot["ours_det_fwd_bwd_us"] / tot["ours_fwd_bwd_us"], 3)
     print(json.dumps(total), flush=True)

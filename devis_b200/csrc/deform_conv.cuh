@@ -12,15 +12,21 @@
 // attention kernels of this library:
 //   * the input is read CHANNELS-LAST (N, H, W, C): a bilinear corner is one contiguous row of C channels, gathered
 //     with 16-byte loads by a group of G lanes (G = 4..32 by channel count);
-//   * a TAP is one (output pixel, kernel position): the tap's geometry is computed once per lane group, its column
-//     slice (C values) is written contiguously: cols[(pixel * K + k) * C + c] -- the GEMM with the weights stays in
-//     cuBLAS (as torchvision's does, at::addmm), it is not part of this file;
+//   * a TAP is one (output pixel, kernel position, offset group): the tap's geometry is computed once per lane group,
+//     its column slice (the group's Cg = C / offset_groups channels) is written contiguously:
+//     cols[(pixel * K + k) * C + g * Cg + c] -- the GEMM with the weights stays in cuBLAS (as torchvision's does,
+//     at::addmm), it is not part of this file;
 //   * backward: ONE pass per tap gathers the four corner rows again, forms the four dot products
 //     A_c = sum_ch grad_col[ch] * corner_c[ch] (reduced over the group with shuffles) from which grad_mask and
 //     grad_offset follow in closed form, and scatters grad_input with 16-byte vector reductions
 //     (red.global.add.v4.f32) -- replacing torchvision's three kernels and its scalar atomics;
 //   * grad_offset / grad_mask are written exactly once (no zero fill); only grad_input is zero-filled by the launcher.
-// groups = 1 and offset_groups = 1 (all DeVIS uses); any kernel size, stride, padding, dilation.
+// Offset groups (torchvision's offset_groups, DCNv2's deformable groups): group g of G reads offset channels
+// 2 * (g * K + k) (+1) and mask channel g * K + k, and covers input channels [g * Cg, (g + 1) * Cg).  A kernel position
+// of a group is a VIRTUAL position v = g * K + k with its own channel window; with G = 1, v = k and every kernel computes
+// what it computed before offset groups existed.  The im2col / col2im kernels and the lane-group fused kernels serve
+// any G; the constant-bank forward, the tcgen05 forward (dcn_igemm.cuh) and dcn_wgrad_kernel serve G = 1 only.
+// groups = 1 (no weight grouping); any kernel size, stride, padding, dilation.
 //
 // Deterministic form (DET = true, float only).  The float scatter of grad_input sums in arrival order, so its last bits
 // change from run to run.  The DET kernels convert every grad_input contribution m * w_corner * gc[c] exactly to a 64-bit
@@ -66,6 +72,7 @@ struct DcnDims {
     int N, H, W, C;       // input, channels-last
     int Ho, Wo;           // output size
     int kh, kw, sh, sw, ph, pw, dh, dw;
+    int og = 1;           // offset groups: C % og == 0
 };
 
 // geometry of one tap, torchvision's bilinear_interpolate: the sample is void unless -1 < h < H and -1 < w < W; corners
@@ -108,12 +115,14 @@ __device__ __forceinline__ DcnTap<T> dcn_tap(T h, T w, int H, int W)
     return t;
 }
 
-// A tap is addressed by the launch grid: blockIdx.z (+ n_base) = batch item, blockIdx.y = kernel position, and the
+// A tap is addressed by the launch grid: blockIdx.z (+ n_base) = batch item, blockIdx.y = virtual kernel position
+// v = g * K + k (offset group g, kernel position k), and the
 // x dimension runs over the output plane with wo fastest: the groups of a warp work on neighbouring output pixels for
 // the same kernel position, so their offset / mask reads are coalesced and their gathers share a neighbourhood of the
 // input.  (32-bit arithmetic only: a 64-bit division per index component cost more than the gather itself.)
 struct DcnTapId {
     int n, k, ho, wo;
+    int v;             // g * K + k: the tap's offset / mask channel (offset group g)
     long long pixel;   // (n * Ho + ho) * Wo + wo
 };
 
@@ -122,6 +131,7 @@ __device__ __forceinline__ DcnTapId dcn_tap_id(int plane_pixel, int n, int k, co
     DcnTapId id;
     id.n = n;
     id.k = k;
+    id.v = k;
     id.ho = plane_pixel / d.Wo;
     id.wo = plane_pixel - id.ho * d.Wo;
     id.pixel = (long long)n * d.Ho * d.Wo + plane_pixel;
@@ -132,20 +142,20 @@ template <typename T>
 __device__ __forceinline__ void dcn_sample_point(const T *offset, const T *mask, const DcnTapId &id, const DcnDims &d,
                                                  T &h, T &w, T &m)
 {
-    const int K = d.kh * d.kw;
+    const int GK = d.og * d.kh * d.kw;
     const long long plane = (long long)d.Ho * d.Wo;
     const long long at = (long long)id.ho * d.Wo + id.wo;
-    const T off_h = offset[((long long)id.n * 2 * K + 2 * id.k) * plane + at];
-    const T off_w = offset[((long long)id.n * 2 * K + 2 * id.k + 1) * plane + at];
-    m = mask ? mask[((long long)id.n * K + id.k) * plane + at] : (T)1;
+    const T off_h = offset[((long long)id.n * 2 * GK + 2 * id.v) * plane + at];
+    const T off_w = offset[((long long)id.n * 2 * GK + 2 * id.v + 1) * plane + at];
+    m = mask ? mask[((long long)id.n * GK + id.v) * plane + at] : (T)1;
     const int ky = id.k / d.kw, kx = id.k - ky * d.kw;
     h = (T)(id.ho * d.sh - d.ph + ky * d.dh) + off_h;
     w = (T)(id.wo * d.sw - d.pw + kx * d.dw) + off_w;
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// forward gather: cols[(pixel * K + k) * C + c] = mask * bilinear(input[n, :, :, c], h, w)
-// V = channels per lane and load (4: float4, C % 4 == 0; 1: any C / double)
+// forward gather: cols[(pixel * K + k) * C + g * Cg + c] = mask * bilinear(input[n, :, :, g * Cg + c], h, w)
+// V = channels per lane and load (4: float4, Cg % 4 == 0; 1: any Cg / double)
 // ---------------------------------------------------------------------------------------------------------------------
 template <typename T, int V, int G>
 __global__ void __launch_bounds__(256) dcn_im2col_kernel(const T *__restrict__ input, const T *__restrict__ offset,
@@ -155,12 +165,14 @@ __global__ void __launch_bounds__(256) dcn_im2col_kernel(const T *__restrict__ i
     const int j = threadIdx.x % G;
     const int pp = (int)((blockIdx.x * blockDim.x + threadIdx.x) / G);
     if (pp >= d.Ho * d.Wo) return;
-    const DcnTapId id = dcn_tap_id(pp, n_base + (int)blockIdx.z, (int)blockIdx.y, d);
+    const int K = d.kh * d.kw, v = (int)blockIdx.y, grp = d.og > 1 ? v / K : 0, Cg = d.C / d.og;
+    DcnTapId id = dcn_tap_id(pp, n_base + (int)blockIdx.z, v - grp * K, d);
+    id.v = v;
     T h, w, m;
     dcn_sample_point(offset, mask, id, d, h, w, m);
     const DcnTap<T> t = dcn_tap(h, w, d.H, d.W);
-    const T *img = input + (long long)id.n * d.H * d.W * d.C;
-    T *out = cols + (id.pixel * (d.kh * d.kw) + id.k) * (long long)d.C;
+    const T *img = input + (long long)id.n * d.H * d.W * d.C + grp * Cg;
+    T *out = cols + (id.pixel * K + id.k) * (long long)d.C + grp * Cg;
     const T f0 = m * t.w[0], f1 = m * t.w[1], f2 = m * t.w[2], f3 = m * t.w[3];
     if (V == 4) {
         const float4 *r0 = reinterpret_cast<const float4 *>(img + (long long)t.row[0] * d.C);
@@ -168,19 +180,19 @@ __global__ void __launch_bounds__(256) dcn_im2col_kernel(const T *__restrict__ i
         const float4 *r2 = reinterpret_cast<const float4 *>(img + (long long)t.row[2] * d.C);
         const float4 *r3 = reinterpret_cast<const float4 *>(img + (long long)t.row[3] * d.C);
         float4 *o = reinterpret_cast<float4 *>(out);
-        for (int c = j; c < d.C / 4; c += G) {
+        for (int c = j; c < Cg / 4; c += G) {
             const float4 a = __ldg(r0 + c), b = __ldg(r1 + c), e = __ldg(r2 + c), f = __ldg(r3 + c);
-            float4 v;
-            v.x = f0 * a.x + f1 * b.x + f2 * e.x + f3 * f.x;
-            v.y = f0 * a.y + f1 * b.y + f2 * e.y + f3 * f.y;
-            v.z = f0 * a.z + f1 * b.z + f2 * e.z + f3 * f.z;
-            v.w = f0 * a.w + f1 * b.w + f2 * e.w + f3 * f.w;
-            o[c] = v;
+            float4 s;
+            s.x = f0 * a.x + f1 * b.x + f2 * e.x + f3 * f.x;
+            s.y = f0 * a.y + f1 * b.y + f2 * e.y + f3 * f.y;
+            s.z = f0 * a.z + f1 * b.z + f2 * e.z + f3 * f.z;
+            s.w = f0 * a.w + f1 * b.w + f2 * e.w + f3 * f.w;
+            o[c] = s;
         }
     } else {
         const T *r0 = img + (long long)t.row[0] * d.C, *r1 = img + (long long)t.row[1] * d.C;
         const T *r2 = img + (long long)t.row[2] * d.C, *r3 = img + (long long)t.row[3] * d.C;
-        for (int c = j; c < d.C; c += G) out[c] = f0 * r0[c] + f1 * r1[c] + f2 * r2[c] + f3 * r3[c];
+        for (int c = j; c < Cg; c += G) out[c] = f0 * r0[c] + f1 * r1[c] + f2 * r2[c] + f3 * r3[c];
     }
 }
 
@@ -188,7 +200,8 @@ __device__ __forceinline__ void dcn_red_add(float *p, float v) { atomicAdd(p, v)
 __device__ __forceinline__ void dcn_red_add(double *p, double v) { atomicAdd(p, v); }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// backward: grad_input (scatter), grad_offset, grad_mask from grad_cols, one pass per tap
+// backward: grad_input (scatter), grad_offset, grad_mask from grad_cols, one pass per tap (the offset / mask gradients of
+// a tap are reduced over its group's Cg channels only)
 // ---------------------------------------------------------------------------------------------------------------------
 template <typename T, int V, int G, bool DET = false>
 __global__ void __launch_bounds__(256) dcn_col2im_kernel(const T *__restrict__ input, const T *__restrict__ offset,
@@ -201,18 +214,20 @@ __global__ void __launch_bounds__(256) dcn_col2im_kernel(const T *__restrict__ i
     int pp = (int)((blockIdx.x * blockDim.x + threadIdx.x) / G);
     const bool live = pp < d.Ho * d.Wo;
     if (!live) pp = d.Ho * d.Wo - 1;   // keep the whole warp in the shuffles below; results of dead groups are dropped
-    const DcnTapId id = dcn_tap_id(pp, n_base + (int)blockIdx.z, (int)blockIdx.y, d);
+    const int K = d.kh * d.kw, v = (int)blockIdx.y, grp = d.og > 1 ? v / K : 0, Cg = d.C / d.og;
+    DcnTapId id = dcn_tap_id(pp, n_base + (int)blockIdx.z, v - grp * K, d);
+    id.v = v;
     T h, w, m;
     dcn_sample_point(offset, mask, id, d, h, w, m);
     const DcnTap<T> t = dcn_tap(h, w, d.H, d.W);
-    const T *img = input + (long long)id.n * d.H * d.W * d.C;
-    T *gimg = grad_input ? grad_input + (long long)id.n * d.H * d.W * d.C : nullptr;
-    const T *gc = grad_cols + (id.pixel * (d.kh * d.kw) + id.k) * (long long)d.C;
+    const T *img = input + (long long)id.n * d.H * d.W * d.C + grp * Cg;
+    T *gimg = grad_input ? grad_input + (long long)id.n * d.H * d.W * d.C + grp * Cg : nullptr;
+    const T *gc = grad_cols + (id.pixel * K + id.k) * (long long)d.C + grp * Cg;
     const T f0 = m * t.w[0], f1 = m * t.w[1], f2 = m * t.w[2], f3 = m * t.w[3];
     long long *gacc = nullptr;
     float det_sh = 0.f;
     if constexpr (DET) {
-        gacc = det.acc + (long long)id.n * d.H * d.W * d.C;
+        gacc = det.acc + (long long)id.n * d.H * d.W * d.C + grp * Cg;
         det_sh = dcn_det_scale(det, kDcnDetFactorsCol2im);
     }
     T A0 = 0, A1 = 0, A2 = 0, A3 = 0;
@@ -222,7 +237,7 @@ __global__ void __launch_bounds__(256) dcn_col2im_kernel(const T *__restrict__ i
         const float4 *r2 = reinterpret_cast<const float4 *>(img + (long long)t.row[2] * d.C);
         const float4 *r3 = reinterpret_cast<const float4 *>(img + (long long)t.row[3] * d.C);
         const float4 *g4 = reinterpret_cast<const float4 *>(gc);
-        for (int c = j; c < d.C / 4; c += G) {
+        for (int c = j; c < Cg / 4; c += G) {
             const float4 g = __ldg(g4 + c);
             const float4 a = __ldg(r0 + c), b = __ldg(r1 + c), e = __ldg(r2 + c), f = __ldg(r3 + c);
             A0 += g.x * a.x + g.y * a.y + g.z * a.z + g.w * a.w;
@@ -248,7 +263,7 @@ __global__ void __launch_bounds__(256) dcn_col2im_kernel(const T *__restrict__ i
     } else {
         const T *r0 = img + (long long)t.row[0] * d.C, *r1 = img + (long long)t.row[1] * d.C;
         const T *r2 = img + (long long)t.row[2] * d.C, *r3 = img + (long long)t.row[3] * d.C;
-        for (int c = j; c < d.C; c += G) {
+        for (int c = j; c < Cg; c += G) {
             const T g = gc[c];
             A0 += g * r0[c];
             A1 += g * r1[c];
@@ -283,14 +298,14 @@ __global__ void __launch_bounds__(256) dcn_col2im_kernel(const T *__restrict__ i
         A1 = t.ok[1] ? A1 : (T)0;
         A2 = t.ok[2] ? A2 : (T)0;
         A3 = t.ok[3] ? A3 : (T)0;
-        const int K = d.kh * d.kw;
+        const int GK = d.og * K;
         const long long plane = (long long)d.Ho * d.Wo, at = (long long)id.ho * d.Wo + id.wo;
         const T val = t.hh * (t.hw * A0 + t.lw * A1) + t.lh * (t.hw * A2 + t.lw * A3);
         const T gh = t.hw * (A2 - A0) + t.lw * (A3 - A1);      // d/dh of the interpolated value
         const T gw = t.hh * (A1 - A0) + t.lh * (A3 - A2);      // d/dw
-        grad_offset[((long long)id.n * 2 * K + 2 * id.k) * plane + at] = t.inside ? m * gh : (T)0;
-        grad_offset[((long long)id.n * 2 * K + 2 * id.k + 1) * plane + at] = t.inside ? m * gw : (T)0;
-        if (grad_mask) grad_mask[((long long)id.n * K + id.k) * plane + at] = t.inside ? val : (T)0;
+        grad_offset[((long long)id.n * 2 * GK + 2 * v) * plane + at] = t.inside ? m * gh : (T)0;
+        grad_offset[((long long)id.n * 2 * GK + 2 * v + 1) * plane + at] = t.inside ? m * gw : (T)0;
+        if (grad_mask) grad_mask[((long long)id.n * GK + v) * plane + at] = t.inside ? val : (T)0;
     }
 }
 
@@ -305,14 +320,20 @@ __global__ void __launch_bounds__(256) dcn_col2im_kernel(const T *__restrict__ i
 // positions the partials are combined over the group with a reduce-scatter butterfly and each lane stores COUT/G
 // outputs.  HBM traffic = input + offsets + mask + output, once each.
 //
-// PACKED WEIGHTS (devis_dcn_pack_weight): wp[((k * nblk + b) * COUT + co) * G + jj] is a float4 holding
-// weight[co][(b*G + jj)*4 + 0..3][ky][kx] (zero beyond C), nblk = ceil(C / (4*G)).  For a fixed (k, b, co) the G lanes
-// of a group read 16*G contiguous bytes and all groups of a warp read the same bytes (one L1 wavefront, broadcast).
+// With offset groups the kernel positions become the G_off * K virtual positions v = g * K + k, each contracting its
+// group's Cg = C / G_off channels (Cg % 4 == 0).
+//
+// PACKED WEIGHTS (devis_dcn_pack_weight_og): wp[((v * nblk + b) * COUT + co) * G + jj], v = g * K + k, is a float4
+// holding weight[co][g*Cg + (b*G + jj)*4 + 0..3][ky][kx] (zero beyond the group's Cg channels), nblk = ceil(Cg / (4*G)):
+// the slabs follow the virtual positions in the order the kernels walk them (with G_off = 1, v = k).  For a fixed
+// (v, b, co) the G lanes of a group read 16*G contiguous bytes and all groups of a warp read the same bytes (one L1
+// wavefront, broadcast).
 // =====================================================================================================================
 __global__ void dcn_pack_weight_kernel(const float *__restrict__ w /* (Cout, C, kh, kw) */, float *__restrict__ wp,
-                                       int cout, int C, int K, int G, int nblk)
+                                       int cout, int C, int K, int G, int nblk, int og)
 {
-    const long long total = (long long)K * nblk * cout * G * 4;
+    const long long total = (long long)K * og * nblk * cout * G * 4;
+    const int Cg = C / og;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
         const int e = (int)(i & 3);
         long long r = i >> 2;
@@ -321,9 +342,10 @@ __global__ void dcn_pack_weight_kernel(const float *__restrict__ w /* (Cout, C, 
         const int co = (int)(r % cout);
         r /= cout;
         const int b = (int)(r % nblk);
-        const int k = (int)(r / nblk);
+        const int v = (int)(r / nblk);
+        const int g = v / K, k = v - g * K;
         const int c = (b * G + jj) * 4 + e;
-        wp[i] = c < C ? w[((long long)co * C + c) * K + k] : 0.f;
+        wp[i] = c < Cg ? w[((long long)co * C + g * Cg + c) * K + k] : 0.f;
     }
 }
 
@@ -405,11 +427,11 @@ __global__ void __launch_bounds__(256, 2) dcn_fused_fwd_kernel(const float *__re
     const DcnTile<G, PPG> tile(d, n_base);
     if (!tile.row_live) return;          // whole warp
     const int j = tile.j;
-    const int K = d.kh * d.kw, C4 = d.C / 4, nblk = (C4 + G - 1) / G;
+    const int K = d.kh * d.kw, GK = d.og * K, C4 = d.C / 4, Cg4 = C4 / d.og, nblk = (Cg4 + G - 1) / G;
     const long long plane = (long long)d.Ho * d.Wo;
     const float4 *img = reinterpret_cast<const float4 *>(input + (long long)tile.n * d.H * d.W * d.C);
-    const float *offset_n = offset + (long long)tile.n * 2 * K * plane;
-    const float *mask_n = mask ? mask + (long long)tile.n * K * plane : nullptr;
+    const float *offset_n = offset + (long long)tile.n * 2 * GK * plane;
+    const float *mask_n = mask ? mask + (long long)tile.n * GK * plane : nullptr;
     float acc[PPG][COUT];
 #pragma unroll
     for (int i = 0; i < PPG; ++i)
@@ -418,7 +440,8 @@ __global__ void __launch_bounds__(256, 2) dcn_fused_fwd_kernel(const float *__re
     DcnPoint nxt[PPG];
 #pragma unroll
     for (int i = 0; i < PPG; ++i) nxt[i] = dcn_load_point(offset_n, mask_n, 0, plane, tile.at[i]);
-    for (int k = 0; k < K; ++k) {
+    // virtual position v = grp * K + k: kernel position k of offset group grp, channel pieces [grp * Cg4, (grp + 1) * Cg4)
+    for (int v = 0, grp = 0, k = 0; v < GK; ++v) {
         const int ky = k / d.kw, kx = k - ky * d.kw;
         float fw[PPG][4];
         int row[PPG][4];
@@ -430,34 +453,35 @@ __global__ void __launch_bounds__(256, 2) dcn_fused_fwd_kernel(const float *__re
 #pragma unroll
             for (int q = 0; q < 4; ++q) {
                 fw[i][q] = nxt[i].m * t.w[q];
-                row[i][q] = t.row[q] * C4;
+                row[i][q] = t.row[q] * C4 + grp * Cg4;
             }
         }
-        if (k + 1 < K) {     // next position's offsets and mask: in flight while this one is gathered and contracted
+        if (v + 1 < GK) {    // next position's offsets and mask: in flight while this one is gathered and contracted
 #pragma unroll
-            for (int i = 0; i < PPG; ++i) nxt[i] = dcn_load_point(offset_n, mask_n, k + 1, plane, tile.at[i]);
+            for (int i = 0; i < PPG; ++i) nxt[i] = dcn_load_point(offset_n, mask_n, v + 1, plane, tile.at[i]);
         }
         for (int b = 0; b < nblk; ++b) {
             const int c = b * G + j;
-            if (c >= C4) break;
-            float4 v[PPG];
+            if (c >= Cg4) break;
+            float4 s[PPG];
 #pragma unroll
             for (int i = 0; i < PPG; ++i) {
                 const float4 a = __ldg(img + row[i][0] + c), bb = __ldg(img + row[i][1] + c), e = __ldg(img + row[i][2] + c), f = __ldg(img + row[i][3] + c);
-                v[i].x = fw[i][0] * a.x + fw[i][1] * bb.x + fw[i][2] * e.x + fw[i][3] * f.x;
-                v[i].y = fw[i][0] * a.y + fw[i][1] * bb.y + fw[i][2] * e.y + fw[i][3] * f.y;
-                v[i].z = fw[i][0] * a.z + fw[i][1] * bb.z + fw[i][2] * e.z + fw[i][3] * f.z;
-                v[i].w = fw[i][0] * a.w + fw[i][1] * bb.w + fw[i][2] * e.w + fw[i][3] * f.w;
+                s[i].x = fw[i][0] * a.x + fw[i][1] * bb.x + fw[i][2] * e.x + fw[i][3] * f.x;
+                s[i].y = fw[i][0] * a.y + fw[i][1] * bb.y + fw[i][2] * e.y + fw[i][3] * f.y;
+                s[i].z = fw[i][0] * a.z + fw[i][1] * bb.z + fw[i][2] * e.z + fw[i][3] * f.z;
+                s[i].w = fw[i][0] * a.w + fw[i][1] * bb.w + fw[i][2] * e.w + fw[i][3] * f.w;
             }
-            const float4 *wk = wp + ((long long)(k * nblk + b) * COUT) * G + j;
+            const float4 *wk = wp + ((long long)(v * nblk + b) * COUT) * G + j;
 #pragma unroll
             for (int co = 0; co < COUT; ++co) {
                 const float4 w4 = __ldg(wk + co * G);
 #pragma unroll
                 for (int i = 0; i < PPG; ++i)
-                    acc[i][co] = fmaf(v[i].x, w4.x, fmaf(v[i].y, w4.y, fmaf(v[i].z, w4.z, fmaf(v[i].w, w4.w, acc[i][co]))));
+                    acc[i][co] = fmaf(s[i].x, w4.x, fmaf(s[i].y, w4.y, fmaf(s[i].z, w4.z, fmaf(s[i].w, w4.w, acc[i][co]))));
             }
         }
+        if (++k == K) k = 0, ++grp;
     }
 #pragma unroll
     for (int i = 0; i < PPG; ++i) {
@@ -491,7 +515,7 @@ __global__ void __launch_bounds__(256, 2) dcn_fused_bwd_kernel(const float *__re
     const DcnTile<G, PPG> tile(d, n_base);
     if (!tile.row_live) return;
     const int j = tile.j;
-    const int K = d.kh * d.kw, C4 = d.C / 4, nblk = (C4 + G - 1) / G;
+    const int K = d.kh * d.kw, GK = d.og * K, C4 = d.C / 4, Cg4 = C4 / d.og, nblk = (Cg4 + G - 1) / G;
     const long long plane = (long long)d.Ho * d.Wo;
     const float4 *img = reinterpret_cast<const float4 *>(input + (long long)tile.n * d.H * d.W * d.C);
     float *gimg = grad_input ? grad_input + (long long)tile.n * d.H * d.W * d.C : nullptr;
@@ -501,10 +525,10 @@ __global__ void __launch_bounds__(256, 2) dcn_fused_bwd_kernel(const float *__re
         gacc = det.acc + (long long)tile.n * d.H * d.W * d.C;
         det_sh = dcn_det_scale(det, kDcnDetFactorsFused);
     }
-    const float *offset_n = offset + (long long)tile.n * 2 * K * plane;
-    const float *mask_n = mask ? mask + (long long)tile.n * K * plane : nullptr;
-    float *goff_n = grad_offset + (long long)tile.n * 2 * K * plane;
-    float *gmask_n = grad_mask ? grad_mask + (long long)tile.n * K * plane : nullptr;
+    const float *offset_n = offset + (long long)tile.n * 2 * GK * plane;
+    const float *mask_n = mask ? mask + (long long)tile.n * GK * plane : nullptr;
+    float *goff_n = grad_offset + (long long)tile.n * 2 * GK * plane;
+    float *gmask_n = grad_mask ? grad_mask + (long long)tile.n * GK * plane : nullptr;
     float g[PPG][COUT];
 #pragma unroll
     for (int i = 0; i < PPG; ++i) {
@@ -515,8 +539,8 @@ __global__ void __launch_bounds__(256, 2) dcn_fused_bwd_kernel(const float *__re
     DcnPoint nxt[PPG];
 #pragma unroll
     for (int i = 0; i < PPG; ++i) nxt[i] = dcn_load_point(offset_n, mask_n, 0, plane, tile.at[i]);
-    for (int k = 0; k < K; ++k) {
-        const int ky = k / d.kw, kx = k - ky * d.kw;
+    for (int v = 0, grp = 0, k = 0; v < GK; ++v) {      // virtual positions, as in dcn_fused_fwd_kernel
+        const int ky = k / d.kw, kx = k - ky * d.kw, cb = grp * Cg4;
         DcnTap<float> t[PPG];
         float fw[PPG][4], m[PPG], A[PPG][4];
 #pragma unroll
@@ -528,19 +552,20 @@ __global__ void __launch_bounds__(256, 2) dcn_fused_bwd_kernel(const float *__re
 #pragma unroll
             for (int q = 0; q < 4; ++q) fw[i][q] = m[i] * t[i].w[q], A[i][q] = 0.f;
         }
-        if (k + 1 < K) {
+        if (v + 1 < GK) {
 #pragma unroll
-            for (int i = 0; i < PPG; ++i) nxt[i] = dcn_load_point(offset_n, mask_n, k + 1, plane, tile.at[i]);
+            for (int i = 0; i < PPG; ++i) nxt[i] = dcn_load_point(offset_n, mask_n, v + 1, plane, tile.at[i]);
         }
         for (int b = 0; b < nblk; ++b) {
-            const int c = b * G + j;
-            if (c >= C4) break;
+            const int cl = b * G + j;
+            if (cl >= Cg4) break;
+            const int c = cb + cl;
             float4 corner[PPG][4];
 #pragma unroll
             for (int i = 0; i < PPG; ++i)
 #pragma unroll
                 for (int q = 0; q < 4; ++q) corner[i][q] = __ldg(img + (long long)t[i].row[q] * C4 + c);
-            const float4 *wk = wp + ((long long)(k * nblk + b) * COUT) * G + j;
+            const float4 *wk = wp + ((long long)(v * nblk + b) * COUT) * G + j;
             float4 gc[PPG];
 #pragma unroll
             for (int i = 0; i < PPG; ++i) gc[i] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -583,11 +608,12 @@ __global__ void __launch_bounds__(256, 2) dcn_fused_bwd_kernel(const float *__re
                 const float val = t[i].hh * (t[i].hw * A0 + t[i].lw * A1) + t[i].lh * (t[i].hw * A2 + t[i].lw * A3);
                 const float gh = t[i].hw * (A2 - A0) + t[i].lw * (A3 - A1);
                 const float gw = t[i].hh * (A1 - A0) + t[i].lh * (A3 - A2);
-                goff_n[(2 * k) * plane + tile.at[i]] = t[i].inside ? m[i] * gh : 0.f;
-                goff_n[(2 * k + 1) * plane + tile.at[i]] = t[i].inside ? m[i] * gw : 0.f;
-                if (gmask_n) gmask_n[k * plane + tile.at[i]] = t[i].inside ? val : 0.f;
+                goff_n[(2 * v) * plane + tile.at[i]] = t[i].inside ? m[i] * gh : 0.f;
+                goff_n[(2 * v + 1) * plane + tile.at[i]] = t[i].inside ? m[i] * gw : 0.f;
+                if (gmask_n) gmask_n[v * plane + tile.at[i]] = t[i].inside ? val : 0.f;
             }
         }
+        if (++k == K) k = 0, ++grp;
     }
 }
 

@@ -14,7 +14,7 @@ int check_dims(const DcnDims &d, int dtype)
 {
     if (dtype != DEVIS_MSDA_F32 && dtype != DEVIS_MSDA_F64) return DEVIS_MSDA_ERR_BAD_DTYPE;
     if (d.N < 0 || d.H <= 0 || d.W <= 0 || d.C <= 0 || d.Ho < 0 || d.Wo < 0 || d.kh <= 0 || d.kw <= 0 || d.sh <= 0 ||
-        d.sw <= 0 || d.ph < 0 || d.pw < 0 || d.dh <= 0 || d.dw <= 0)
+        d.sw <= 0 || d.ph < 0 || d.pw < 0 || d.dh <= 0 || d.dw <= 0 || d.og < 1 || d.C % d.og)
         return DEVIS_MSDA_ERR_BAD_SHAPE;
     if ((long long)d.H * d.W >= (1LL << 31)) return DEVIS_MSDA_ERR_TOO_LARGE;
     return DEVIS_MSDA_OK;
@@ -38,7 +38,8 @@ int check_det(const DcnDims &d, int dtype, const void *workspace, size_t workspa
     return DEVIS_MSDA_OK;
 }
 
-// zero the accumulators and the bound factors; factor 0 = max|grad| (n_grad floats), factor 1 = max|mask| (1 without one)
+// zero the accumulators and the bound factors; factor 0 = max|grad| (n_grad floats), factor 1 = max|mask| (1 without one;
+// N * og * kh * kw * Ho * Wo elements)
 int det_begin(void *workspace, const DcnDims &d, const void *grad, size_t n_grad, const void *mask, cudaStream_t st,
               DetScale &det, unsigned *&slots)
 {
@@ -52,7 +53,7 @@ int det_begin(void *workspace, const DcnDims &d, const void *grad, size_t n_grad
     absmax_kernel<false><<<blocks, 256, 0, st>>>(grad, n_grad, slots);
     int rc = devis_capi_check_launch(DEVIS_MSDA_KERNEL_AUX);
     if (rc) return rc;
-    if (mask) absmax_kernel<false><<<blocks, 256, 0, st>>>(mask, (size_t)d.N * d.kh * d.kw * d.Ho * d.Wo, slots + 1);
+    if (mask) absmax_kernel<false><<<blocks, 256, 0, st>>>(mask, (size_t)d.N * d.og * d.kh * d.kw * d.Ho * d.Wo, slots + 1);
     else set_word_kernel<<<1, 1, 0, st>>>(slots + 1, 0x3f800000u);
     return devis_capi_check_launch(DEVIS_MSDA_KERNEL_AUX);
 }
@@ -65,9 +66,16 @@ int det_finish(const DetScale &det, const DcnDims &d, void *grad_input, int n_fa
     return devis_capi_check_launch(DEVIS_MSDA_KERNEL_AUX);
 }
 
-// lanes per tap: a group covers its channels in 16-byte pieces; 8 lanes = one 128-byte line per corner row.
-// Grid: x = output plane (wo fastest), y = kernel position, z = batch item (in slices of at most 65535).
+// lanes per tap: a group covers its offset group's Cg = C / og channels in 16-byte pieces; 8 lanes = one 128-byte line
+// per corner row.  Grid: x = output plane (wo fastest), y = virtual kernel position g * K + k, z = batch item (in slices
+// of at most 65535).
 constexpr int kMaxGridZ = 65535;
+
+// the grid's y dimension of the gather / scatter kernels, checked before any CUDA call
+int check_grid_y(const DcnDims &d)
+{
+    return (long long)d.og * d.kh * d.kw > 65535 ? DEVIS_MSDA_ERR_TOO_LARGE : DEVIS_MSDA_OK;
+}
 
 template <class F4, class F8, class S8, class S32>
 int dispatch(const DcnDims &d, int dtype, F4 f4, F8 f8, S8 s8, S32 s32)
@@ -75,12 +83,13 @@ int dispatch(const DcnDims &d, int dtype, F4 f4, F8 f8, S8 s8, S32 s32)
     const long long plane = (long long)d.Ho * d.Wo;
     if (d.N == 0 || plane == 0) return DEVIS_MSDA_OK;
     int G;
-    const bool vec = dtype == DEVIS_MSDA_F32 && d.C % 4 == 0;
-    if (vec) G = d.C / 4 >= 8 ? 8 : 4;
-    else G = d.C >= 32 ? 32 : 8;
-    if (plane * G + 255 >= (1LL << 31) || d.kh * d.kw > 65535) return DEVIS_MSDA_ERR_TOO_LARGE;
+    const int Cg = d.C / d.og;
+    const bool vec = dtype == DEVIS_MSDA_F32 && Cg % 4 == 0;
+    if (vec) G = Cg / 4 >= 8 ? 8 : 4;
+    else G = Cg >= 32 ? 32 : 8;
+    if (plane * G + 255 >= (1LL << 31)) return DEVIS_MSDA_ERR_TOO_LARGE;     // grid y: check_grid_y, by the callers
     for (int n0 = 0; n0 < d.N; n0 += kMaxGridZ) {
-        const dim3 grid((unsigned)((plane * G + 255) / 256), (unsigned)(d.kh * d.kw),
+        const dim3 grid((unsigned)((plane * G + 255) / 256), (unsigned)(d.og * d.kh * d.kw),
                         (unsigned)(d.N - n0 < kMaxGridZ ? d.N - n0 : kMaxGridZ));
         if (vec) {
             if (G == 8) f8(grid, n0);
@@ -103,9 +112,19 @@ int devis_dcn_im2col(const void *input, const void *offset, const void *mask, vo
                      int width, int channels, int out_h, int out_w, int kernel_h, int kernel_w, int stride_h,
                      int stride_w, int pad_h, int pad_w, int dil_h, int dil_w, int dtype, void *stream)
 {
+    return devis_dcn_im2col_og(input, offset, mask, cols, batch, height, width, channels, out_h, out_w, kernel_h,
+                               kernel_w, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w, 1, dtype, stream);
+}
+
+int devis_dcn_im2col_og(const void *input, const void *offset, const void *mask, void *cols, int batch, int height,
+                        int width, int channels, int out_h, int out_w, int kernel_h, int kernel_w, int stride_h,
+                        int stride_w, int pad_h, int pad_w, int dil_h, int dil_w, int offset_groups, int dtype,
+                        void *stream)
+{
     const DcnDims d{batch, height, width, channels, out_h, out_w, kernel_h, kernel_w,
-                    stride_h, stride_w, pad_h, pad_w, dil_h, dil_w};
-    const int rc = check_dims(d, dtype);
+                    stride_h, stride_w, pad_h, pad_w, dil_h, dil_w, offset_groups};
+    int rc = check_dims(d, dtype);
+    if (!rc) rc = check_grid_y(d);
     if (rc) return rc;
     const long long n_taps = (long long)batch * out_h * out_w * kernel_h * kernel_w;
     if (n_taps > 0 && (!input || !offset || !cols)) return DEVIS_MSDA_ERR_NULL_POINTER;
@@ -147,9 +166,21 @@ int devis_dcn_col2im_ex(const void *input, const void *offset, const void *mask,
                         int out_w, int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w, int dil_h,
                         int dil_w, int dtype, unsigned flags, void *workspace, size_t workspace_bytes, void *stream)
 {
+    return devis_dcn_col2im_og(input, offset, mask, grad_cols, grad_input, grad_offset, grad_mask, batch, height, width,
+                               channels, out_h, out_w, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w,
+                               1, dtype, flags, workspace, workspace_bytes, stream);
+}
+
+int devis_dcn_col2im_og(const void *input, const void *offset, const void *mask, const void *grad_cols, void *grad_input,
+                        void *grad_offset, void *grad_mask, int batch, int height, int width, int channels, int out_h,
+                        int out_w, int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w, int dil_h,
+                        int dil_w, int offset_groups, int dtype, unsigned flags, void *workspace, size_t workspace_bytes,
+                        void *stream)
+{
     const DcnDims d{batch, height, width, channels, out_h, out_w, kernel_h, kernel_w,
-                    stride_h, stride_w, pad_h, pad_w, dil_h, dil_w};
+                    stride_h, stride_w, pad_h, pad_w, dil_h, dil_w, offset_groups};
     int rc = check_dims(d, dtype);
+    if (!rc) rc = check_grid_y(d);
     if (rc) return rc;
     const bool det_flag = (flags & DEVIS_MSDA_FLAG_DETERMINISTIC) && grad_input;
     if (det_flag) {
@@ -220,19 +251,22 @@ struct FusedPlan {
     bool any() const { return lanes_fwd || lanes_bwd || constant; }
 };
 
-FusedPlan fused_plan(int C, int cout, int kh, int kw, int dtype)
+// og offset groups: the lane-group kernels contract each group's Cg = C / og channels (Cg % 4 == 0); the constant-bank
+// forward serves og = 1 only (its weight chunking works per kernel position)
+FusedPlan fused_plan(int C, int cout, int kh, int kw, int dtype, int og)
 {
     FusedPlan p;
-    if (dtype != DEVIS_MSDA_F32 || C <= 0 || C % 4 || kh <= 0 || kw <= 0 || cout <= 0) return p;
+    if (dtype != DEVIS_MSDA_F32 || og < 1 || C <= 0 || C % og || (C / og) % 4 || kh <= 0 || kw <= 0 || cout <= 0) return p;
     const long long K = (long long)kh * kw;
+    const int Cg = C / og;
     const bool small = cout == 1 || cout == 2 || cout == 4 || cout == 8 || cout == 16;
-    p.G = C / 4 > 4 ? 8 : 4;
+    p.G = Cg / 4 > 4 ? 8 : 4;
     const bool c_served = C == 16 || C == 32 || C == 40 || C == 64 || C == 72;   // dcn_fusedc_fwd_kernel<C, CT> instantiations
-    p.constant = c_served && cout % 16 == 0 && cout <= 64;
+    p.constant = og == 1 && c_served && cout % 16 == 0 && cout <= 64;
     p.CT = cout % 32 == 0 ? 32 : 16;
     p.lanes_bwd = small;
     p.lanes_fwd = small && !p.constant;
-    if (p.lanes_fwd || p.lanes_bwd) p.lanes_elems = (size_t)K * ((C / 4 + p.G - 1) / p.G) * cout * p.G * 4;
+    if (p.lanes_fwd || p.lanes_bwd) p.lanes_elems = (size_t)K * og * ((Cg / 4 + p.G - 1) / p.G) * cout * p.G * 4;
     if (p.constant) p.const_elems = (size_t)K * C * cout;
     return p;
 }
@@ -267,30 +301,48 @@ extern "C" {
 
 int devis_dcn_fused_form(int channels, int out_channels, int kernel_h, int kernel_w, int dtype)
 {
-    const FusedPlan p = fused_plan(channels, out_channels, kernel_h, kernel_w, dtype);
+    return devis_dcn_fused_form_og(channels, out_channels, kernel_h, kernel_w, 1, dtype);
+}
+
+int devis_dcn_fused_form_og(int channels, int out_channels, int kernel_h, int kernel_w, int offset_groups, int dtype)
+{
+    const FusedPlan p = fused_plan(channels, out_channels, kernel_h, kernel_w, dtype, offset_groups);
     return ((p.lanes_fwd || p.constant) ? 1 : 0) | (p.lanes_bwd ? 2 : 0);
 }
 
 size_t devis_dcn_packed_weight_elems(int channels, int out_channels, int kernel_h, int kernel_w)
 {
-    const FusedPlan p = fused_plan(channels, out_channels, kernel_h, kernel_w, DEVIS_MSDA_F32);
+    return devis_dcn_packed_weight_elems_og(channels, out_channels, kernel_h, kernel_w, 1);
+}
+
+size_t devis_dcn_packed_weight_elems_og(int channels, int out_channels, int kernel_h, int kernel_w, int offset_groups)
+{
+    const FusedPlan p = fused_plan(channels, out_channels, kernel_h, kernel_w, DEVIS_MSDA_F32, offset_groups);
     return p.lanes_elems + p.const_elems;
 }
 
 int devis_dcn_pack_weight(const void *weight, void *packed, int channels, int out_channels, int kernel_h, int kernel_w,
                           void *stream)
 {
-    if (kernel_h <= 0 || kernel_w <= 0 || channels <= 0 || out_channels <= 0) return DEVIS_MSDA_ERR_BAD_SHAPE;
-    const FusedPlan p = fused_plan(channels, out_channels, kernel_h, kernel_w, DEVIS_MSDA_F32);
+    return devis_dcn_pack_weight_og(weight, packed, channels, out_channels, kernel_h, kernel_w, 1, stream);
+}
+
+int devis_dcn_pack_weight_og(const void *weight, void *packed, int channels, int out_channels, int kernel_h, int kernel_w,
+                             int offset_groups, void *stream)
+{
+    if (kernel_h <= 0 || kernel_w <= 0 || channels <= 0 || out_channels <= 0 || offset_groups < 1 ||
+        channels % offset_groups)
+        return DEVIS_MSDA_ERR_BAD_SHAPE;
+    const FusedPlan p = fused_plan(channels, out_channels, kernel_h, kernel_w, DEVIS_MSDA_F32, offset_groups);
     if (!p.any()) return DEVIS_MSDA_ERR_UNSUPPORTED;
     if (!weight || !packed) return DEVIS_MSDA_ERR_NULL_POINTER;
     const int K = kernel_h * kernel_w;
     cudaStream_t st = (cudaStream_t)stream;
     if (p.lanes_elems) {
-        const int nblk = (channels / 4 + p.G - 1) / p.G;
+        const int nblk = (channels / offset_groups / 4 + p.G - 1) / p.G;
         const unsigned blocks = (unsigned)((p.lanes_elems + 255) / 256 > 1184 ? 1184 : (p.lanes_elems + 255) / 256);
         dcn_pack_weight_kernel<<<blocks, 256, 0, st>>>((const float *)weight, (float *)packed, out_channels, channels, K,
-                                                       p.G, nblk);
+                                                       p.G, nblk, offset_groups);
         const int rc = devis_capi_check_launch(DEVIS_MSDA_KERNEL_DCN);
         if (rc) return rc;
     }
@@ -327,11 +379,21 @@ int devis_dcn_fused_forward(const void *input, const void *offset, const void *m
                             int out_w, int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w,
                             int dil_h, int dil_w, int out_channels, void *stream)
 {
+    return devis_dcn_fused_forward_og(input, offset, mask, packed_weight, bias, out, batch, height, width, channels, out_h,
+                                      out_w, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w, 1,
+                                      out_channels, stream);
+}
+
+int devis_dcn_fused_forward_og(const void *input, const void *offset, const void *mask, const void *packed_weight,
+                               const void *bias, void *out, int batch, int height, int width, int channels, int out_h,
+                               int out_w, int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w,
+                               int dil_h, int dil_w, int offset_groups, int out_channels, void *stream)
+{
     const DcnDims d{batch, height, width, channels, out_h, out_w, kernel_h, kernel_w,
-                    stride_h, stride_w, pad_h, pad_w, dil_h, dil_w};
+                    stride_h, stride_w, pad_h, pad_w, dil_h, dil_w, offset_groups};
     const int rc = check_dims(d, DEVIS_MSDA_F32);
     if (rc) return rc;
-    const FusedPlan plan = fused_plan(channels, out_channels, kernel_h, kernel_w, DEVIS_MSDA_F32);
+    const FusedPlan plan = fused_plan(channels, out_channels, kernel_h, kernel_w, DEVIS_MSDA_F32, offset_groups);
     if (!plan.lanes_fwd && !plan.constant) return DEVIS_MSDA_ERR_UNSUPPORTED;
     const long long n_pixels = (long long)batch * out_h * out_w;
     if (n_pixels == 0) return DEVIS_MSDA_OK;
@@ -414,9 +476,21 @@ int devis_dcn_fused_backward(const void *input, const void *offset, const void *
                              int stride_h, int stride_w, int pad_h, int pad_w, int dil_h, int dil_w, int out_channels,
                              void *stream)
 {
-    return devis_dcn_fused_backward_ex(input, offset, mask, packed_weight, grad_out, grad_input, grad_offset, grad_mask,
+    return devis_dcn_fused_backward_og(input, offset, mask, packed_weight, grad_out, grad_input, grad_offset, grad_mask,
                                        batch, height, width, channels, out_h, out_w, kernel_h, kernel_w, stride_h, stride_w,
-                                       pad_h, pad_w, dil_h, dil_w, out_channels, 0u, nullptr, 0, stream);
+                                       pad_h, pad_w, dil_h, dil_w, 1, out_channels, 0u, nullptr, 0, stream);
+}
+
+int devis_dcn_fused_backward_ex(const void *input, const void *offset, const void *mask, const void *packed_weight,
+                                const void *grad_out, void *grad_input, void *grad_offset, void *grad_mask, int batch,
+                                int height, int width, int channels, int out_h, int out_w, int kernel_h, int kernel_w,
+                                int stride_h, int stride_w, int pad_h, int pad_w, int dil_h, int dil_w, int out_channels,
+                                unsigned flags, void *workspace, size_t workspace_bytes, void *stream)
+{
+    return devis_dcn_fused_backward_og(input, offset, mask, packed_weight, grad_out, grad_input, grad_offset, grad_mask,
+                                       batch, height, width, channels, out_h, out_w, kernel_h, kernel_w, stride_h, stride_w,
+                                       pad_h, pad_w, dil_h, dil_w, 1, out_channels, flags, workspace, workspace_bytes,
+                                       stream);
 }
 
 }  // extern "C"
@@ -427,17 +501,17 @@ constexpr auto dcn_fused_bwd_det_kernel = dcn_fused_bwd_kernel<COUT, G, PPG, tru
 
 extern "C" {
 
-int devis_dcn_fused_backward_ex(const void *input, const void *offset, const void *mask, const void *packed_weight,
+int devis_dcn_fused_backward_og(const void *input, const void *offset, const void *mask, const void *packed_weight,
                                 const void *grad_out, void *grad_input, void *grad_offset, void *grad_mask, int batch,
                                 int height, int width, int channels, int out_h, int out_w, int kernel_h, int kernel_w,
-                                int stride_h, int stride_w, int pad_h, int pad_w, int dil_h, int dil_w, int out_channels,
-                                unsigned flags, void *workspace, size_t workspace_bytes, void *stream)
+                                int stride_h, int stride_w, int pad_h, int pad_w, int dil_h, int dil_w, int offset_groups,
+                                int out_channels, unsigned flags, void *workspace, size_t workspace_bytes, void *stream)
 {
     const DcnDims d{batch, height, width, channels, out_h, out_w, kernel_h, kernel_w,
-                    stride_h, stride_w, pad_h, pad_w, dil_h, dil_w};
+                    stride_h, stride_w, pad_h, pad_w, dil_h, dil_w, offset_groups};
     int rc = check_dims(d, DEVIS_MSDA_F32);
     if (rc) return rc;
-    const FusedPlan plan = fused_plan(channels, out_channels, kernel_h, kernel_w, DEVIS_MSDA_F32);
+    const FusedPlan plan = fused_plan(channels, out_channels, kernel_h, kernel_w, DEVIS_MSDA_F32, offset_groups);
     if (!plan.lanes_bwd) return DEVIS_MSDA_ERR_UNSUPPORTED;
     const bool det_flag = (flags & DEVIS_MSDA_FLAG_DETERMINISTIC) && grad_input;
     if (det_flag) {

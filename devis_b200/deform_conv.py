@@ -8,7 +8,9 @@ ModulatedDeformableConv2d.forward (src/models/deformable_segmentation.py:262-267
                        bilinear(input[n, ci], y*stride - pad + ky*dil + offset[n, 2k, y, x],
                                                x*stride - pad + kx*dil + offset[n, 2k+1, y, x])
 
-with zero padding.  Here the gather (and, backward, the scatter plus the offset / mask gradients) are the hand-written
+with zero padding.  With G offset groups (``offset`` of 2 * G * kh * kw channels, ``mask`` of G * kh * kw) input channel
+ci belongs to group g = ci // (Cin / G), and its samples use ``offset[n, 2 * (g * kh * kw + k) (+1)]`` and
+``mask[n, g * kh * kw + k]``.  Here the gather (and, backward, the scatter plus the offset / mask gradients) are the hand-written
 sm_100a kernels behind ``devis_dcn_im2col`` / ``devis_dcn_col2im`` (include/devis_deform_conv.h,
 devis_b200/csrc/deform_conv.cuh); the contractions with ``weight`` are cuBLAS GEMMs, as in torchvision (at::addmm).
 The input is read channels-last: pass a ``torch.channels_last`` tensor to avoid the layout copy; the result is returned
@@ -21,10 +23,13 @@ Two forms (both hand-written kernels of this library, chosen per layer by ``devi
               take the grad_cols GEMM + scatter kernel) + the weight gradient from columns recomputed in bounded chunks,
               so nothing of column size is kept between forward and backward;
   * im2col -- everything else: column matrix + cuBLAS GEMM, as torchvision does.
-``set_fused(False)`` forces the im2col form (A/B tests).
+``set_fused(False)`` forces the im2col form (A/B tests).  The wide layers' forward runs on the tensor cores
+(IGemmDeformConv2dFunction) and the narrow layers' weight gradient in one kernel (devis_dcn_weight_grad); both serve one
+offset group only, so with G > 1 those layers take the im2col form and the weight gradient takes the GEMM on recomputed
+columns.  The lane-group fused kernels serve G > 1 when (Cin / G) % 4 == 0 (devis_dcn_fused_form_og).
 
-Supported: groups == 1 and offset_groups == 1 (everything DeVIS uses), float32 / float64 (half and bfloat16 are
-computed in float32 like torchvision's autocast wrapper does), CUDA only -- there is no CPU fallback.
+Supported: groups == 1, any offset_groups, float32 / float64 (half and bfloat16 are computed in float32 like
+torchvision's autocast wrapper does), CUDA only -- there is no CPU fallback.
 """
 
 import warnings
@@ -122,14 +127,18 @@ def set_fused(enabled):
     return old
 
 
-def _fused_form(c, cout, kh, kw, dtype):
-    """bit 0: fused forward kernel serves the layer, bit 1: fused data-backward kernel does (devis_dcn_fused_form)"""
+def _fused_form(c, cout, kh, kw, dtype, offset_groups=1):
+    """bit 0: fused forward kernel serves the layer, bit 1: fused data-backward kernel does (devis_dcn_fused_form_og)"""
     if not _FUSED or dtype != torch.float32:
         return 0
-    return int(_lib.load().devis_dcn_fused_form(c, cout, kh, kw, _lib.F32))
+    return int(_lib.load().devis_dcn_fused_form_og(c, cout, kh, kw, offset_groups, _lib.F32))
 
 
-def _packed_weight(weight):
+def _offset_groups(offset, kh, kw):
+    return offset.shape[1] // (2 * kh * kw)
+
+
+def _packed_weight(weight, offset_groups=1):
     """weight (Cout, Cin, kh, kw) in the layout the fused kernels read.  Repacked on EVERY call: one small kernel over
     <= 100 KB for the layers the fused form serves.  (Round 1 cached the packed copy per tensor object and ``_version``;
     writes through ``Parameter.data`` -- ``nn.Module.to()``, EMA / weight-swap code -- do not bump ``_version``, so the
@@ -138,9 +147,11 @@ def _packed_weight(weight):
     lib = _lib.load()
     w = weight.detach()
     w = w if w.is_contiguous() else w.contiguous()
-    packed = torch.empty(int(lib.devis_dcn_packed_weight_elems(c, cout, kh, kw)), dtype=torch.float32, device=weight.device)
+    packed = torch.empty(int(lib.devis_dcn_packed_weight_elems_og(c, cout, kh, kw, offset_groups)), dtype=torch.float32,
+                         device=weight.device)
     with torch.cuda.device(weight.device):
-        _lib.check(lib.devis_dcn_pack_weight(_ptr(w), _ptr(packed), c, cout, kh, kw, torch.cuda.current_stream().cuda_stream))
+        _lib.check(lib.devis_dcn_pack_weight_og(_ptr(w), _ptr(packed), c, cout, kh, kw, offset_groups,
+                                                torch.cuda.current_stream().cuda_stream))
     return packed
 
 
@@ -160,15 +171,16 @@ class FusedDeformConv2dFunction(Function):
             mask = mask if mask.is_contiguous() else mask.contiguous()
         if bias is not None:
             bias = bias if bias.is_contiguous() else bias.contiguous()
-        packed = _packed_weight(weight)
+        og = _offset_groups(offset, kh, kw)
+        packed = _packed_weight(weight) if og == 1 else _packed_weight(weight, og)   # G = 1: the hook's original signature
         out = torch.empty((n, ho, wo, cout), dtype=input.dtype, device=input.device)
         dims = (n, h, w, c, ho, wo, kh, kw, sh, sw, ph, pw, dh, dw)
         with torch.cuda.device(input.device):
-            _lib.check(_lib.load().devis_dcn_fused_forward(_ptr(x), _ptr(offset), _ptr(mask), _ptr(packed), _ptr(bias),
-                                                           _ptr(out), *dims, cout,
-                                                           torch.cuda.current_stream().cuda_stream))
-        ctx.dims, ctx.cout, ctx.has_bias = dims, cout, bias is not None
-        ctx.form = _fused_form(c, cout, kh, kw, input.dtype)
+            _lib.check(_lib.load().devis_dcn_fused_forward_og(_ptr(x), _ptr(offset), _ptr(mask), _ptr(packed), _ptr(bias),
+                                                              _ptr(out), *dims, og, cout,
+                                                              torch.cuda.current_stream().cuda_stream))
+        ctx.dims, ctx.og, ctx.cout, ctx.has_bias = dims, og, cout, bias is not None
+        ctx.form = _fused_form(c, cout, kh, kw, input.dtype, og)
         ctx.weight = weight.detach() if not ctx.form & 2 else None    # only the GEMM route of the backward reads it
         ctx.save_for_backward(x, offset, mask, packed)
         return out.permute(0, 3, 1, 2)
@@ -178,7 +190,7 @@ class FusedDeformConv2dFunction(Function):
     def backward(ctx, grad_out):
         x, offset, mask, packed = ctx.saved_tensors
         n, h, w, c, ho, wo, kh, kw = ctx.dims[:8]
-        cout, k = ctx.cout, kh * kw
+        cout, k, og = ctx.cout, kh * kw, ctx.og
         g = grad_out.permute(0, 2, 3, 1)
         g = g if g.is_contiguous() else g.contiguous()                    # (N, Ho, Wo, Cout)
         need_in, need_off, need_w, need_b, need_m = ctx.needs_input_grad[:5]
@@ -196,10 +208,10 @@ class FusedDeformConv2dFunction(Function):
                     ws, ws_bytes = _workspace(lib, per, h, w, c, flags, x.device)
                     for n0 in range(0, n, per):
                         n1 = min(n, n0 + per)
-                        _lib.check(lib.devis_dcn_fused_backward_ex(
+                        _lib.check(lib.devis_dcn_fused_backward_og(
                             _ptr(x[n0:n1]), _ptr(offset[n0:n1]), _ptr(mask[n0:n1]) if mask is not None else None,
                             _ptr(packed), _ptr(g[n0:n1]), _ptr(gx[n0:n1]) if need_in else None, _ptr(grad_off[n0:n1]),
-                            _ptr(grad_m[n0:n1]) if mask is not None else None, n1 - n0, *ctx.dims[1:], cout, flags,
+                            _ptr(grad_m[n0:n1]) if mask is not None else None, n1 - n0, *ctx.dims[1:], og, cout, flags,
                             _ptr(ws), ws_bytes, stream))
                 else:
                     # wider layers: column gradient by GEMM (a bounded chunk of the batch at a time) + scatter kernel
@@ -210,18 +222,18 @@ class FusedDeformConv2dFunction(Function):
                     for n0 in range(0, n, per):
                         n1 = min(n, n0 + per)
                         grad_cols = g2[n0 * ho * wo:n1 * ho * wo] @ w2
-                        _lib.check(lib.devis_dcn_col2im_ex(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
+                        _lib.check(lib.devis_dcn_col2im_og(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
                                                            _ptr(mask[n0:n1]) if mask is not None else None, _ptr(grad_cols),
                                                            _ptr(gx[n0:n1]) if need_in else None, _ptr(grad_off[n0:n1]),
                                                            _ptr(grad_m[n0:n1]) if mask is not None else None, n1 - n0,
-                                                           *ctx.dims[1:], _DTYPES[x.dtype], flags, _ptr(ws), ws_bytes,
+                                                           *ctx.dims[1:], og, _DTYPES[x.dtype], flags, _ptr(ws), ws_bytes,
                                                            stream))
                 grad_in = gx.permute(0, 3, 1, 2) if need_in else None
-            if need_w and x.dtype == torch.float32 and not torch.are_deterministic_algorithms_enabled() \
+            if need_w and og == 1 and x.dtype == torch.float32 and not torch.are_deterministic_algorithms_enabled() \
                     and lib.devis_dcn_wgrad_supported(c, cout, kh, kw, _DTYPES[x.dtype]):
-                # narrow layers: gather + contraction with grad_out in one kernel, no column matrix (dcn_wgrad_kernel).
-                # Its cross-block float atomics are order-dependent: under torch.use_deterministic_algorithms the GEMM
-                # route below, deterministic like torchvision's, is taken instead.
+                # narrow layers: gather + contraction with grad_out in one kernel, no column matrix (dcn_wgrad_kernel,
+                # one offset group only).  Its cross-block float atomics are order-dependent: under
+                # torch.use_deterministic_algorithms the GEMM route below, deterministic like torchvision's, is taken.
                 gw3 = torch.empty((cout, k, c), dtype=x.dtype, device=x.device)
                 _lib.check(lib.devis_dcn_weight_grad(_ptr(x), _ptr(offset), _ptr(mask), _ptr(g), _ptr(gw3), *ctx.dims,
                                                      cout, stream))
@@ -235,9 +247,9 @@ class FusedDeformConv2dFunction(Function):
                 for n0 in range(0, n, per):
                     n1 = min(n, n0 + per)
                     rows = (n1 - n0) * ho * wo
-                    _lib.check(lib.devis_dcn_im2col(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
-                                                    _ptr(mask[n0:n1]) if mask is not None else None, _ptr(cols),
-                                                    n1 - n0, *ctx.dims[1:], _DTYPES[x.dtype], stream))
+                    _lib.check(lib.devis_dcn_im2col_og(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
+                                                       _ptr(mask[n0:n1]) if mask is not None else None, _ptr(cols),
+                                                       n1 - n0, *ctx.dims[1:], og, _DTYPES[x.dtype], stream))
                     gw2 += _wgrad(g2[n0 * ho * wo:n1 * ho * wo], cols[:rows])
                 grad_w = gw2.view(cout, kh, kw, c).permute(0, 3, 1, 2)
         if need_b and ctx.has_bias:
@@ -259,15 +271,15 @@ class DeformConv2dFunction(Function):
         offset = offset if offset.is_contiguous() else offset.contiguous()
         if mask is not None:
             mask = mask if mask.is_contiguous() else mask.contiguous()
-        k = kh * kw
+        k, og = kh * kw, _offset_groups(offset, kh, kw)
         cols = torch.empty((n * ho * wo, k * c), dtype=input.dtype, device=input.device)
         dims = (n, h, w, c, ho, wo, kh, kw, sh, sw, ph, pw, dh, dw)
         with torch.cuda.device(input.device):
-            _lib.check(_lib.load().devis_dcn_im2col(_ptr(x), _ptr(offset), _ptr(mask), _ptr(cols), *dims,
-                                                    _DTYPES[input.dtype], torch.cuda.current_stream().cuda_stream))
+            _lib.check(_lib.load().devis_dcn_im2col_og(_ptr(x), _ptr(offset), _ptr(mask), _ptr(cols), *dims, og,
+                                                       _DTYPES[input.dtype], torch.cuda.current_stream().cuda_stream))
         w2 = weight.permute(0, 2, 3, 1).reshape(cout, k * c)              # columns are [k][ci]
         out = torch.addmm(bias, cols, w2.t()) if bias is not None else cols @ w2.t()
-        ctx.dims = dims
+        ctx.dims, ctx.og = dims, og
         ctx.has_bias = bias is not None
         ctx.save_for_backward(x, offset, mask, cols, w2)
         return out.view(n, ho, wo, cout).permute(0, 3, 1, 2)
@@ -298,13 +310,13 @@ class DeformConv2dFunction(Function):
                 ws, ws_bytes = _workspace(lib, per, h, w, c, flags, x.device)
                 for n0 in range(0, n, per):
                     n1 = min(n, n0 + per)
-                    _lib.check(lib.devis_dcn_col2im_ex(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
+                    _lib.check(lib.devis_dcn_col2im_og(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
                                                        _ptr(mask[n0:n1]) if mask is not None else None,
                                                        _ptr(grad_cols[n0 * ho * wo:n1 * ho * wo]),
                                                        _ptr(gx[n0:n1]) if need_in else None, _ptr(grad_off[n0:n1]),
                                                        _ptr(grad_m[n0:n1]) if mask is not None else None, n1 - n0,
-                                                       *ctx.dims[1:], _DTYPES[x.dtype], flags, _ptr(ws), ws_bytes,
-                                                       stream))
+                                                       *ctx.dims[1:], ctx.og, _DTYPES[x.dtype], flags, _ptr(ws),
+                                                       ws_bytes, stream))
             grad_in = gx.permute(0, 3, 1, 2) if need_in else None
         return grad_in, grad_off, grad_w, grad_b, grad_m, None, None, None
 
@@ -329,7 +341,7 @@ class IGemmDeformConv2dFunction(Function):
     """apply(input, offset, weight, bias, mask, stride, padding, dilation) -> (N, Cout, Ho, Wo)
 
     Forward of the wide mask-head layers as an implicit GEMM on the tensor cores (devis_dcn_igemm_forward, tcgen05 /
-    TMEM): no column matrix is written or kept.  Precision follows ``torch.backends.cuda.matmul.allow_tf32`` exactly as
+    TMEM): no column matrix is written or kept.  One offset group only.  Precision follows ``torch.backends.cuda.matmul.allow_tf32`` exactly as
     torchvision's ``addmm`` would: off (the default) -> 3xTF32, fp32-grade; on -> one TF32 pass.  The backward is the
     im2col form's (cuBLAS GEMMs + devis_dcn_col2im), with the columns RECOMPUTED for the weight gradient, so nothing of
     column size lives between forward and backward."""
@@ -424,17 +436,20 @@ def deform_conv2d(input, offset, weight, bias=None, stride=(1, 1), padding=(0, 0
     cout, cin_g, kh, kw = weight.shape
     if cin_g != c:
         raise RuntimeError(f"deform_conv2d: groups = {c // max(cin_g, 1)} is not supported by this build (groups = 1 only)")
-    if offset.shape[1] != 2 * kh * kw:
-        if offset.shape[1] % (2 * kh * kw) == 0 and offset.shape[1] > 0:
-            raise RuntimeError("deform_conv2d: offset_groups > 1 is not supported by this build")
-        raise RuntimeError(f"deform_conv2d: offset.shape[1] must be 2 * kernel_h * kernel_w = {2 * kh * kw}, got {offset.shape[1]}")
+    k = kh * kw
+    if offset.shape[1] == 0 or offset.shape[1] % (2 * k):
+        raise RuntimeError(f"deform_conv2d: offset.shape[1] must be a multiple of 2 * kernel_h * kernel_w = {2 * k}, "
+                           f"got {offset.shape[1]}")
+    og = _offset_groups(offset, kh, kw)
+    if c % og:
+        raise RuntimeError(f"deform_conv2d: input channels ({c}) must be divisible by offset_groups ({og})")
     ho, wo = _out_size(h, kh, stride[0], padding[0], dilation[0]), _out_size(w, kw, stride[1], padding[1], dilation[1])
     if ho <= 0 or wo <= 0:
         raise RuntimeError(f"deform_conv2d: calculated output size too small ({ho} x {wo})")
-    if tuple(offset.shape) != (n, 2 * kh * kw, ho, wo):
-        raise RuntimeError(f"deform_conv2d: offset must be {(n, 2 * kh * kw, ho, wo)}, got {tuple(offset.shape)}")
-    if mask is not None and tuple(mask.shape) != (n, kh * kw, ho, wo):
-        raise RuntimeError(f"deform_conv2d: mask must be {(n, kh * kw, ho, wo)}, got {tuple(mask.shape)}")
+    if tuple(offset.shape) != (n, 2 * og * k, ho, wo):
+        raise RuntimeError(f"deform_conv2d: offset must be {(n, 2 * og * k, ho, wo)}, got {tuple(offset.shape)}")
+    if mask is not None and tuple(mask.shape) != (n, og * k, ho, wo):
+        raise RuntimeError(f"deform_conv2d: mask must be {(n, og * k, ho, wo)}, got {tuple(mask.shape)}")
     if bias is not None and tuple(bias.shape) != (cout,):
         raise RuntimeError("deform_conv2d: bias must have out_channels elements")
     out_dtype = input.dtype
@@ -446,7 +461,7 @@ def deform_conv2d(input, offset, weight, bias=None, stride=(1, 1), padding=(0, 0
     same = lambda t: None if t is None else (t if t.dtype == input.dtype else t.to(input.dtype))
     # fused forward when the layer is served; when gradients are needed only if its data backward is fused as well
     # (otherwise the im2col form, which keeps its columns for the backward, is the faster training path)
-    form = _fused_form(c, cout, kh, kw, input.dtype) if n > 0 else 0
+    form = _fused_form(c, cout, kh, kw, input.dtype, og) if n > 0 else 0
     needs_grad = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (input, offset, weight, bias, mask))
     fn = FusedDeformConv2dFunction if form & 1 and (form & 2 or not needs_grad) else DeformConv2dFunction
     # Forward on the tensor cores (tcgen05 implicit GEMM) for the layers with enough contraction to pay for it: everything
@@ -454,7 +469,8 @@ def deform_conv2d(input, offset, weight, bias=None, stride=(1, 1), padding=(0, 0
     # (measured, benchmarks/igemm_narrow.py: 72 -> 32 @45x80 385 us against 613 us; 32 -> 16 @90x160 629 against 486 us and
     # 16 -> 4 623 against 246 us stay where they are).  With gradients the 72 -> 32 layer keeps the im2col form: its backward
     # reuses the forward's columns, which is 270 us faster there than recomputing them (at 560 MB of columns for 60 instances).
-    if n > 0 and _igemm_supported(c, cout, kh, kw, input.dtype) and \
+    # The tensor-core forward serves one offset group only.
+    if og == 1 and n > 0 and _igemm_supported(c, cout, kh, kw, input.dtype) and \
             (not form & 1 or (c * kh * kw >= 576 and cout >= 32 and not form & 2 and not needs_grad)):
         fn = IGemmDeformConv2dFunction
     out = fn.apply(input, same(offset), same(weight), same(bias), same(mask), stride, padding, dilation)

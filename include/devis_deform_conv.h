@@ -15,8 +15,17 @@
  * torchvision's layout: channel 2k is the row offset and 2k+1 the column offset of kernel position k = ky*kw + kx;
  * mask may be NULL (plain deformable convolution).  Columns: cols[((n*Ho + ho)*Wo + wo) * kh*kw*C + k*C + c], i.e. a
  * row-major (N*Ho*Wo, kh*kw*C) matrix; multiply it with weight.permute(0, 2, 3, 1).reshape(Cout, kh*kw*C)^T.
- * groups = 1 and offset_groups = 1 only.  dtype: DEVIS_MSDA_F32 or DEVIS_MSDA_F64.  Asynchronous on `stream`,
+ * groups = 1 only (no weight grouping).  dtype: DEVIS_MSDA_F32 or DEVIS_MSDA_F64.  Asynchronous on `stream`,
  * no allocation, no synchronisation; returns DEVIS_MSDA_OK or a DEVIS_MSDA_ERR_* code (devis_msda.h).
+ *
+ * Offset groups (torchvision's offset_groups, DCNv2's deformable groups).  The _og entry points take `offset_groups`
+ * = G right after dil_w; the functions without the suffix are the same call with G = 1.  With G groups `offset` is
+ * (N, 2*G*kh*kw, Ho, Wo), group-major: channel 2*(g*kh*kw + k) is the row offset and 2*(g*kh*kw + k) + 1 the column
+ * offset of kernel position k in group g; `mask` is (N, G*kh*kw, Ho, Wo), channel g*kh*kw + k.  Group g samples input
+ * channels [g*C/G, (g+1)*C/G) at its own points; the column layout above is unchanged (column k*C + c holds channel c
+ * sampled at the point of c's group).  Checked on the host before any CUDA call: offset_groups < 1 or
+ * channels % offset_groups != 0 -> DEVIS_MSDA_ERR_BAD_SHAPE; for im2col / col2im G*kh*kw > 65535 (the launch grid)
+ * -> DEVIS_MSDA_ERR_TOO_LARGE.
  */
 #ifndef DEVIS_DEFORM_CONV_H_
 #define DEVIS_DEFORM_CONV_H_
@@ -32,6 +41,10 @@ extern "C" {
 int devis_dcn_im2col(const void *input_nhwc, const void *offset, const void *mask, void *cols, int batch, int height,
                      int width, int channels, int out_h, int out_w, int kernel_h, int kernel_w, int stride_h,
                      int stride_w, int pad_h, int pad_w, int dil_h, int dil_w, int dtype, void *stream);
+int devis_dcn_im2col_og(const void *input_nhwc, const void *offset, const void *mask, void *cols, int batch, int height,
+                        int width, int channels, int out_h, int out_w, int kernel_h, int kernel_w, int stride_h,
+                        int stride_w, int pad_h, int pad_w, int dil_h, int dil_w, int offset_groups, int dtype,
+                        void *stream);
 
 /* Backward of the gather given grad_cols (same layout as cols):
  *   grad_input_nhwc  like input  -- zero-filled by this call, then accumulated (may be NULL: not needed)
@@ -54,13 +67,20 @@ int devis_dcn_col2im(const void *input_nhwc, const void *offset, const void *mas
  * without the flag).  Checked on the host before any CUDA call: float64 with the flag -> DEVIS_MSDA_ERR_UNSUPPORTED;
  * out_h * out_w * kernel_h * kernel_w >= 2^26 (the int64 sum could overflow) -> DEVIS_MSDA_ERR_TOO_LARGE; a missing or
  * short workspace -> DEVIS_MSDA_ERR_WORKSPACE.  The flag is ignored when grad_input_nhwc is NULL.
- * devis_dcn_col2im / devis_dcn_fused_backward are the _ex forms with flags = 0. */
+ * devis_dcn_col2im / devis_dcn_fused_backward are the _ex forms with flags = 0; the _ex forms are the _og forms with
+ * offset_groups = 1.  The bounds and the headroom rule do not depend on offset_groups (a tap reaches an input element
+ * through one group only). */
 size_t devis_dcn_backward_workspace_bytes(int batch, int height, int width, int channels, unsigned flags);
 int devis_dcn_col2im_ex(const void *input_nhwc, const void *offset, const void *mask, const void *grad_cols,
                         void *grad_input_nhwc, void *grad_offset, void *grad_mask, int batch, int height, int width,
                         int channels, int out_h, int out_w, int kernel_h, int kernel_w, int stride_h, int stride_w,
                         int pad_h, int pad_w, int dil_h, int dil_w, int dtype, unsigned flags, void *workspace,
                         size_t workspace_bytes, void *stream);
+int devis_dcn_col2im_og(const void *input_nhwc, const void *offset, const void *mask, const void *grad_cols,
+                        void *grad_input_nhwc, void *grad_offset, void *grad_mask, int batch, int height, int width,
+                        int channels, int out_h, int out_w, int kernel_h, int kernel_w, int stride_h, int stride_w,
+                        int pad_h, int pad_w, int dil_h, int dil_w, int offset_groups, int dtype, unsigned flags,
+                        void *workspace, size_t workspace_bytes, void *stream);
 
 
 /* ---- fused form: gather + contraction with the weights in one kernel; the column matrix is never written ------------
@@ -73,6 +93,9 @@ int devis_dcn_col2im_ex(const void *input_nhwc, const void *offset, const void *
  * a multiple of 16 up to 64 with kh*kw*channels <= 1024 (weights held in the constant bank, 16 output channels per
  * launch; calls from different streams are ordered against each other on the device because they share that bank).
  * Backward (data gradients): out_channels in {1, 2, 4, 8, 16}.
+ * Offset groups (the _og forms; without the suffix G = 1): G > 1 needs (channels / G) % 4 == 0 and is served by the
+ * lane-group kernels only (out_channels in {1, 2, 4, 8, 16}, forward and backward); the constant-bank forward serves
+ * G = 1 only.  A fused call for a layer devis_dcn_fused_form_og does not serve returns DEVIS_MSDA_ERR_UNSUPPORTED.
  * devis_dcn_pack_weight: rearranges torchvision's weight (out_channels, channels, kh, kw) into the layouts the fused
  * kernels read (devis_dcn_packed_weight_elems floats; deform_conv.cuh "PACKED WEIGHTS").
  * devis_dcn_fused_forward: out[(n*Ho + ho)*Wo + wo][co] (channels-last, (N, Ho, Wo, out_channels)) = bias[co] +
@@ -81,13 +104,21 @@ int devis_dcn_col2im_ex(const void *input_nhwc, const void *offset, const void *
  *   grad_input_nhwc (zero-filled here, then accumulated; may be NULL), grad_offset, grad_mask (fully written).
  *   The weight gradient is cols^T x grad_out: devis_dcn_im2col + GEMM on the caller's side. */
 int devis_dcn_fused_form(int channels, int out_channels, int kernel_h, int kernel_w, int dtype);
+int devis_dcn_fused_form_og(int channels, int out_channels, int kernel_h, int kernel_w, int offset_groups, int dtype);
 size_t devis_dcn_packed_weight_elems(int channels, int out_channels, int kernel_h, int kernel_w);
+size_t devis_dcn_packed_weight_elems_og(int channels, int out_channels, int kernel_h, int kernel_w, int offset_groups);
 int devis_dcn_pack_weight(const void *weight_oihw, void *packed, int channels, int out_channels, int kernel_h,
                           int kernel_w, void *stream);
+int devis_dcn_pack_weight_og(const void *weight_oihw, void *packed, int channels, int out_channels, int kernel_h,
+                             int kernel_w, int offset_groups, void *stream);
 int devis_dcn_fused_forward(const void *input_nhwc, const void *offset, const void *mask, const void *packed_weight,
                             const void *bias, void *out_nhwc, int batch, int height, int width, int channels, int out_h,
                             int out_w, int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w,
                             int dil_h, int dil_w, int out_channels, void *stream);
+int devis_dcn_fused_forward_og(const void *input_nhwc, const void *offset, const void *mask, const void *packed_weight,
+                               const void *bias, void *out_nhwc, int batch, int height, int width, int channels,
+                               int out_h, int out_w, int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h,
+                               int pad_w, int dil_h, int dil_w, int offset_groups, int out_channels, void *stream);
 int devis_dcn_fused_backward(const void *input_nhwc, const void *offset, const void *mask, const void *packed_weight,
                              const void *grad_out_nhwc, void *grad_input_nhwc, void *grad_offset, void *grad_mask,
                              int batch, int height, int width, int channels, int out_h, int out_w, int kernel_h,
@@ -98,13 +129,20 @@ int devis_dcn_fused_backward_ex(const void *input_nhwc, const void *offset, cons
                                 int batch, int height, int width, int channels, int out_h, int out_w, int kernel_h,
                                 int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w, int dil_h, int dil_w,
                                 int out_channels, unsigned flags, void *workspace, size_t workspace_bytes, void *stream);
+int devis_dcn_fused_backward_og(const void *input_nhwc, const void *offset, const void *mask, const void *packed_weight,
+                                const void *grad_out_nhwc, void *grad_input_nhwc, void *grad_offset, void *grad_mask,
+                                int batch, int height, int width, int channels, int out_h, int out_w, int kernel_h,
+                                int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w, int dil_h, int dil_w,
+                                int offset_groups, int out_channels, unsigned flags, void *workspace,
+                                size_t workspace_bytes, void *stream);
 
 /* devis_dcn_weight_grad: the weight gradient of a narrow layer without a column matrix,
  *   grad_weight[co][k][c] = sum over (n, ho, wo) of mask * bilinear(input[n, .., c]) * grad_out_nhwc[n, ho, wo, co]
  * i.e. (out_channels, kernel_h * kernel_w, channels) row-major, zero-filled here; permute to (Cout, C, kh, kw) on the
  * caller's side.  Replaces torchvision's deformable_im2col + at::addmm pair of the backward
  * (torchvision/csrc/ops/cuda/deform_conv2d_kernel.cu, backward_gradient_parameters) for float32 layers with
- * channels in {16, 32} and out_channels in {1, 2, 4, 8, 16}: devis_dcn_wgrad_supported says so (1 / 0). */
+ * channels in {16, 32} and out_channels in {1, 2, 4, 8, 16}: devis_dcn_wgrad_supported says so (1 / 0).
+ * One offset group only; with more, the weight gradient is devis_dcn_im2col_og + GEMM. */
 int devis_dcn_wgrad_supported(int channels, int out_channels, int kernel_h, int kernel_w, int dtype);
 int devis_dcn_weight_grad(const void *input_nhwc, const void *offset, const void *mask, const void *grad_out_nhwc,
                           void *grad_weight, int batch, int height, int width, int channels, int out_h, int out_w,
@@ -121,7 +159,8 @@ int devis_dcn_weight_grad(const void *input_nhwc, const void *offset, const void
  *              result (<= 1e-5 against the float64 fixtures); DEVIS_DCN_PRECISION_TF32: one TF32 pass, for callers that
  *              have torch.backends.cuda.matmul.allow_tf32 on (torchvision's addmm honours that switch as well).
  * devis_dcn_igemm_pack_weight: torchvision's weight (out_channels, channels, kh, kw) -> the kernel's swizzled hi / lo
- * slabs (devis_dcn_igemm_packed_weight_elems floats).  out: (N, Ho, Wo, out_channels) channels-last, fully written. */
+ * slabs (devis_dcn_igemm_packed_weight_elems floats).  out: (N, Ho, Wo, out_channels) channels-last, fully written.
+ * One offset group only. */
 #define DEVIS_DCN_PRECISION_3XTF32 0
 #define DEVIS_DCN_PRECISION_TF32 1
 int devis_dcn_igemm_supported(int channels, int out_channels, int kernel_h, int kernel_w, int dtype);

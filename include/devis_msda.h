@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define DEVIS_MSDA_ABI_VERSION 3
+#define DEVIS_MSDA_ABI_VERSION 4
 
 /* element types of value / output / grad_output */
 #define DEVIS_MSDA_F32 0  /* value, loc, weights, outputs and all gradients float            */
