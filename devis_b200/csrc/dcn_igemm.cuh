@@ -208,7 +208,7 @@ __global__ void __launch_bounds__(kIgThreads, MINB) dcn_igemm_fwd_kernel(const I
             float4 *gfac = reinterpret_cast<float4 *>(grow + kIgBM);
             if (tid < kIgBM) {                                      // geometry of (pixel tid, kernel position k), once
                 const long long pix = pix0 + tid;
-                int4 rows = make_int4(0, 0, 0, 0);
+                int4 rows = make_int4(-1, -1, -1, -1);                  // -1: corner outside the map, never read
                 float4 fac = make_float4(0.f, 0.f, 0.f, 0.f);
                 if (pix < a.P) {
                     const int n = (int)(pix / plane), pp = (int)(pix - (long long)n * plane);
@@ -217,8 +217,8 @@ __global__ void __launch_bounds__(kIgThreads, MINB) dcn_igemm_fwd_kernel(const I
                     dcn_sample_point(a.offset, a.mask, id, d, h, w, m);
                     const DcnTap<float> t = dcn_tap(h, w, d.H, d.W);
                     const int img = n * d.H * d.W;
-                    rows = make_int4((img + t.row[0]) * d.C, (img + t.row[1]) * d.C, (img + t.row[2]) * d.C,
-                                     (img + t.row[3]) * d.C);
+                    rows = make_int4(t.ok[0] ? (img + t.row[0]) * d.C : -1, t.ok[1] ? (img + t.row[1]) * d.C : -1,
+                                     t.ok[2] ? (img + t.row[2]) * d.C : -1, t.ok[3] ? (img + t.row[3]) * d.C : -1);
                     fac = make_float4(m * t.w[0], m * t.w[1], m * t.w[2], m * t.w[3]);
                 }
                 grow[tid] = rows;
@@ -241,14 +241,10 @@ __global__ void __launch_bounds__(kIgThreads, MINB) dcn_igemm_fwd_kernel(const I
                     const int p = g + 32 * i;
                     const int4 r = grow[p];
                     f[i] = gfac[p];
-                    if (live) {
-                        v[i][0] = __ldg(reinterpret_cast<const float4 *>(a.input + r.x + c0));
-                        v[i][1] = __ldg(reinterpret_cast<const float4 *>(a.input + r.y + c0));
-                        v[i][2] = __ldg(reinterpret_cast<const float4 *>(a.input + r.z + c0));
-                        v[i][3] = __ldg(reinterpret_cast<const float4 *>(a.input + r.w + c0));
-                    } else {
-                        v[i][0] = v[i][1] = v[i][2] = v[i][3] = make_float4(0.f, 0.f, 0.f, 0.f);
-                    }
+                    v[i][0] = dcn_corner4(reinterpret_cast<const float4 *>(a.input + max(r.x, 0) + c0), live && r.x >= 0);
+                    v[i][1] = dcn_corner4(reinterpret_cast<const float4 *>(a.input + max(r.y, 0) + c0), live && r.y >= 0);
+                    v[i][2] = dcn_corner4(reinterpret_cast<const float4 *>(a.input + max(r.z, 0) + c0), live && r.z >= 0);
+                    v[i][3] = dcn_corner4(reinterpret_cast<const float4 *>(a.input + max(r.w, 0) + c0), live && r.w >= 0);
                 }
                 float4 col[4];
 #pragma unroll

@@ -76,7 +76,10 @@ struct DcnDims {
 };
 
 // geometry of one tap, torchvision's bilinear_interpolate: the sample is void unless -1 < h < H and -1 < w < W; corners
-// outside the map contribute zero.  Rows are clamped in-bounds and their weights zeroed, so loads are unconditional.
+// outside the map contribute zero.  Rows are clamped in-bounds and their weights zeroed, but a corner outside the map
+// (ok == false) must never contribute its value: the clamped row is some other pixel, and 0 * Inf = NaN would carry a
+// non-finite value there into taps that never sample it.  The gathers load corners through dcn_corner / dcn_corner4
+// (not read, value 0 when dead); the scatter kernels use them only in dot products zeroed by ok afterwards.
 template <typename T>
 struct DcnTap {
     T w[4];          // bilinear weights of TL, TR, BL, BR with outside corners zeroed
@@ -113,6 +116,21 @@ __device__ __forceinline__ DcnTap<T> dcn_tap(T h, T w, int H, int W)
     t.row[2] = h1c * W + w0c;
     t.row[3] = h1c * W + w1c;
     return t;
+}
+
+// one corner value of a gather: the load is predicated off for a corner outside the map, whose value is 0.  (Loading the
+// clamped row unconditionally and selecting 0 afterwards needs fewer registers in dcn_wgrad_kernel, but measured slower
+// on every mask-head layer, 7 to 33 % for the tensor-core forward: the dead corners of border taps then cost memory
+// traffic.)
+template <typename T>
+__device__ __forceinline__ T dcn_corner(const T *p, bool ok)
+{
+    return ok ? *p : (T)0;
+}
+
+__device__ __forceinline__ float4 dcn_corner4(const float4 *p, bool ok)
+{
+    return ok ? __ldg(p) : make_float4(0.f, 0.f, 0.f, 0.f);
 }
 
 // A tap is addressed by the launch grid: blockIdx.z (+ n_base) = batch item, blockIdx.y = virtual kernel position
@@ -181,7 +199,8 @@ __global__ void __launch_bounds__(256) dcn_im2col_kernel(const T *__restrict__ i
         const float4 *r3 = reinterpret_cast<const float4 *>(img + (long long)t.row[3] * d.C);
         float4 *o = reinterpret_cast<float4 *>(out);
         for (int c = j; c < Cg / 4; c += G) {
-            const float4 a = __ldg(r0 + c), b = __ldg(r1 + c), e = __ldg(r2 + c), f = __ldg(r3 + c);
+            const float4 a = dcn_corner4(r0 + c, t.ok[0]), b = dcn_corner4(r1 + c, t.ok[1]);
+            const float4 e = dcn_corner4(r2 + c, t.ok[2]), f = dcn_corner4(r3 + c, t.ok[3]);
             float4 s;
             s.x = f0 * a.x + f1 * b.x + f2 * e.x + f3 * f.x;
             s.y = f0 * a.y + f1 * b.y + f2 * e.y + f3 * f.y;
@@ -192,7 +211,9 @@ __global__ void __launch_bounds__(256) dcn_im2col_kernel(const T *__restrict__ i
     } else {
         const T *r0 = img + (long long)t.row[0] * d.C, *r1 = img + (long long)t.row[1] * d.C;
         const T *r2 = img + (long long)t.row[2] * d.C, *r3 = img + (long long)t.row[3] * d.C;
-        for (int c = j; c < Cg; c += G) out[c] = f0 * r0[c] + f1 * r1[c] + f2 * r2[c] + f3 * r3[c];
+        for (int c = j; c < Cg; c += G)
+            out[c] = f0 * dcn_corner(r0 + c, t.ok[0]) + f1 * dcn_corner(r1 + c, t.ok[1]) + f2 * dcn_corner(r2 + c, t.ok[2]) +
+                     f3 * dcn_corner(r3 + c, t.ok[3]);
     }
 }
 
@@ -445,15 +466,17 @@ __global__ void __launch_bounds__(256, 2) dcn_fused_fwd_kernel(const float *__re
         const int ky = k / d.kw, kx = k - ky * d.kw;
         float fw[PPG][4];
         int row[PPG][4];
+        bool ok[PPG][4];
 #pragma unroll
         for (int i = 0; i < PPG; ++i) {
             const float h = (float)(tile.ho * d.sh - d.ph + ky * d.dh) + nxt[i].oh;
             const float w = (float)(tile.wo[i] * d.sw - d.pw + kx * d.dw) + nxt[i].ow;
-            const DcnTap<float> t = dcn_tap(h, w, d.H, d.W);      // a sample outside the map has four zero weights
+            const DcnTap<float> t = dcn_tap(h, w, d.H, d.W);      // a sample outside the map has four dead corners
 #pragma unroll
             for (int q = 0; q < 4; ++q) {
                 fw[i][q] = nxt[i].m * t.w[q];
                 row[i][q] = t.row[q] * C4 + grp * Cg4;
+                ok[i][q] = t.ok[q];
             }
         }
         if (v + 1 < GK) {    // next position's offsets and mask: in flight while this one is gathered and contracted
@@ -466,7 +489,8 @@ __global__ void __launch_bounds__(256, 2) dcn_fused_fwd_kernel(const float *__re
             float4 s[PPG];
 #pragma unroll
             for (int i = 0; i < PPG; ++i) {
-                const float4 a = __ldg(img + row[i][0] + c), bb = __ldg(img + row[i][1] + c), e = __ldg(img + row[i][2] + c), f = __ldg(img + row[i][3] + c);
+                const float4 a = dcn_corner4(img + row[i][0] + c, ok[i][0]), bb = dcn_corner4(img + row[i][1] + c, ok[i][1]);
+                const float4 e = dcn_corner4(img + row[i][2] + c, ok[i][2]), f = dcn_corner4(img + row[i][3] + c, ok[i][3]);
                 s[i].x = fw[i][0] * a.x + fw[i][1] * bb.x + fw[i][2] * e.x + fw[i][3] * f.x;
                 s[i].y = fw[i][0] * a.y + fw[i][1] * bb.y + fw[i][2] * e.y + fw[i][3] * f.y;
                 s[i].z = fw[i][0] * a.z + fw[i][1] * bb.z + fw[i][2] * e.z + fw[i][3] * f.z;
@@ -636,6 +660,7 @@ __global__ void __launch_bounds__(256, 2) dcn_fused_bwd_kernel(const float *__re
 constexpr int kDcnConstFloats = 16384;                 // 64 KB
 __constant__ __align__(16) float dcn_cw[kDcnConstFloats];            // [k][c][16] of the current 16-channel tile
 constexpr int kDcnCTileW = 32, kDcnCTileH = 8, kDcnCStride = kDcnCTileW * kDcnCTileH + 1;
+constexpr int kDcnCOutside = -0x7fffffff - 1;         // gather record of a pixel outside the output plane
 
 // packed layout for this form: wc[((t * K + k) * C + c) * CT + q] = weight[CT t + q][c][k], CT = output channels per thread
 __global__ void dcn_pack_weight_const_kernel(const float *__restrict__ w /* (Cout, C, K) */, float *__restrict__ wc, int cout,
@@ -709,22 +734,27 @@ __global__ void __launch_bounds__(256, CT == 16 ? 3 : 2)
             const float m = nxt.m;
             if (k + 1 < k1) nxt = dcn_load_point(offset_n, mask_n, k + 1, plane, my_at);
             rec_f[warp * 32 + lane] = make_float4(m * t.w[0], m * t.w[1], m * t.w[2], m * t.w[3]);
-            rec_r[warp * 32 + lane] = make_int4(my_live ? t.row[0] * C4 : -1, t.row[1] * C4, t.row[2] * C4, t.row[3] * C4);
+            // corner rows; -1 = corner outside the map (value 0, never read), kDcnCOutside = pixel outside the plane
+            const int r0 = t.ok[0] ? t.row[0] * C4 : -1;
+            rec_r[warp * 32 + lane] = make_int4(my_live ? r0 : kDcnCOutside, t.ok[1] ? t.row[1] * C4 : -1,
+                                                t.ok[2] ? t.row[2] * C4 : -1, t.ok[3] ? t.row[3] * C4 : -1);
         }
         if (k > k0) __syncthreads();                     // everyone is done reading the previous position's columns
         else __syncwarp();
 #pragma unroll 2
         for (int it = 0; it < kDcnCTileH; ++it) {
             const int4 rr = rec_r[warp * 32 + grp * 8 + it];
-            if (rr.x < 0) continue;                      // pixel outside the plane: its columns are never read
+            if (rr.x == kDcnCOutside) continue;          // pixel outside the plane: its columns are never read
             const float4 ff = rec_f[warp * 32 + grp * 8 + it];
-            const float4 *r0 = img + rr.x, *r1 = img + rr.y, *r2 = img + rr.z, *r3 = img + rr.w;
+            const bool ok0 = rr.x >= 0, ok1 = rr.y >= 0, ok2 = rr.z >= 0, ok3 = rr.w >= 0;
+            const float4 *r0 = img + max(rr.x, 0), *r1 = img + max(rr.y, 0), *r2 = img + max(rr.z, 0), *r3 = img + max(rr.w, 0);
             float *dst = cols_s + it * 32 + warp * 4 + grp;
 #pragma unroll
             for (int b = 0; b < nblk; ++b) {
                 const int c = b * 8 + j;
                 if (c >= C4) break;
-                const float4 a = __ldg(r0 + c), bb = __ldg(r1 + c), e = __ldg(r2 + c), f = __ldg(r3 + c);
+                const float4 a = dcn_corner4(r0 + c, ok0), bb = dcn_corner4(r1 + c, ok1);
+                const float4 e = dcn_corner4(r2 + c, ok2), f = dcn_corner4(r3 + c, ok3);
                 dst[(4 * c + 0) * kDcnCStride] = ff.x * a.x + ff.y * bb.x + ff.z * e.x + ff.w * f.x;
                 dst[(4 * c + 1) * kDcnCStride] = ff.x * a.y + ff.y * bb.y + ff.z * e.y + ff.w * f.y;
                 dst[(4 * c + 2) * kDcnCStride] = ff.x * a.z + ff.y * bb.z + ff.z * e.z + ff.w * f.z;
@@ -818,8 +848,10 @@ __global__ void __launch_bounds__(256) dcn_wgrad_kernel(const float *__restrict_
             const float w = (float)(id.wo * d.sw - d.pw + kx * d.dw) + c_ow;
             const DcnTap<float> t = dcn_tap(h, w, d.H, d.W);
             const float f0 = m * t.w[0], f1 = m * t.w[1], f2 = m * t.w[2], f3 = m * t.w[3];
-            const float4 a = __ldg(img + (long long)t.row[0] * G + j), b = __ldg(img + (long long)t.row[1] * G + j);
-            const float4 e = __ldg(img + (long long)t.row[2] * G + j), f = __ldg(img + (long long)t.row[3] * G + j);
+            const float4 a = dcn_corner4(img + (long long)t.row[0] * G + j, t.ok[0]);
+            const float4 b = dcn_corner4(img + (long long)t.row[1] * G + j, t.ok[1]);
+            const float4 e = dcn_corner4(img + (long long)t.row[2] * G + j, t.ok[2]);
+            const float4 f = dcn_corner4(img + (long long)t.row[3] * G + j, t.ok[3]);
             float v[4];
             v[0] = f0 * a.x + f1 * b.x + f2 * e.x + f3 * f.x;
             v[1] = f0 * a.y + f1 * b.y + f2 * e.y + f3 * f.y;

@@ -3,7 +3,8 @@
 Pure-PyTorch, differentiable restatement of torchvision's modulated deformable convolution, the third-party operator
 DeVIS's mask head calls (src/models/deformable_segmentation.py:265; torchvision pinned at 0.12 by docs/INSTALL.md:9,
 0.26 in this image).  Follows torchvision/csrc/ops/cpu/deform_conv2d_kernel.cpp:
-  bilinear_interpolate   : the sample is 0 unless -1 < h < H and -1 < w < W; corners outside the map contribute 0
+  bilinear_interpolate   : the sample is 0 unless -1 < h < H and -1 < w < W; corners outside the map contribute 0 and
+                           are never read (a non-finite pixel only reaches the taps whose live corners include it)
   deformable_im2col      : sample point = (ho*stride - pad + ky*dil + offset[2k], wo*stride - pad + kx*dil + offset[2k+1]),
                            column value = mask[k] * interpolated input
   deform_conv2d forward  : out = weight (Cout, Cin*kh*kw) x columns + bias
@@ -37,7 +38,10 @@ def deform_conv2d_torch(x, offset, weight, bias=None, stride=(1, 1), padding=(0,
     def corner(yy, xx, wgt):
         ok = inside & (yy >= 0) & (yy <= h - 1) & (xx >= 0) & (xx <= w - 1)
         idx = (yy.clamp(0, h - 1) * w + xx.clamp(0, w - 1)).long().reshape(n, 1, -1).expand(n, c, -1)
-        val = torch.gather(flat, 2, idx).view(n, c, k, ho, wo)
+        # a corner outside the map is never read (torchvision's bilinear_interpolate): its gathered value is replaced by
+        # 0 before it is weighted, so a non-finite pixel at the clamped position cannot leak in as 0 * Inf = NaN.  The
+        # select is on the value, not on the product, for the same reason in the weight and offset gradients.
+        val = torch.where(ok[:, None], torch.gather(flat, 2, idx).view(n, c, k, ho, wo), 0)
         return val * (wgt * ok.to(dt))[:, None]
 
     cols = corner(y0, x0, hy * hx) + corner(y0, x0 + 1, hy * lx) + corner(y0 + 1, x0, ly * hx) + corner(y0 + 1, x0 + 1, ly * lx)

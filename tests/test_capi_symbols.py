@@ -50,6 +50,8 @@ def test_argument_validation_happens_before_any_cuda_call():
     from devis_b200 import _lib
     lib = _lib.load()
     null = None
+    # per-family launch counters before the calls below: GPU tests earlier in the same process may have launched kernels
+    launched = [lib.devis_msda_kernel_launches(f) for f in range(64)]
     assert lib.devis_msda_forward(null, null, null, null, null, null, 1, 4, 2, 32, 1, 1, 1, 64, 7, null) == -3
     assert lib.devis_msda_forward(null, null, null, null, null, null, 1, 4, 0, 32, 1, 1, 1, 64, 0, null) == -2
     assert lib.devis_msda_forward(null, null, null, null, null, null, 3, 4, 2, 32, 1, 1, 1, 2, 0, null) == -4
@@ -86,10 +88,11 @@ def test_argument_validation_happens_before_any_cuda_call():
     fused = lambda ref_dim, tref, d=32: lib.devis_tmsda_fused_forward(
         *([null] * 15), 2, 8, 8, d, 1, 3, 4, 4, 1, ref_dim, tref, 0, null)
     assert fused(3, 0) == -2 and fused(2, 3) == -2 and fused(2, 0, 16) == -8 and fused(4, 2) == -1
-    # per-family launch counters exist for every family the header names and nothing has been launched
+    # per-family launch counters exist for every family the header names and none of the calls above launched anything
     header = open(HEADER).read()
     n_fam = int(re.search(r"#define DEVIS_MSDA_KERNEL_FAMILIES (\d+)", header).group(1))
-    assert n_fam == 10 and all(lib.devis_msda_kernel_launches(f) == 0 for f in range(n_fam))
+    assert n_fam == 10 and [lib.devis_msda_kernel_launches(f) for f in range(64)] == launched
+    assert all(v == 0 for v in launched[n_fam:])
     assert lib.devis_msda_kernel_launches(-1) == 0 and lib.devis_msda_kernel_launches(n_fam) == 0
     for name in ("TREF_LEVEL0", "TREF_OWN", "TREF_SAMPLED"):
         assert re.search(rf"#define DEVIS_TMSDA_{name} {getattr(_lib, name)}\b", header)

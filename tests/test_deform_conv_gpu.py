@@ -263,18 +263,46 @@ def test_mask_head_fp32_every_layer_matches_oracle_on_identical_inputs():
     offset moves every sample of the next layer), so the end-to-end error of ANY float32 implementation against the
     float64 fixture is ~1e-2.  The meaningful float32 statement is per layer: each of the five deformable convolutions
     (im2col, lane-group and constant-bank kernels all occur) agrees with the float64 oracle evaluated on the very inputs
-    it received."""
+    it received -- its output, and the gradients of its input, offset, weight, bias and mask for the grad_out it
+    received in the backward."""
+    import devis_b200.deformable_segmentation as seg
     from oracle.deform_conv_torch import deform_conv2d_torch
-    seen = []
+    layers = []
+    orig = seg.deform_conv2d
 
-    def check(input, offset, weight, bias, padding, mask, out):
-        d = lambda t: None if t is None else t.detach().double()
-        pad = (padding, padding) if isinstance(padding, int) else padding
-        ref = deform_conv2d_torch(d(input), d(offset), d(weight), d(bias), (1, 1), pad, (1, 1), d(mask))
-        seen.append(nmax(out.detach().cpu().numpy(), ref.cpu().numpy()))
+    def capturing(input, offset, weight, bias=None, stride=(1, 1), padding=(0, 0), dilation=(1, 1), mask=None):
+        # fresh graph nodes in front of the layer: the gradients hooked on them are this call's alone (the input also
+        # feeds the offset and mask branches, the weight is a Parameter)
+        rec = {"args": [input, offset, weight, bias, mask], "padding": padding, "grads": {}}
+        ins = []
+        for i, t in enumerate(rec["args"]):
+            if t is not None and t.requires_grad:
+                t = t.view_as(t)
+                t.register_hook(lambda gr, i=i: rec["grads"].__setitem__(i, gr.detach().clone()))
+            ins.append(t)
+        out = orig(ins[0], ins[1], ins[2], ins[3], stride, padding, dilation, ins[4])
+        out.register_hook(lambda gr: rec.__setitem__("gout", gr.detach().clone()))
+        rec["out"] = out.detach()
+        layers.append(rec)
+        return out
 
-    g, y, feats = _run_mask_head(torch.float32, check)
-    assert len(seen) == 5 and max(seen) < 1e-5, seen
+    seg.deform_conv2d = capturing
+    try:
+        g, y, feats = _run_mask_head(torch.float32)
+    finally:
+        seg.deform_conv2d = orig
+    assert len(layers) == 5
+    for li, rec in enumerate(layers):
+        pad = (rec["padding"],) * 2 if isinstance(rec["padding"], int) else rec["padding"]
+        leaves = [None if t is None else t.detach().double().requires_grad_(i in rec["grads"])
+                  for i, t in enumerate(rec["args"])]
+        ref = deform_conv2d_torch(leaves[0], leaves[1], leaves[2], leaves[3], (1, 1), pad, (1, 1), leaves[4])
+        assert nmax(rec["out"].cpu().numpy(), ref.detach().cpu().numpy()) < 1e-5, li
+        ref.backward(rec["gout"].double())
+        assert set(rec["grads"]) >= {0, 1, 2}, (li, sorted(rec["grads"]))
+        for i, got in rec["grads"].items():
+            e = nmax(got.cpu().numpy(), leaves[i].grad.cpu().numpy())
+            assert e < 1e-4, (li, ("input", "offset", "weight", "bias", "mask")[i], e)
     assert nmax(y.cpu().numpy(), g["out"]) < 0.2            # sanity only, see above
     assert all(torch.isfinite(f.grad).all() for f in feats)
 

@@ -138,3 +138,60 @@ def test_deform_conv_restatement_matches_installed_torchvision_directly():
     assert nmax(a.numpy(), b.numpy()) < 1e-13
     for k in ga:
         assert nmax(ga[k].numpy(), gb[k].numpy()) < 1e-12
+
+
+def _edge_problem(case, seed, poisoned):
+    """float64 problem of dcn_cases: offsets on a 2^-10 grid with a quarter of the coordinates on the edges of the map;
+    ``poisoned``: pixels (0..1, 0..1) non-finite, reached only by taps outside the map"""
+    import dcn_cases as dc
+    x, off, weight, bias, mask, gout = dc.operands(case, seed, edge_share=0.25)
+    if poisoned:
+        x, _, off = dc.poison(case, x, off)
+    return x, off, weight, bias, mask, gout
+
+
+def _fwd_bwd(fn, case, x, off, weight, bias, mask, gout):
+    leaves = [t.clone().requires_grad_(True) for t in (x, off, weight, bias, mask)]
+    out = fn(leaves[0], leaves[1], leaves[2], leaves[3], stride=case.stride, padding=case.pad, dilation=case.dil,
+             mask=leaves[4])
+    out.backward(gout)
+    return [out.detach()] + [t.grad for t in leaves]
+
+
+@pytest.mark.parametrize("poisoned", [False, True], ids=["finite", "nonfinite_outside"])
+@pytest.mark.parametrize("geometry", ["k3", "asym"])
+def test_deform_conv_restatement_matches_torchvision_at_edges(geometry, poisoned):
+    """the oracle against the installed torchvision (CPU, float64), forward and every gradient: taps on integer
+    coordinates, on H - 1 / W - 1, inside (-1, 0) and exactly on -1 and H / W; a 2 x 3 kernel with unequal stride,
+    padding and dilation; and non-finite pixels that only taps outside the map reach (torchvision never reads a corner
+    outside the map, so they must not turn the result into NaN).
+
+    One convention differs, at a single point: a tap exactly on -1 is void (value 0, the same on both sides), and its
+    offset gradient is 0 here and in this library's kernels, while torchvision's coordinate gradient takes the one-sided
+    derivative from inside the map.  Both offset components of such a tap are checked to be 0 here; the component whose
+    coordinate is -1 is left out of the comparison with torchvision."""
+    tv = pytest.importorskip("torchvision.ops")
+    import dcn_cases as dc
+    from oracle import deform_conv_torch
+    geo = dict(kh=2, kw=3, stride=(2, 1), pad=(1, 2), dil=(1, 2)) if geometry == "asym" else {}
+    case = dc.Case("edges", 2, 5, 3, 9, 11, **geo)
+    ops = _edge_problem(case, 5, poisoned)
+    a = _fwd_bwd(deform_conv_torch.deform_conv2d_torch, case, *ops)
+    b = _fwd_bwd(tv.deform_conv2d, case, *ops)
+    by, bx = dc._base(case)
+    o = ops[1].view(case.n, case.k, 2, case.ho, case.wo)
+    # the offset component whose own coordinate is exactly -1; the other component of such a tap is compared too, except
+    # where torchvision's own value is not finite (its coordinate gradient reads the edge row of a void tap at weight 0,
+    # 0 * Inf when that row is poisoned)
+    comp = torch.stack([(by + o[:, :, 0]) == -1, (bx + o[:, :, 1]) == -1], dim=2)
+    tap = (comp[:, :, 0] | comp[:, :, 1])[:, :, None].expand_as(comp)
+    comp, tap = comp.reshape(ops[1].shape), tap.reshape(ops[1].shape)
+    assert comp.any()
+    assert (a[2][tap] == 0).all()
+    b[2] = torch.where(comp | (tap & ~torch.isfinite(b[2])), 0, b[2])
+    for name, p, q in zip(("out", "gx", "goffset", "gweight", "gbias", "gmask"), a, b):
+        assert torch.isfinite(q).all() or name == "gx", name          # torchvision's own result is finite
+        if name == "gx" and poisoned:                                  # nothing reaches the poisoned pixels
+            assert (q[:, :, :2, :2] == 0).all() and (p[:, :, :2, :2] == 0).all()
+        assert torch.isfinite(p).all(), name
+        assert nmax(p.numpy(), q.numpy()) < 1e-12, name
