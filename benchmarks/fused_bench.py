@@ -1,7 +1,7 @@
 """Times the fused-prologue whole-clip op (TemporalMSDeformAttnFusedFunction: softmax + location arithmetic inside the
 kernels) forward and forward+backward at the DeVIS R50 T=6 encoder shape, through autograd, with CUDA events.
 
-    python benchmarks/fused_bench.py [--dtype fp32|bf16] [--iters 30]
+    python benchmarks/fused_bench.py [--dtype fp32|bf16|fp16] [--iters 30]
 """
 import argparse
 import json
@@ -18,7 +18,7 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--dtype", default="fp32")
 ap.add_argument("--iters", type=int, default=30)
 a = ap.parse_args()
-dtype = {"fp32": torch.float32, "bf16": torch.bfloat16}[a.dtype]
+dtype = {"fp32": torch.float32, "bf16": torch.bfloat16, "fp16": torch.float16}[a.dtype]
 torch.manual_seed(0)
 T, shapes_l, M, D, pc, pt = 6, synthetic.DEVIS_SHAPES, 8, 32, 4, 4
 nl, wt = len(shapes_l), T - 1

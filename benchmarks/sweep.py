@@ -1,7 +1,7 @@
 """Developer sweep (not the contract benchmark -- that is bench.py): times the whole-clip kernels at the
 DeVIS R50 T=6 encoder shape for launch-shape variants, calling the C ABI directly on preallocated buffers.
 
-    python benchmarks/sweep.py [--dist local|uniform] [--dtype fp32|bf16] [--iters 20]
+    python benchmarks/sweep.py [--dist local|uniform] [--dtype fp32|bf16|fp16] [--iters 20]
 """
 import argparse
 import itertools
@@ -26,7 +26,8 @@ class RawClip:
         self.geom = clip_geometry.ClipGeometry(clip["shapes"], v.shape[0], clip["frame_table"])
         self.t, self.s, self.m, self.d = v.shape
         self.lq, self.pc, self.pt = clip["loc_curr"].shape[1], clip["loc_curr"].shape[4], clip["loc_temporal"].shape[4]
-        self.code = {torch.float32: 0, torch.float64: 1, torch.bfloat16: 2}[v.dtype]
+        self.code = {torch.float32: _lib.F32, torch.float64: _lib.F64, torch.bfloat16: _lib.BF16,
+                     torch.float16: _lib.F16}[v.dtype]
         self.out = torch.empty(self.t, self.lq, self.m * self.d, dtype=v.dtype, device=v.device)
         self.gv = torch.empty(v.shape, dtype=torch.float32, device=v.device)
         self.gv_half = torch.empty(v.shape, dtype=torch.bfloat16, device=v.device) if v.dtype == torch.bfloat16 else None
@@ -86,7 +87,7 @@ def main():
     ap.add_argument("--quick", action="store_true")
     ap.add_argument("--det", action="store_true", help="also time the deterministic backward")
     a = ap.parse_args()
-    dtype = {"fp32": torch.float32, "bf16": torch.bfloat16}[a.dtype]
+    dtype = {"fp32": torch.float32, "bf16": torch.bfloat16, "fp16": torch.float16}[a.dtype]
     clip = synthetic.make_clip(dist=a.dist, dtype=dtype, queries=a.queries or None, device="cuda", sigma_px=a.sigma)
     fb, bb = synthetic.algorithmic_bytes(6, 4820, 8, 32, clip["loc_curr"].shape[1], 96, elem=clip["value"].element_size())
     rows = []

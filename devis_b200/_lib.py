@@ -12,8 +12,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # DEVIS_MSDA_LIB selects another build of the same ABI (kernel A/B experiments); the default is the in-tree library
 LIB_PATH = os.environ.get("DEVIS_MSDA_LIB") or os.path.join(_HERE, "libdevis_msda.so")
 
-ABI_VERSION = 4
-F32, F64, BF16 = 0, 1, 2
+ABI_VERSION = 5
+F32, F64, BF16, F16 = 0, 1, 2, 3
 FLAG_DETERMINISTIC, FLAG_NO_GRAD_VALUE, FLAG_BF16_GRAD_VALUE = 1, 2, 4
 # temporal_ref_mode of the fused-prologue entry points (DEVIS_TMSDA_TREF_*)
 TREF_LEVEL0, TREF_OWN, TREF_SAMPLED = 0, 1, 2

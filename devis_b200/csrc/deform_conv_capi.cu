@@ -50,10 +50,10 @@ int det_begin(void *workspace, const DcnDims &d, const void *grad, size_t n_grad
     slots = reinterpret_cast<unsigned *>(det.acc + n_acc);
     det.max_bits = slots;
     const int blocks = devis_capi_helper_blocks();
-    absmax_kernel<false><<<blocks, 256, 0, st>>>(grad, n_grad, slots);
+    absmax_kernel<Elem::F32><<<blocks, 256, 0, st>>>(grad, n_grad, slots);
     int rc = devis_capi_check_launch(DEVIS_MSDA_KERNEL_AUX);
     if (rc) return rc;
-    if (mask) absmax_kernel<false><<<blocks, 256, 0, st>>>(mask, (size_t)d.N * d.og * d.kh * d.kw * d.Ho * d.Wo, slots + 1);
+    if (mask) absmax_kernel<Elem::F32><<<blocks, 256, 0, st>>>(mask, (size_t)d.N * d.og * d.kh * d.kw * d.Ho * d.Wo, slots + 1);
     else set_word_kernel<<<1, 1, 0, st>>>(slots + 1, 0x3f800000u);
     return devis_capi_check_launch(DEVIS_MSDA_KERNEL_AUX);
 }
@@ -543,7 +543,7 @@ int devis_dcn_fused_backward_og(const void *input, const void *offset, const voi
         rc = det_begin(workspace, d, grad_out, (size_t)n_pixels * out_channels, mask, st, ds, slots);
         if (rc) return rc;
         // factors 2, 3: max|W| over the lane-group layout (zero padded: same maximum) and Cout
-        absmax_kernel<false><<<devis_capi_helper_blocks(), 256, 0, st>>>(packed_weight, plan.lanes_elems, slots + 2);
+        absmax_kernel<Elem::F32><<<devis_capi_helper_blocks(), 256, 0, st>>>(packed_weight, plan.lanes_elems, slots + 2);
         rc = devis_capi_check_launch(DEVIS_MSDA_KERNEL_AUX);
         if (rc) return rc;
         const float cout_f = (float)out_channels;

@@ -40,7 +40,7 @@ template <class SlotSrc>
 struct BwdArgs {
     const void *value;
     const void *grad_out;
-    void *grad_value;   // fp32 accumulation target (also for bf16 value; bf16 under HALF_ACC); nullptr = skip
+    void *grad_value;   // fp32 accumulation target (also for 16-bit value; bf16 under HALF_ACC); nullptr = skip
     DetScale det;       // deterministic mode: det.acc != nullptr replaces the float reductions
     Segment seg[2];
     int n_seg;
@@ -75,7 +75,7 @@ __device__ __forceinline__ void reduce_scatter_taps(float (&d)[LPG][4], int j, f
 // HALF_ACC (bf16 value only, DEVIS_MSDA_FLAG_BF16_GRAD_VALUE): grad_value is a bf16 tensor laid out like value and
 // the scatter uses 8-byte packed reductions (red.global.add.noftz.v2.bf16x2, SASS REDG.E.ADD.BF16x4.RN): a row leaves
 // the SM as 2 sectors instead of 4, which is what the backward is bound by (DESIGN.md 3.6).
-template <bool BF16, int LPG, int QPG, class SlotSrc, bool HALF_ACC = false>
+template <Elem E, int LPG, int QPG, class SlotSrc, bool HALF_ACC = false>
 __global__ void __launch_bounds__(256, DEVIS_BWD_MIN_BLOCKS) msda_bwd_kernel(const BwdArgs<SlotSrc> a)
 {
     using X = TapExchange<LPG>;
@@ -103,22 +103,22 @@ __global__ void __launch_bounds__(256, DEVIS_BWD_MIN_BLOCKS) msda_bwd_kernel(con
         go[i] = make_float4(0.f, 0.f, 0.f, 0.f);
         if (qlive[i]) {
             const size_t row = ((size_t)outer * Lq + q[i]) * M + m;
-            go[i] = BF16 ? ldg_bf16x4(reinterpret_cast<const uint2 *>(a.grad_out) + row * LPG + j)
-                         : ld_stream_f4(reinterpret_cast<const float4 *>(a.grad_out) + row * LPG + j, pol);
+            if constexpr (E != Elem::F32) go[i] = ldg_16x4<E>(reinterpret_cast<const uint2 *>(a.grad_out) + row * LPG + j);
+            else go[i] = ld_stream_f4(reinterpret_cast<const float4 *>(a.grad_out) + row * LPG + j, pol);
         }
     }
 
-    constexpr unsigned kQuadBytes = BF16 ? 8u : 16u;
+    constexpr unsigned kQuadBytes = E != Elem::F32 ? 8u : 16u;
     const unsigned rowbytes = (unsigned)(M * LPG) * kQuadBytes;
     const char *vbase = reinterpret_cast<const char *>(a.value) + (size_t)(m * LPG + j) * kQuadBytes;
     // keep the per-lane base as ONE 64-bit register pair: each corner address is then base + u32 offset
     // (IADD3 + IADD3.X) instead of a re-derived IMAD.WIDE chain (5 instructions per address in round 1a)
     asm volatile("" : "+l"(vbase));
     // grad_value is fp32 unless HALF_ACC: 16 bytes per channel quad; offsets published for `value` scale by 16/kQuadBytes
-    static_assert(!HALF_ACC || BF16, "bf16 accumulation needs bf16 value");
+    static_assert(!HALF_ACC || E == Elem::BF16, "bf16 accumulation needs bf16 value");
     constexpr unsigned kGvQuadBytes = HALF_ACC ? 8u : 16u;
     char *gvb = a.grad_value ? reinterpret_cast<char *>(a.grad_value) + (size_t)(m * LPG + j) * kGvQuadBytes : nullptr;
-    constexpr unsigned kGvShift = (BF16 && !HALF_ACC) ? 1u : 0u;
+    constexpr unsigned kGvShift = (E != Elem::F32 && !HALF_ACC) ? 1u : 0u;
     // deterministic mode: 8-byte fixed-point accumulators, same row pitch in elements -> offsets scale by
     // 2 * 16 / kQuadBytes; within a (row, head) the channels are permuted (det_add4): lane j starts at word j
     char *detb = a.det.acc ? reinterpret_cast<char *>(a.det.acc) + (size_t)(m * LPG) * 32u + (size_t)j * 8u : nullptr;
@@ -159,11 +159,11 @@ __global__ void __launch_bounds__(256, DEVIS_BWD_MIN_BLOCKS) msda_bwd_kernel(con
                     float4 c;
                     X::fetch(buf, jj, g, off, c);
                     float4 v00, v01, v10, v11;
-                    if (BF16) {
-                        v00 = ldg_bf16x4(reinterpret_cast<const uint2 *>(vbase + off.x));
-                        v01 = ldg_bf16x4(reinterpret_cast<const uint2 *>(vbase + off.y));
-                        v10 = ldg_bf16x4(reinterpret_cast<const uint2 *>(vbase + off.z));
-                        v11 = ldg_bf16x4(reinterpret_cast<const uint2 *>(vbase + off.w));
+                    if constexpr (E != Elem::F32) {
+                        v00 = ldg_16x4<E>(reinterpret_cast<const uint2 *>(vbase + off.x));
+                        v01 = ldg_16x4<E>(reinterpret_cast<const uint2 *>(vbase + off.y));
+                        v10 = ldg_16x4<E>(reinterpret_cast<const uint2 *>(vbase + off.z));
+                        v11 = ldg_16x4<E>(reinterpret_cast<const uint2 *>(vbase + off.w));
                     } else {
                         v00 = ldg_f4(reinterpret_cast<const float4 *>(vbase + off.x), pol);
                         v01 = ldg_f4(reinterpret_cast<const float4 *>(vbase + off.y), pol);

@@ -67,7 +67,7 @@ __host__ __device__ inline size_t sort_smem_bytes(int n_slots_total, int lut_ent
 // msda_bwd_kernel's det_add4 adds, same scale) and both the in-register run sums and the global reductions are integer
 // additions: associative, so the result does not depend on the arrival order of the ranks -- and is bit-identical to
 // the direct deterministic scatter, with 5x fewer 64-bit reductions leaving the SM.
-template <bool BF16, bool DET = false>
+template <Elem E, bool DET = false>
 __global__ void __launch_bounds__(kSortThreads, DEVIS_BWDS_MIN_BLOCKS) msda_bwds_kernel(const SortArgs a)
 {
     constexpr int LPG = 8;
@@ -164,21 +164,21 @@ __global__ void __launch_bounds__(kSortThreads, DEVIS_BWDS_MIN_BLOCKS) msda_bwds
         if (p < n_pix) {
             const int q = b.src.lsi[lq] + (ty0 + p / tw) * Wq + tx0 + (p - (p / tw) * tw);
             const size_t row = ((size_t)outer * Lq + q) * M + m;
-            go[i] = BF16 ? ldg_bf16x4(reinterpret_cast<const uint2 *>(b.grad_out) + row * LPG + j)
-                         : ldg_f4(reinterpret_cast<const float4 *>(b.grad_out) + row * LPG + j);
+            if constexpr (E != Elem::F32) go[i] = ldg_16x4<E>(reinterpret_cast<const uint2 *>(b.grad_out) + row * LPG + j);
+            else go[i] = ldg_f4(reinterpret_cast<const float4 *>(b.grad_out) + row * LPG + j);
         }
         reinterpret_cast<float4 *>(s_go)[p * LPG + j] = go[i];
     }
     __syncthreads();
 
-    constexpr unsigned kQuadBytes = BF16 ? 8u : 16u;
+    constexpr unsigned kQuadBytes = E != Elem::F32 ? 8u : 16u;
     const unsigned rowbytes = (unsigned)(M * LPG) * kQuadBytes;
     const char *vbase = reinterpret_cast<const char *>(b.value) + (size_t)(m * LPG + j) * kQuadBytes;
     asm volatile("" : "+l"(vbase));
     // fp32 grad_value (host-checked), or the deterministic mode's 8-byte accumulators in det_add4's permuted order
     char *gvb = DET ? reinterpret_cast<char *>(b.det.acc) + (size_t)(m * LPG) * 32u + (size_t)j * 8u
                     : reinterpret_cast<char *>(b.grad_value) + (size_t)(m * LPG + j) * 16u;
-    constexpr unsigned kGvShift = (BF16 ? 1u : 0u) + (DET ? 1u : 0u);
+    constexpr unsigned kGvShift = (E != Elem::F32 ? 1u : 0u) + (DET ? 1u : 0u);
     const size_t gv_rowbytes = (size_t)(M * LPG) * (DET ? 32u : 16u);
     const float det_sh = DET ? ldexpf(1.f, kDetFracBits - det_exponent(b.det.max_bits)) : 0.f;
 
@@ -254,11 +254,11 @@ __global__ void __launch_bounds__(kSortThreads, DEVIS_BWDS_MIN_BLOCKS) msda_bwds
                     const bool direct = (off.x & 1u) == 0u;
                     off.x &= ~1u;
                     float4 v00, v01, v10, v11;
-                    if (BF16) {
-                        v00 = ldg_bf16x4(reinterpret_cast<const uint2 *>(vbase + off.x));
-                        v01 = ldg_bf16x4(reinterpret_cast<const uint2 *>(vbase + off.y));
-                        v10 = ldg_bf16x4(reinterpret_cast<const uint2 *>(vbase + off.z));
-                        v11 = ldg_bf16x4(reinterpret_cast<const uint2 *>(vbase + off.w));
+                    if constexpr (E != Elem::F32) {
+                        v00 = ldg_16x4<E>(reinterpret_cast<const uint2 *>(vbase + off.x));
+                        v01 = ldg_16x4<E>(reinterpret_cast<const uint2 *>(vbase + off.y));
+                        v10 = ldg_16x4<E>(reinterpret_cast<const uint2 *>(vbase + off.z));
+                        v11 = ldg_16x4<E>(reinterpret_cast<const uint2 *>(vbase + off.w));
                     } else {
                         v00 = ldg_f4(reinterpret_cast<const float4 *>(vbase + off.x));
                         v01 = ldg_f4(reinterpret_cast<const float4 *>(vbase + off.y));

@@ -89,9 +89,13 @@ int devis_capi_check_launch(int family)
 namespace {
 
 int cuda_fail(cudaError_t e) { return devis_capi_cuda_fail(e); }
+
+// DEVIS_MSDA_BF16 and DEVIS_MSDA_F16 take the same kernels, launch shapes and byte thresholds (2-byte elements); only
+// the widening on load and the rounding on store differ (Elem)
+bool is_16bit(int dtype) { return dtype == DEVIS_MSDA_BF16 || dtype == DEVIS_MSDA_F16; }
 int check_launch(int family) { return devis_capi_check_launch(family); }
 
-size_t elem_size(int dtype) { return dtype == DEVIS_MSDA_F64 ? 8 : dtype == DEVIS_MSDA_BF16 ? 2 : 4; }
+size_t elem_size(int dtype) { return dtype == DEVIS_MSDA_F64 ? 8 : is_16bit(dtype) ? 2 : 4; }
 
 // channel counts served by the grouped-lane kernels: D = 4 * LPG.  They address value with 32-bit byte
 // offsets, so tensors of 4 GiB and more go to the generic kernels.
@@ -145,26 +149,32 @@ int launch_forward(const FwdArgs<SlotSrc> &a, int dtype, cudaStream_t st)
     size_t smem = (size_t)a.n_slots_total * sizeof(int4);
     const int lpg = lanes_per_group(dtype, d);
     // D = 32 with P % 4 == 0 in every segment and value below 2 GiB (signed 32-bit tap offsets): the round-2 kernels with
-    // 16-byte tap records and the dead corners skipped.  fp32 value: eight lanes x 4 channels (msda_fwdv_kernel); bf16
+    // 16-byte tap records and the dead corners skipped.  fp32 value: eight lanes x 4 channels (msda_fwdv_kernel); bf16 / fp16
     // value: four lanes x 8 channels (msda_fwd8v_kernel: 64-byte rows cost 0.75 instead of 1.0 data-pipe cycles that way;
     // for fp32 the four-lane shape needs LDG.E.256 and loses, profiles/r2s_fwd_wide_f32_variants.json).  With 8 heads the
     // size of a value row is a compile-time immediate of the gathers.  Everything else takes msda_fwd_kernel below.
     bool compact = lpg == 8 && (unsigned long long)d.outer * d.S * d.M * d.D * elem_size(dtype) < (1ull << 31);
     for (int sg = 0; sg < a.n_seg; ++sg) compact = compact && (a.seg[sg].P % 4 == 0);
-    if (compact && dtype == DEVIS_MSDA_BF16) {
+    if (compact && is_16bit(dtype)) {
         const LaunchShape s = pick_shape(d.Lq, kShapeFwdBf16, 2, 0, 1);
         smem += (size_t)(s.threads / 32) * Tap16::kBytesPerWarp;
         const int qc = s.threads / 4;
         const long long chunks = ((long long)d.Lq + (long long)qc * s.qpg - 1) / ((long long)qc * s.qpg);
         if (chunks * d.M > 0x7fffffffLL) return DEVIS_MSDA_ERR_TOO_LARGE;
         const dim3 grid((unsigned)(chunks * d.M), (unsigned)d.outer);
-        if (d.M == 8) {
-            if (s.qpg == 2) msda_fwd8v_kernel<2, SlotSrc, 512><<<grid, s.threads, smem, st>>>(a);
-            else msda_fwd8v_kernel<1, SlotSrc, 512><<<grid, s.threads, smem, st>>>(a);
-        } else {
-            if (s.qpg == 2) msda_fwd8v_kernel<2, SlotSrc, 0><<<grid, s.threads, smem, st>>>(a);
-            else msda_fwd8v_kernel<1, SlotSrc, 0><<<grid, s.threads, smem, st>>>(a);
-        }
+#define DEVIS_FWD8V(E)                                                                                   \
+    do {                                                                                                 \
+        if (d.M == 8) {                                                                                  \
+            if (s.qpg == 2) msda_fwd8v_kernel<E, 2, SlotSrc, 512><<<grid, s.threads, smem, st>>>(a);     \
+            else msda_fwd8v_kernel<E, 1, SlotSrc, 512><<<grid, s.threads, smem, st>>>(a);                \
+        } else {                                                                                         \
+            if (s.qpg == 2) msda_fwd8v_kernel<E, 2, SlotSrc, 0><<<grid, s.threads, smem, st>>>(a);       \
+            else msda_fwd8v_kernel<E, 1, SlotSrc, 0><<<grid, s.threads, smem, st>>>(a);                  \
+        }                                                                                                \
+    } while (0)
+        if (dtype == DEVIS_MSDA_F16) DEVIS_FWD8V(Elem::F16);
+        else DEVIS_FWD8V(Elem::BF16);
+#undef DEVIS_FWD8V
         return check_launch(DEVIS_MSDA_KERNEL_FWD_GROUPED);
     }
     if (compact) {
@@ -179,8 +189,8 @@ int launch_forward(const FwdArgs<SlotSrc> &a, int dtype, cudaStream_t st)
         const dim3 grid((unsigned)(chunks * d.M), (unsigned)d.outer);
 #define DEVIS_FWDV(QPG)                                                                              \
     do {                                                                                             \
-        if (d.M == 8) msda_fwdv_kernel<false, QPG, SlotSrc, 1024><<<grid, s.threads, smem, st>>>(a); \
-        else msda_fwdv_kernel<false, QPG, SlotSrc, 0><<<grid, s.threads, smem, st>>>(a);             \
+        if (d.M == 8) msda_fwdv_kernel<Elem::F32, QPG, SlotSrc, 1024><<<grid, s.threads, smem, st>>>(a); \
+        else msda_fwdv_kernel<Elem::F32, QPG, SlotSrc, 0><<<grid, s.threads, smem, st>>>(a);             \
     } while (0)
         if (s.qpg == 4) DEVIS_FWDV(4);
         else if (s.qpg == 2) DEVIS_FWDV(2);
@@ -189,7 +199,7 @@ int launch_forward(const FwdArgs<SlotSrc> &a, int dtype, cudaStream_t st)
         return check_launch(DEVIS_MSDA_KERNEL_FWD_GROUPED);
     }
     if (lpg) {
-        const LaunchShape s = pick_shape(d.Lq, dtype == DEVIS_MSDA_BF16 ? kShapeFwdBf16 : kShapeFwdF32, 4, 0, 1);
+        const LaunchShape s = pick_shape(d.Lq, is_16bit(dtype) ? kShapeFwdBf16 : kShapeFwdF32, 4, 0, 1);
         smem += exchange_bytes(lpg, s.threads);
         const int qc = s.threads / lpg;
         const long long chunks = ((long long)d.Lq + (long long)qc * s.qpg - 1) / ((long long)qc * s.qpg);
@@ -203,11 +213,14 @@ int launch_forward(const FwdArgs<SlotSrc> &a, int dtype, cudaStream_t st)
         else DEVIS_FWD(BF, LPG, 1);                 \
     } while (0)
         if (dtype == DEVIS_MSDA_BF16) {
-            if (lpg == 8) DEVIS_FWD_Q(true, 8);
-            else DEVIS_FWD_Q(true, 4);
+            if (lpg == 8) DEVIS_FWD_Q(Elem::BF16, 8);
+            else DEVIS_FWD_Q(Elem::BF16, 4);
+        } else if (dtype == DEVIS_MSDA_F16) {
+            if (lpg == 8) DEVIS_FWD_Q(Elem::F16, 8);
+            else DEVIS_FWD_Q(Elem::F16, 4);
         } else {
-            if (lpg == 8) DEVIS_FWD_Q(false, 8);
-            else DEVIS_FWD_Q(false, 4);
+            if (lpg == 8) DEVIS_FWD_Q(Elem::F32, 8);
+            else DEVIS_FWD_Q(Elem::F32, 4);
         }
 #undef DEVIS_FWD_Q
 #undef DEVIS_FWD
@@ -219,6 +232,7 @@ int launch_forward(const FwdArgs<SlotSrc> &a, int dtype, cudaStream_t st)
     const dim3 grid((unsigned)blocks, (unsigned)d.outer);
     if (dtype == DEVIS_MSDA_F32) msda_fwd_generic_kernel<float, SlotSrc><<<grid, threads, smem, st>>>(a);
     else if (dtype == DEVIS_MSDA_F64) msda_fwd_generic_kernel<double, SlotSrc><<<grid, threads, smem, st>>>(a);
+    else if (dtype == DEVIS_MSDA_F16) msda_fwd_generic_kernel<__half, SlotSrc><<<grid, threads, smem, st>>>(a);
     else msda_fwd_generic_kernel<__nv_bfloat16, SlotSrc><<<grid, threads, smem, st>>>(a);
     return check_launch(DEVIS_MSDA_KERNEL_FWD_GENERIC);
 }
@@ -258,13 +272,14 @@ int launch_backward(BwdArgs<SlotSrc> a, int dtype, unsigned flags, void *workspa
         if (d.outer > 0 && d.Lq > 0) {
             const size_t n_go = (size_t)d.outer * d.Lq * d.M * d.D;
             const int blocks = devis_capi_helper_blocks();
-            if (dtype == DEVIS_MSDA_BF16) absmax_kernel<true><<<blocks, 256, 0, st>>>(a.grad_out, n_go, slots);
-            else absmax_kernel<false><<<blocks, 256, 0, st>>>(a.grad_out, n_go, slots);
+            if (dtype == DEVIS_MSDA_BF16) absmax_kernel<Elem::BF16><<<blocks, 256, 0, st>>>(a.grad_out, n_go, slots);
+            else if (dtype == DEVIS_MSDA_F16) absmax_kernel<Elem::F16><<<blocks, 256, 0, st>>>(a.grad_out, n_go, slots);
+            else absmax_kernel<Elem::F32><<<blocks, 256, 0, st>>>(a.grad_out, n_go, slots);
             int rc = check_launch(DEVIS_MSDA_KERNEL_AUX);
             if (rc) return rc;
             for (int sg = 0; sg < a.n_seg; ++sg) {
                 const size_t n_aw = (size_t)d.outer * d.Lq * d.M * a.seg[sg].n_slots * a.seg[sg].P;
-                absmax_kernel<false><<<blocks, 256, 0, st>>>(a.seg[sg].aw, n_aw, slots + 1);
+                absmax_kernel<Elem::F32><<<blocks, 256, 0, st>>>(a.seg[sg].aw, n_aw, slots + 1);
                 rc = check_launch(DEVIS_MSDA_KERNEL_AUX);
                 if (rc) return rc;
             }
@@ -306,14 +321,17 @@ int launch_backward(BwdArgs<SlotSrc> a, int dtype, unsigned flags, void *workspa
         else DEVIS_BWD(BF, LPG, 1);                 \
     } while (0)
         if (half_acc) {
-            if (lpg == 8) msda_bwd_kernel<true, 8, 1, SlotSrc, true><<<grid, s.threads, smem, st>>>(a);
-            else msda_bwd_kernel<true, 4, 1, SlotSrc, true><<<grid, s.threads, smem, st>>>(a);
+            if (lpg == 8) msda_bwd_kernel<Elem::BF16, 8, 1, SlotSrc, true><<<grid, s.threads, smem, st>>>(a);
+            else msda_bwd_kernel<Elem::BF16, 4, 1, SlotSrc, true><<<grid, s.threads, smem, st>>>(a);
         } else if (dtype == DEVIS_MSDA_BF16) {
-            if (lpg == 8) DEVIS_BWD_Q(true, 8);
-            else DEVIS_BWD_Q(true, 4);
+            if (lpg == 8) DEVIS_BWD_Q(Elem::BF16, 8);
+            else DEVIS_BWD_Q(Elem::BF16, 4);
+        } else if (dtype == DEVIS_MSDA_F16) {
+            if (lpg == 8) DEVIS_BWD_Q(Elem::F16, 8);
+            else DEVIS_BWD_Q(Elem::F16, 4);
         } else {
-            if (lpg == 8) DEVIS_BWD_Q(false, 8);
-            else DEVIS_BWD_Q(false, 4);
+            if (lpg == 8) DEVIS_BWD_Q(Elem::F32, 8);
+            else DEVIS_BWD_Q(Elem::F32, 4);
         }
 #undef DEVIS_BWD_Q
 #undef DEVIS_BWD
@@ -326,6 +344,7 @@ int launch_backward(BwdArgs<SlotSrc> a, int dtype, unsigned flags, void *workspa
     const dim3 grid((unsigned)blocks, (unsigned)d.outer);
     if (dtype == DEVIS_MSDA_F32) msda_bwd_generic_kernel<float, SlotSrc><<<grid, threads, smem, st>>>(a);
     else if (dtype == DEVIS_MSDA_F64) msda_bwd_generic_kernel<double, SlotSrc><<<grid, threads, smem, st>>>(a);
+    else if (dtype == DEVIS_MSDA_F16) msda_bwd_generic_kernel<__half, SlotSrc><<<grid, threads, smem, st>>>(a);
     else msda_bwd_generic_kernel<__nv_bfloat16, SlotSrc><<<grid, threads, smem, st>>>(a);
     const int rc = check_launch(DEVIS_MSDA_KERNEL_BWD_GENERIC);
     return rc ? rc : finalize();
@@ -333,7 +352,7 @@ int launch_backward(BwdArgs<SlotSrc> a, int dtype, unsigned flags, void *workspa
 
 // ---- sorted deterministic whole-clip backward (msda_bwd_sort.cuh) ------------------------------------------------
 // Serves the deterministic mode of the encoder form: one query per pyramid pixel (the caller says so by passing a
-// query_order), D = 32, fp32 / bf16 value, levels stored back to back, an even number of levels, 4 points per slot.
+// query_order), D = 32, fp32 / bf16 / fp16 value, levels stored back to back, an even number of levels, 4 points per slot.
 // ~4x faster than the direct 64-bit scatter and bit-identical to it.  (The float variant of the same scheme lost to the
 // direct float scatter -- data-pipe bound, DESIGN.md section 7 -- and is no longer built; benchmarks/experimental keeps
 // the round-1 windowed kernel for the record.)  Developer keys: 6 = 1 forces the direct scatter, 7 = window margin in
@@ -357,12 +376,12 @@ bool sort_applicable(const BwdArgs<ClipTable> &a, int dtype, unsigned flags)
     return true;
 }
 
-template <bool BF>
+template <Elem E>
 int launch_sort_kernel(const SortArgs &w, dim3 grid, size_t smem, cudaStream_t st)
 {
-    const cudaError_t e = cudaFuncSetAttribute(msda_bwds_kernel<BF, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    const cudaError_t e = cudaFuncSetAttribute(msda_bwds_kernel<E, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return cuda_fail(e);
-    msda_bwds_kernel<BF, true><<<grid, kSortThreads, smem, st>>>(w);
+    msda_bwds_kernel<E, true><<<grid, kSortThreads, smem, st>>>(w);
     return check_launch(DEVIS_MSDA_KERNEL_BWD_SORTED);
 }
 
@@ -385,12 +404,14 @@ int launch_backward_sort(const BwdArgs<ClipTable> &a, int dtype, cudaStream_t st
     const size_t smem = sort_smem_bytes(a.n_slots_total, w.lut_entries);
     if ((long long)tiles * d.M > 0x7fffffffLL) return DEVIS_MSDA_ERR_TOO_LARGE;
     const dim3 grid((unsigned)(tiles * d.M), (unsigned)d.outer);
-    return dtype == DEVIS_MSDA_BF16 ? launch_sort_kernel<true>(w, grid, smem, st) : launch_sort_kernel<false>(w, grid, smem, st);
+    if (dtype == DEVIS_MSDA_BF16) return launch_sort_kernel<Elem::BF16>(w, grid, smem, st);
+    if (dtype == DEVIS_MSDA_F16) return launch_sort_kernel<Elem::F16>(w, grid, smem, st);
+    return launch_sort_kernel<Elem::F32>(w, grid, smem, st);
 }
 
 int check_common(int outer, int S, int M, int D, int L, int Lq, int dtype)
 {
-    if (dtype != DEVIS_MSDA_F32 && dtype != DEVIS_MSDA_F64 && dtype != DEVIS_MSDA_BF16) return DEVIS_MSDA_ERR_BAD_DTYPE;
+    if (dtype != DEVIS_MSDA_F32 && dtype != DEVIS_MSDA_F64 && !is_16bit(dtype)) return DEVIS_MSDA_ERR_BAD_DTYPE;
     if (outer < 0 || S < 0 || M <= 0 || D <= 0 || L <= 0 || Lq < 0) return DEVIS_MSDA_ERR_BAD_SHAPE;
     if (outer > 65535) return DEVIS_MSDA_ERR_TOO_LARGE;
     // value rows are indexed with 31-bit integers in every kernel
@@ -696,11 +717,11 @@ int devis_tmsda_fused_forward(const void *value, const int64_t *spatial_shapes_h
     do {                                                                                                           \
         cudaStream_t st_ = (cudaStream_t)stream;                                                                   \
         if (dtype == DEVIS_MSDA_BF16) {                                                                            \
-            if (num_heads == 8) tmsda_fused_fwd_kernel<true, QPG, GEN, 512><<<grid, threads, smem, st_>>>(a);      \
-            else tmsda_fused_fwd_kernel<true, QPG, GEN, 0><<<grid, threads, smem, st_>>>(a);                       \
+            if (num_heads == 8) tmsda_fused_fwd_kernel<Elem::BF16, QPG, GEN, 512><<<grid, threads, smem, st_>>>(a);\
+            else tmsda_fused_fwd_kernel<Elem::BF16, QPG, GEN, 0><<<grid, threads, smem, st_>>>(a);                 \
         } else {                                                                                                   \
-            if (num_heads == 8) tmsda_fused_fwd_kernel<false, QPG, GEN, 1024><<<grid, threads, smem, st_>>>(a);    \
-            else tmsda_fused_fwd_kernel<false, QPG, GEN, 0><<<grid, threads, smem, st_>>>(a);                      \
+            if (num_heads == 8) tmsda_fused_fwd_kernel<Elem::F32, QPG, GEN, 1024><<<grid, threads, smem, st_>>>(a);\
+            else tmsda_fused_fwd_kernel<Elem::F32, QPG, GEN, 0><<<grid, threads, smem, st_>>>(a);                  \
         }                                                                                                          \
     } while (0)
     // the general (decoder) form: boxes, per-level / instance-aware temporal reference points, by-products
@@ -709,11 +730,16 @@ int devis_tmsda_fused_forward(const void *value, const int64_t *spatial_shapes_h
     if (general) {
         rc = fused_grid(a, 0, grid, threads, smem, 1);
         if (rc) return rc;
-        DEVIS_FUSED_FWD(1, true);
+        if (dtype == DEVIS_MSDA_F16) {
+            if (num_heads == 8) tmsda_fused_fwd_kernel<Elem::F16, 1, true, 512><<<grid, threads, smem, (cudaStream_t)stream>>>(a);
+            else tmsda_fused_fwd_kernel<Elem::F16, 1, true, 0><<<grid, threads, smem, (cudaStream_t)stream>>>(a);
+        } else {
+            DEVIS_FUSED_FWD(1, true);
+        }
         return check_launch(DEVIS_MSDA_KERNEL_FUSED_FWD);
     }
-    // bf16 value: four lanes x 8 channels per (query, head) like msda_fwd8v_kernel
-    if (dtype == DEVIS_MSDA_BF16) {
+    // bf16 / fp16 value: four lanes x 8 channels per (query, head) like msda_fwd8v_kernel
+    if (is_16bit(dtype)) {
         threads = g_tuning[0].load();
         if (threads == 0) threads = num_query >= 1024 ? 128 : 64;
         threads = threads < 32 ? 32 : threads > 256 ? 256 : (threads / 32) * 32;
@@ -721,8 +747,13 @@ int devis_tmsda_fused_forward(const void *value, const int64_t *spatial_shapes_h
         if (chunks * num_heads > 0x7fffffffLL) return DEVIS_MSDA_ERR_TOO_LARGE;
         grid = dim3((unsigned)(chunks * num_heads), (unsigned)num_frames);
         smem = (size_t)(a.n_slots[0] + a.n_slots[1]) * sizeof(int4) + (size_t)(threads / 32) * Tap16::kBytesPerWarp;
-        if (num_heads == 8) tmsda_fused_fwd8_kernel<512><<<grid, threads, smem, (cudaStream_t)stream>>>(a);
-        else tmsda_fused_fwd8_kernel<0><<<grid, threads, smem, (cudaStream_t)stream>>>(a);
+        if (dtype == DEVIS_MSDA_F16) {
+            if (num_heads == 8) tmsda_fused_fwd8_kernel<Elem::F16, 512><<<grid, threads, smem, (cudaStream_t)stream>>>(a);
+            else tmsda_fused_fwd8_kernel<Elem::F16, 0><<<grid, threads, smem, (cudaStream_t)stream>>>(a);
+        } else {
+            if (num_heads == 8) tmsda_fused_fwd8_kernel<Elem::BF16, 512><<<grid, threads, smem, (cudaStream_t)stream>>>(a);
+            else tmsda_fused_fwd8_kernel<Elem::BF16, 0><<<grid, threads, smem, (cudaStream_t)stream>>>(a);
+        }
         return check_launch(DEVIS_MSDA_KERNEL_FUSED_FWD);
     }
     // two queries per lane group for fp32 at encoder sizes, like msda_fwdv_kernel (tuning key 1 overrides)
@@ -780,8 +811,9 @@ int devis_tmsda_fused_backward(const void *value, const int64_t *spatial_shapes_
         if (num_frames > 0 && num_query > 0) {
             const size_t n_go = (size_t)num_frames * num_query * num_heads * channels;
             const int blocks = devis_capi_helper_blocks();
-            if (dtype == DEVIS_MSDA_BF16) absmax_kernel<true><<<blocks, 256, 0, st>>>(grad_output, n_go, slots);
-            else absmax_kernel<false><<<blocks, 256, 0, st>>>(grad_output, n_go, slots);
+            if (dtype == DEVIS_MSDA_BF16) absmax_kernel<Elem::BF16><<<blocks, 256, 0, st>>>(grad_output, n_go, slots);
+            else if (dtype == DEVIS_MSDA_F16) absmax_kernel<Elem::F16><<<blocks, 256, 0, st>>>(grad_output, n_go, slots);
+            else absmax_kernel<Elem::F32><<<blocks, 256, 0, st>>>(grad_output, n_go, slots);
             rc = check_launch(DEVIS_MSDA_KERNEL_AUX);
             if (rc) return rc;
             set_word_kernel<<<1, 1, 0, st>>>(slots + 1, 0x3f800000u);      // max|attn| = 1: softmax outputs
@@ -831,11 +863,13 @@ int devis_tmsda_fused_backward(const void *value, const int64_t *spatial_shapes_
     const bool general = ref_dim == 4 || (a.n_seg > 1 && temporal_ref_mode != 0) || grad_ref;
     if (det) {
         if (general) {
-            if (dtype == DEVIS_MSDA_BF16) tmsda_fused_bwd_kernel<true, false, true, true><<<grid, threads, smem, st>>>(a);
-            else tmsda_fused_bwd_kernel<false, false, true, true><<<grid, threads, smem, st>>>(a);
+            if (dtype == DEVIS_MSDA_BF16) tmsda_fused_bwd_kernel<Elem::BF16, false, true, true><<<grid, threads, smem, st>>>(a);
+            else if (dtype == DEVIS_MSDA_F16) tmsda_fused_bwd_kernel<Elem::F16, false, true, true><<<grid, threads, smem, st>>>(a);
+            else tmsda_fused_bwd_kernel<Elem::F32, false, true, true><<<grid, threads, smem, st>>>(a);
         } else {
-            if (dtype == DEVIS_MSDA_BF16) tmsda_fused_bwd_kernel<true, false, false, true><<<grid, threads, smem, st>>>(a);
-            else tmsda_fused_bwd_kernel<false, false, false, true><<<grid, threads, smem, st>>>(a);
+            if (dtype == DEVIS_MSDA_BF16) tmsda_fused_bwd_kernel<Elem::BF16, false, false, true><<<grid, threads, smem, st>>>(a);
+            else if (dtype == DEVIS_MSDA_F16) tmsda_fused_bwd_kernel<Elem::F16, false, false, true><<<grid, threads, smem, st>>>(a);
+            else tmsda_fused_bwd_kernel<Elem::F32, false, false, true><<<grid, threads, smem, st>>>(a);
         }
         rc = check_launch(DEVIS_MSDA_KERNEL_FUSED_BWD);
         if (rc || n_value == 0) return rc;
@@ -844,13 +878,15 @@ int devis_tmsda_fused_backward(const void *value, const int64_t *spatial_shapes_
         return check_launch(DEVIS_MSDA_KERNEL_AUX);
     }
     if (general) {
-        if (half_acc) tmsda_fused_bwd_kernel<true, true, true><<<grid, threads, smem, st>>>(a);
-        else if (dtype == DEVIS_MSDA_BF16) tmsda_fused_bwd_kernel<true, false, true><<<grid, threads, smem, st>>>(a);
-        else tmsda_fused_bwd_kernel<false, false, true><<<grid, threads, smem, st>>>(a);
+        if (half_acc) tmsda_fused_bwd_kernel<Elem::BF16, true, true><<<grid, threads, smem, st>>>(a);
+        else if (dtype == DEVIS_MSDA_BF16) tmsda_fused_bwd_kernel<Elem::BF16, false, true><<<grid, threads, smem, st>>>(a);
+        else if (dtype == DEVIS_MSDA_F16) tmsda_fused_bwd_kernel<Elem::F16, false, true><<<grid, threads, smem, st>>>(a);
+        else tmsda_fused_bwd_kernel<Elem::F32, false, true><<<grid, threads, smem, st>>>(a);
     } else {
-        if (half_acc) tmsda_fused_bwd_kernel<true, true><<<grid, threads, smem, st>>>(a);
-        else if (dtype == DEVIS_MSDA_BF16) tmsda_fused_bwd_kernel<true><<<grid, threads, smem, st>>>(a);
-        else tmsda_fused_bwd_kernel<false><<<grid, threads, smem, st>>>(a);
+        if (half_acc) tmsda_fused_bwd_kernel<Elem::BF16, true><<<grid, threads, smem, st>>>(a);
+        else if (dtype == DEVIS_MSDA_BF16) tmsda_fused_bwd_kernel<Elem::BF16><<<grid, threads, smem, st>>>(a);
+        else if (dtype == DEVIS_MSDA_F16) tmsda_fused_bwd_kernel<Elem::F16><<<grid, threads, smem, st>>>(a);
+        else tmsda_fused_bwd_kernel<Elem::F32><<<grid, threads, smem, st>>>(a);
     }
     return check_launch(DEVIS_MSDA_KERNEL_FUSED_BWD);
 }

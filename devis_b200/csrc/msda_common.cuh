@@ -12,6 +12,7 @@
 //   tap         one sampling point of one (query, head): a bilinear read of 4 value rows
 #pragma once
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -20,6 +21,11 @@ namespace devis {
 constexpr int kMaxLevels = 16;        // host-side table of the whole-clip op
 constexpr int kMaxFrameTable = 2048;  // T * t_window entries (uint8 each)
 constexpr int kMaxSlots = 1024;       // slots per query (dynamic smem: 16 B each)
+
+// Element type of value / output / grad_output in the lane-group kernels: float, or one of the two 16-bit types
+// (DEVIS_MSDA_BF16, DEVIS_MSDA_F16).  A 16-bit element is widened exactly to fp32 on load, every sum is formed in fp32,
+// and a 16-bit result is rounded to nearest once, on the store.
+enum class Elem { F32, BF16, F16 };
 
 struct Segment {
     const void *loc;   // (outer, Lq, M, n_slots, P, 2)
@@ -420,6 +426,23 @@ __device__ __forceinline__ float4 ldg_bf16x4(const uint2 *p)
     return o;
 }
 
+// four consecutive fp16 channels, widened exactly (cvt.f32.f16)
+__device__ __forceinline__ float4 ldg_f16x4(const uint2 *p)
+{
+    const uint2 r = __ldg(p);
+    const float2 lo = __half22float2(*reinterpret_cast<const __half2 *>(&r.x));
+    const float2 hi = __half22float2(*reinterpret_cast<const __half2 *>(&r.y));
+    return make_float4(lo.x, lo.y, hi.x, hi.y);
+}
+
+// four consecutive channels of a 16-bit element type E
+template <Elem E>
+__device__ __forceinline__ float4 ldg_16x4(const uint2 *p)
+{
+    static_assert(E != Elem::F32, "16-bit element types only");
+    return E == Elem::F16 ? ldg_f16x4(p) : ldg_bf16x4(p);
+}
+
 __device__ __forceinline__ void red_add_f4(float *p, float a, float b, float c, float d)
 {
     asm volatile("red.global.add.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(p), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
@@ -501,15 +524,16 @@ __device__ __forceinline__ void det_add4(long long *p, float sh, float a, float 
     atomicAdd(reinterpret_cast<unsigned long long *>(p) + 3 * LPG, (unsigned long long)__float2ll_rn(d * sh));
 }
 
-// max|x| over n elements (float or bf16) into *slot, as the bits of a non-negative float (atomicMax on the
+// max|x| over n elements (float, bf16 or fp16) into *slot, as the bits of a non-negative float (atomicMax on the
 // bit pattern is exact and order independent)
-template <bool BF16>
+template <Elem E>
 __global__ void __launch_bounds__(256) absmax_kernel(const void *x, size_t n, unsigned *slot)
 {
     float m = 0.f;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
-        const float v = BF16 ? __bfloat162float(reinterpret_cast<const __nv_bfloat16 *>(x)[i])
-                             : reinterpret_cast<const float *>(x)[i];
+        const float v = E == Elem::BF16  ? __bfloat162float(reinterpret_cast<const __nv_bfloat16 *>(x)[i])
+                        : E == Elem::F16 ? __half2float(reinterpret_cast<const __half *>(x)[i])
+                                         : reinterpret_cast<const float *>(x)[i];
         m = fmaxf(m, fabsf(v));
     }
 #pragma unroll
@@ -544,6 +568,42 @@ __device__ __forceinline__ uint2 pack_bf16x4(float4 v)
     r.x = *reinterpret_cast<const unsigned *>(&lo);
     r.y = *reinterpret_cast<const unsigned *>(&hi);
     return r;
+}
+
+// round to nearest, once (cvt.rn.f16x2.f32); fp32 values beyond the fp16 range become +-inf, as in a torch cast
+__device__ __forceinline__ uint2 pack_f16x4(float4 v)
+{
+    const __half2 lo = __floats2half2_rn(v.x, v.y), hi = __floats2half2_rn(v.z, v.w);
+    uint2 r;
+    r.x = *reinterpret_cast<const unsigned *>(&lo);
+    r.y = *reinterpret_cast<const unsigned *>(&hi);
+    return r;
+}
+
+template <Elem E>
+__device__ __forceinline__ uint2 pack_16x4(float4 v)
+{
+    static_assert(E != Elem::F32, "16-bit element types only");
+    return E == Elem::F16 ? pack_f16x4(v) : pack_bf16x4(v);
+}
+
+// eight raw 16-bit channels (one 16-byte gather) widened exactly to fp32; bf16 -> fp32 is a shift / mask
+template <Elem E>
+__device__ __forceinline__ void unpack_16x8(const uint4 &raw, float (&v)[8])
+{
+    static_assert(E != Elem::F32, "16-bit element types only");
+    const unsigned w[4] = {raw.x, raw.y, raw.z, raw.w};
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        if (E == Elem::F16) {
+            const float2 f = __half22float2(*reinterpret_cast<const __half2 *>(&w[i]));
+            v[2 * i] = f.x;
+            v[2 * i + 1] = f.y;
+        } else {
+            v[2 * i] = __uint_as_float(w[i] << 16);
+            v[2 * i + 1] = __uint_as_float(w[i] & 0xffff0000u);
+        }
+    }
 }
 
 }  // namespace devis

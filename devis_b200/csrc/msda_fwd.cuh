@@ -43,7 +43,7 @@ struct FwdArgs {
     const int *q_perm;  // optional query visiting order (length Lq), nullptr = identity
 };
 
-template <bool BF16, int LPG, int QPG, class SlotSrc>
+template <Elem E, int LPG, int QPG, class SlotSrc>
 __global__ void __launch_bounds__(256, DEVIS_FWD_MIN_BLOCKS) msda_fwd_kernel(const FwdArgs<SlotSrc> a)
 {
     using X = TapExchange<LPG>;
@@ -69,7 +69,7 @@ __global__ void __launch_bounds__(256, DEVIS_FWD_MIN_BLOCKS) msda_fwd_kernel(con
     }
 
     // value row = M*LPG channel quads; this lane reads quad (m*LPG + j) of every row it touches
-    constexpr unsigned kQuadBytes = BF16 ? 8u : 16u;
+    constexpr unsigned kQuadBytes = E != Elem::F32 ? 8u : 16u;
     const unsigned rowbytes = (unsigned)(M * LPG) * kQuadBytes;
     const char *vbase = reinterpret_cast<const char *>(a.value) + (size_t)(m * LPG + j) * kQuadBytes;
     // keep the per-lane base as ONE 64-bit register pair: each corner address is then base + u32 offset
@@ -115,11 +115,11 @@ __global__ void __launch_bounds__(256, DEVIS_FWD_MIN_BLOCKS) msda_fwd_kernel(con
                     for (int u = 0; u < TB; ++u) X::fetch(buf, j0 + u, g, off[u], c[u]);
 #pragma unroll
                     for (int u = 0; u < TB; ++u) {
-                        if (BF16) {
-                            v[u][0] = ldg_bf16x4(reinterpret_cast<const uint2 *>(vbase + off[u].x));
-                            v[u][1] = ldg_bf16x4(reinterpret_cast<const uint2 *>(vbase + off[u].y));
-                            v[u][2] = ldg_bf16x4(reinterpret_cast<const uint2 *>(vbase + off[u].z));
-                            v[u][3] = ldg_bf16x4(reinterpret_cast<const uint2 *>(vbase + off[u].w));
+                        if constexpr (E != Elem::F32) {
+                            v[u][0] = ldg_16x4<E>(reinterpret_cast<const uint2 *>(vbase + off[u].x));
+                            v[u][1] = ldg_16x4<E>(reinterpret_cast<const uint2 *>(vbase + off[u].y));
+                            v[u][2] = ldg_16x4<E>(reinterpret_cast<const uint2 *>(vbase + off[u].z));
+                            v[u][3] = ldg_16x4<E>(reinterpret_cast<const uint2 *>(vbase + off[u].w));
                         } else {
                             v[u][0] = ldg_f4(reinterpret_cast<const float4 *>(vbase + off[u].x));
                             v[u][1] = ldg_f4(reinterpret_cast<const float4 *>(vbase + off[u].y));
@@ -144,8 +144,8 @@ __global__ void __launch_bounds__(256, DEVIS_FWD_MIN_BLOCKS) msda_fwd_kernel(con
     for (int i = 0; i < QPG; ++i) {
         if (!qlive[i]) continue;
         const size_t row = ((size_t)outer * Lq + q[i]) * M + m;
-        if (BF16)
-            reinterpret_cast<uint2 *>(a.out)[row * LPG + j] = pack_bf16x4(acc[i]);
+        if constexpr (E != Elem::F32)
+            reinterpret_cast<uint2 *>(a.out)[row * LPG + j] = pack_16x4<E>(acc[i]);
         else
             st_stream_f4(reinterpret_cast<float4 *>(a.out) + row * LPG + j, acc[i]);
     }
@@ -211,6 +211,15 @@ __device__ __forceinline__ void ldg_bf16x4_if(float4 &v, const char *p, unsigned
     v.z = __uint_as_float(hi << 16);
     v.w = __uint_as_float(hi & 0xffff0000u);
 }
+// four consecutive fp16 channels, widened (the conversion is exact and cannot fault; only the FFMAs carry the predicate)
+__device__ __forceinline__ void ldg_f16x4_if(float4 &v, const char *p, unsigned live)
+{
+    unsigned lo = __float_as_uint(v.x), hi = __float_as_uint(v.z);
+    asm("{\n\t.reg .pred p;\n\tsetp.ne.u32 p, %3, 0;\n\t@p ld.global.nc.v2.u32 {%0,%1}, [%2];\n\t}" : "+r"(lo), "+r"(hi) : "l"(p), "r"(live));
+    const float2 a = __half22float2(*reinterpret_cast<const __half2 *>(&lo));
+    const float2 b = __half22float2(*reinterpret_cast<const __half2 *>(&hi));
+    v = make_float4(a.x, a.y, b.x, b.y);
+}
 __device__ __forceinline__ void fma4_if(float4 &acc, float c, const float4 &v, unsigned live)
 {
     asm("{\n\t.reg .pred p;\n\tsetp.ne.u32 p, %9, 0;\n\t"
@@ -220,7 +229,7 @@ __device__ __forceinline__ void fma4_if(float4 &acc, float c, const float4 &v, u
 }
 
 // TB = taps whose gathers are in flight together (v: their destinations, owned by the kernel)
-template <bool BF16, int ROWB, int TB>
+template <Elem E, int ROWB, int TB>
 __device__ __forceinline__ void consume_tap16v(const float *buf, int g, unsigned rowbytes_rt, unsigned pitch_lo,
                                                unsigned pitch_hi, const char *vbase, float4 &acc, float4 (&v)[TB][4])
 {
@@ -248,7 +257,8 @@ __device__ __forceinline__ void consume_tap16v(const float *buf, int g, unsigned
 #pragma unroll
             for (int e = 0; e < 4; ++e) {
                 const char *addr = ((e & 2) ? pb[u] : pt[u]) + ((e & 1) ? rowb : 0u);
-                if (BF16) ldg_bf16x4_if(v[u][e], addr, flags[u] & (1u << e));
+                if (E == Elem::BF16) ldg_bf16x4_if(v[u][e], addr, flags[u] & (1u << e));
+                else if (E == Elem::F16) ldg_f16x4_if(v[u][e], addr, flags[u] & (1u << e));
                 else ldg_f4_if(v[u][e], addr, flags[u] & (1u << e));
             }
 #pragma unroll
@@ -268,7 +278,7 @@ __device__ __forceinline__ uint4 make_tap16v(const TapGeomV &t, float w, unsigne
     return rec;
 }
 
-template <bool BF16, int QPG, class SlotSrc, int ROWB>
+template <Elem E, int QPG, class SlotSrc, int ROWB>
 __global__ void __launch_bounds__(DEVIS_FWDV_MAXT, DEVIS_FWDV_MIN_BLOCKS) msda_fwdv_kernel(const FwdArgs<SlotSrc> a)
 {
     constexpr int LPG = 8;
@@ -290,7 +300,7 @@ __global__ void __launch_bounds__(DEVIS_FWDV_MAXT, DEVIS_FWDV_MIN_BLOCKS) msda_f
         q[i] = qlive[i] ? (a.q_perm ? a.q_perm[qi] : qi) : 0;
     }
 
-    constexpr unsigned kQuadBytes = BF16 ? 8u : 16u;
+    constexpr unsigned kQuadBytes = E != Elem::F32 ? 8u : 16u;
     const unsigned rowbytes = ROWB ? (unsigned)ROWB : (unsigned)(M * LPG) * kQuadBytes;
     const char *vbase = reinterpret_cast<const char *>(a.value) + (size_t)(m * LPG + j) * kQuadBytes;
     asm volatile("" : "+l"(vbase));
@@ -350,7 +360,7 @@ __global__ void __launch_bounds__(DEVIS_FWDV_MAXT, DEVIS_FWDV_MIN_BLOCKS) msda_f
                 parity ^= 1;
                 *reinterpret_cast<uint4 *>(buf + Tap16x8::word(j, g)) = make_tap16v(t, cur[i].w, rowbytes);
                 __syncwarp();
-                consume_tap16v<BF16, ROWB, DEVIS_FWDV_TB>(buf, g, rowbytes, pitch_lo, pitch_hi, vbase, acc[i], v);
+                consume_tap16v<E, ROWB, DEVIS_FWDV_TB>(buf, g, rowbytes, pitch_lo, pitch_hi, vbase, acc[i], v);
             }
         }
         slot_base += a.seg[sg].n_slots;
@@ -360,8 +370,8 @@ __global__ void __launch_bounds__(DEVIS_FWDV_MAXT, DEVIS_FWDV_MIN_BLOCKS) msda_f
     for (int i = 0; i < QPG; ++i) {
         if (!qlive[i]) continue;
         const size_t row = ((size_t)outer * Lq + q[i]) * M + m;
-        if (BF16)
-            reinterpret_cast<uint2 *>(a.out)[row * LPG + j] = pack_bf16x4(acc[i]);
+        if constexpr (E != Elem::F32)
+            reinterpret_cast<uint2 *>(a.out)[row * LPG + j] = pack_16x4<E>(acc[i]);
         else
             st_stream_f4(reinterpret_cast<float4 *>(a.out) + row * LPG + j, acc[i]);
     }
@@ -391,13 +401,13 @@ __device__ __forceinline__ void ldg_u4_if(uint4 &v, const char *p, unsigned live
         : "+r"(v.x), "+r"(v.y), "+r"(v.z), "+r"(v.w)
         : "l"(p), "r"(live));
 }
-__device__ __forceinline__ void fma8_bf16_if(float (&acc)[8], float c, const uint4 &raw, unsigned live)
+template <Elem E>
+__device__ __forceinline__ void fma8_16_if(float (&acc)[8], float c, const uint4 &raw, unsigned live)
 {
-    // bf16 -> fp32 is a shift / mask; done unconditionally (cheap, no faults), only the FFMAs carry the predicate
-    const float v0 = __uint_as_float(raw.x << 16), v1 = __uint_as_float(raw.x & 0xffff0000u);
-    const float v2 = __uint_as_float(raw.y << 16), v3 = __uint_as_float(raw.y & 0xffff0000u);
-    const float v4 = __uint_as_float(raw.z << 16), v5 = __uint_as_float(raw.z & 0xffff0000u);
-    const float v6 = __uint_as_float(raw.w << 16), v7 = __uint_as_float(raw.w & 0xffff0000u);
+    // the widening is done unconditionally (cheap, exact, no faults), only the FFMAs carry the predicate
+    float u[8];
+    unpack_16x8<E>(raw, u);
+    const float v0 = u[0], v1 = u[1], v2 = u[2], v3 = u[3], v4 = u[4], v5 = u[5], v6 = u[6], v7 = u[7];
     asm("{\n\t.reg .pred p;\n\tsetp.ne.u32 p, %17, 0;\n\t"
         "@p fma.rn.f32 %0, %8, %9, %0;\n\t@p fma.rn.f32 %1, %8, %10, %1;\n\t@p fma.rn.f32 %2, %8, %11, %2;\n\t"
         "@p fma.rn.f32 %3, %8, %12, %3;\n\t@p fma.rn.f32 %4, %8, %13, %4;\n\t@p fma.rn.f32 %5, %8, %14, %5;\n\t"
@@ -406,8 +416,8 @@ __device__ __forceinline__ void fma8_bf16_if(float (&acc)[8], float c, const uin
         : "f"(c), "f"(v0), "f"(v1), "f"(v2), "f"(v3), "f"(v4), "f"(v5), "f"(v6), "f"(v7), "r"(live));
 }
 
-// one exchange of 4 published records (4 lanes x 8 bf16 channels per row), dead corners skipped
-template <int ROWB>
+// one exchange of 4 published records (4 lanes x 8 16-bit channels per row), dead corners skipped
+template <Elem E, int ROWB>
 __device__ __forceinline__ void consume_tap16x4v(const float *buf, int g, unsigned rowbytes_rt, unsigned pitch,
                                                  const char *vbase, float (&acc)[8], uint4 (&v)[4])
 {
@@ -423,16 +433,18 @@ __device__ __forceinline__ void consume_tap16x4v(const float *buf, int g, unsign
 #pragma unroll
         for (int e = 0; e < 4; ++e) ldg_u4_if(v[e], ((e & 2) ? pb : pt) + ((e & 1) ? rowb : 0u), r.x & (1u << e));
 #pragma unroll
-        for (int e = 0; e < 4; ++e) fma8_bf16_if(acc, c[e], v[e], r.x & (1u << e));
+        for (int e = 0; e < 4; ++e) fma8_16_if<E>(acc, c[e], v[e], r.x & (1u << e));
     }
 }
 
 // (no minimum-blocks hint: ptxas settles at 62-64 registers, 359 us; a hint of 1 made it unroll to 184 registers and 711 us.
 // The fp32 form of this shape -- 32-byte predicated gathers, LDG.E.256 -- was measured at 527-543 us against 478 us for
 // msda_fwdv_kernel and is not kept, profiles/r2s_fwd_wide_f32_variants.json)
-template <int QPG, class SlotSrc, int ROWB>
+// E: BF16 or F16 (64-byte rows of a head either way)
+template <Elem E, int QPG, class SlotSrc, int ROWB>
 __global__ void __launch_bounds__(256) msda_fwd8v_kernel(const FwdArgs<SlotSrc> a)
 {
+    static_assert(E != Elem::F32, "16-bit value only");
     constexpr int LPG = 4;
     extern __shared__ int4 s_slot[];
     const int outer = blockIdx.y;
@@ -452,7 +464,7 @@ __global__ void __launch_bounds__(256) msda_fwd8v_kernel(const FwdArgs<SlotSrc> 
         q[i] = qlive[i] ? (a.q_perm ? a.q_perm[qi] : qi) : 0;
     }
 
-    constexpr unsigned kLaneBytes = 16u;                       // 8 bf16 channels
+    constexpr unsigned kLaneBytes = 16u;                       // 8 16-bit channels
     const unsigned rowbytes = ROWB ? (unsigned)ROWB : (unsigned)(M * LPG) * kLaneBytes;
     const char *vbase = reinterpret_cast<const char *>(a.value) + (size_t)(m * LPG + j) * kLaneBytes;
     asm volatile("" : "+l"(vbase));
@@ -462,7 +474,7 @@ __global__ void __launch_bounds__(256) msda_fwd8v_kernel(const FwdArgs<SlotSrc> 
     for (int i = 0; i < QPG; ++i)
 #pragma unroll
         for (int c = 0; c < 8; ++c) acc[i][c] = 0.f;
-    uint4 v[4];                                                // gather destinations (see ldg_f4_if): raw bf16x8 per corner
+    uint4 v[4];                                                // gather destinations (see ldg_f4_if): 8 raw channels per corner
 #pragma unroll
     for (int e = 0; e < 4; ++e) v[e] = make_uint4(0u, 0u, 0u, 0u);
 
@@ -489,7 +501,7 @@ __global__ void __launch_bounds__(256) msda_fwd8v_kernel(const FwdArgs<SlotSrc> 
                 parity ^= 1;
                 *reinterpret_cast<uint4 *>(buf + Tap16::word(j, g)) = make_tap16v(t, w, rowbytes);
                 __syncwarp();
-                consume_tap16x4v<ROWB>(buf, g, rowbytes, pitch, vbase, acc[i], v);
+                consume_tap16x4v<E, ROWB>(buf, g, rowbytes, pitch, vbase, acc[i], v);
             }
         }
         slot_base += a.seg[sg].n_slots;
@@ -499,8 +511,8 @@ __global__ void __launch_bounds__(256) msda_fwd8v_kernel(const FwdArgs<SlotSrc> 
     for (int i = 0; i < QPG; ++i) {
         if (!qlive[i]) continue;
         const size_t row = ((size_t)outer * Lq + q[i]) * M + m;
-        const uint2 lo = pack_bf16x4(make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]));
-        const uint2 hi = pack_bf16x4(make_float4(acc[i][4], acc[i][5], acc[i][6], acc[i][7]));
+        const uint2 lo = pack_16x4<E>(make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]));
+        const uint2 hi = pack_16x4<E>(make_float4(acc[i][4], acc[i][5], acc[i][6], acc[i][7]));
         reinterpret_cast<uint4 *>(a.out)[row * LPG + j] = make_uint4(lo.x, lo.y, hi.x, hi.y);
     }
 }

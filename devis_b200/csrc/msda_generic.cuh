@@ -1,4 +1,4 @@
-// msda_generic.cuh -- any-channel-count, any-dtype (fp32 / fp64 / bf16) kernels.
+// msda_generic.cuh -- any-channel-count, any-dtype (fp32 / fp64 / bf16 / fp16) kernels.
 //
 // The reference instantiates its kernels for float and double and for every channel count
 // (cuda/ms_deform_attn_cuda.cu:64,134; the backward picks one of six kernels by D,
@@ -36,6 +36,13 @@ template <> struct Scalar<__nv_bfloat16> {
     {
         reinterpret_cast<__nv_bfloat16 *>(p)[i] = __float2bfloat16_rn(v);
     }
+    static __device__ __forceinline__ float coord(float l, int n) { return __fadd_rn(__fmul_rn(l, (float)n), -0.5f); }
+};
+
+template <> struct Scalar<__half> {
+    using C = float;
+    static __device__ __forceinline__ float load(const void *p, size_t i) { return __half2float(reinterpret_cast<const __half *>(p)[i]); }
+    static __device__ __forceinline__ void store(void *p, size_t i, float v) { reinterpret_cast<__half *>(p)[i] = __float2half_rn(v); }
     static __device__ __forceinline__ float coord(float l, int n) { return __fadd_rn(__fmul_rn(l, (float)n), -0.5f); }
 };
 
@@ -130,7 +137,7 @@ __global__ void __launch_bounds__(128) msda_bwd_generic_kernel(const BwdArgs<Slo
     const int q = (int)(item / M), m = (int)(item - (long long)q * M);
     const size_t row = ((size_t)outer * Lq + q) * M + m;
     const size_t ps = (size_t)M * D;
-    C *gv = reinterpret_cast<C *>(a.grad_value);  // float for fp32/bf16, double for fp64
+    C *gv = reinterpret_cast<C *>(a.grad_value);  // float for fp32/bf16/fp16, double for fp64
     long long *det = a.det.acc;                    // deterministic fixed-point accumulators (never with fp64)
     const float det_sh = det ? ldexpf(1.f, kDetFracBits - det_exponent(a.det.max_bits)) : 0.f;
     auto scatter = [&](long long r, C v) {

@@ -193,7 +193,7 @@ __device__ __forceinline__ void raw_to_operands(const FusedArgs &a, int sg, cons
 #ifndef DEVIS_FUSED_FWD_TB
 #define DEVIS_FUSED_FWD_TB 2
 #endif
-template <bool BF16, int QPG, bool GEN = false, int ROWB = 0>
+template <Elem E, int QPG, bool GEN = false, int ROWB = 0>
 __global__ void __launch_bounds__(256, DEVIS_FUSED_FWD_MIN_BLOCKS) tmsda_fused_fwd_kernel(const FusedArgs a)
 {
     constexpr int LPG = 8;
@@ -217,7 +217,7 @@ __global__ void __launch_bounds__(256, DEVIS_FUSED_FWD_MIN_BLOCKS) tmsda_fused_f
         row[i] = qrow[i] * M + m;
     }
 
-    constexpr unsigned kQuadBytes = BF16 ? 8u : 16u;
+    constexpr unsigned kQuadBytes = E != Elem::F32 ? 8u : 16u;
     const unsigned rowbytes = (unsigned)(M * LPG) * kQuadBytes;
     const char *vbase = reinterpret_cast<const char *>(a.value) + (size_t)(m * LPG + j) * kQuadBytes;
     asm volatile("" : "+l"(vbase));
@@ -274,7 +274,7 @@ __global__ void __launch_bounds__(256, DEVIS_FUSED_FWD_MIN_BLOCKS) tmsda_fused_f
                 const TapGeomV t = tap_geometry_v(x, y, sl, live);
                 *reinterpret_cast<uint4 *>(buf + Tap16x8::word(j, g)) = make_tap16v(t, w, rowbytes);
                 __syncwarp();
-                consume_tap16v<BF16, ROWB, DEVIS_FUSED_FWD_TB>(buf, g, rowbytes, pitch_lo, pitch_hi, vbase, acc[i], v);
+                consume_tap16v<E, ROWB, DEVIS_FUSED_FWD_TB>(buf, g, rowbytes, pitch_lo, pitch_hi, vbase, acc[i], v);
             }
         }
         slot_base += a.n_slots[sg];
@@ -282,20 +282,20 @@ __global__ void __launch_bounds__(256, DEVIS_FUSED_FWD_MIN_BLOCKS) tmsda_fused_f
 #pragma unroll
     for (int i = 0; i < QPG; ++i) {
         if (!qlive[i]) continue;
-        if (BF16)
-            reinterpret_cast<uint2 *>(a.out)[row[i] * LPG + j] = pack_bf16x4(acc[i]);
+        if constexpr (E != Elem::F32)
+            reinterpret_cast<uint2 *>(a.out)[row[i] * LPG + j] = pack_16x4<E>(acc[i]);
         else
             st_stream_f4(reinterpret_cast<float4 *>(a.out) + row[i] * LPG + j, acc[i]);
     }
 }
 
-// Four lanes per (query, head), 8 channels per lane (msda_fwd8v_kernel's shape): the forward of choice for bf16 value,
-// whose 64-byte rows cost 0.75 instead of 1.0 data-pipe cycles when 4 lanes fetch 16 bytes each.
-// bf16 value only (the fp32 form of this shape loses to the eight-lane kernel); dead corners skipped, consume_tap16x4v
-template <int ROWB>
+// Four lanes per (query, head), 8 channels per lane (msda_fwd8v_kernel's shape): the forward of choice for 16-bit value
+// (bf16 or fp16), whose 64-byte rows cost 0.75 instead of 1.0 data-pipe cycles when 4 lanes fetch 16 bytes each.
+// 16-bit value only (the fp32 form of this shape loses to the eight-lane kernel); dead corners skipped, consume_tap16x4v
+template <Elem E, int ROWB>
 __global__ void __launch_bounds__(256) tmsda_fused_fwd8_kernel(const FusedArgs a)
 {
-    constexpr bool BF16 = true;
+    static_assert(E != Elem::F32, "16-bit value only");
     constexpr int LPG = 4;
     extern __shared__ int4 s_slot[];
     const int outer = blockIdx.y, n_slots_total = a.n_slots[0] + (a.n_seg > 1 ? a.n_slots[1] : 0);
@@ -310,7 +310,7 @@ __global__ void __launch_bounds__(256) tmsda_fused_fwd8_kernel(const FusedArgs a
     const int q = qlive ? (a.q_perm ? a.q_perm[qi] : qi) : 0;
     const size_t qrow = (size_t)outer * Lq + q, row = qrow * M + m;
 
-    constexpr unsigned kLaneBytes = BF16 ? 16u : 32u;      // 8 channels
+    constexpr unsigned kLaneBytes = 16u;                   // 8 channels
     const unsigned rowbytes = (unsigned)(M * LPG) * kLaneBytes;
     const char *vbase = reinterpret_cast<const char *>(a.value) + (size_t)(m * LPG + j) * kLaneBytes;
     asm volatile("" : "+l"(vbase));
@@ -342,20 +342,14 @@ __global__ void __launch_bounds__(256) tmsda_fused_fwd8_kernel(const FusedArgs a
             const TapGeomV t = tap_geometry_v(x, y, sl, qlive);
             *reinterpret_cast<uint4 *>(buf + Tap16::word(j, g)) = make_tap16v(t, w, rowbytes);
             __syncwarp();
-            consume_tap16x4v<ROWB>(buf, g, rowbytes, pitch, vbase, acc, v);
+            consume_tap16x4v<E, ROWB>(buf, g, rowbytes, pitch, vbase, acc, v);
         }
         slot_base += a.n_slots[sg];
     }
     if (qlive) {
-        if (BF16) {
-            const uint2 lo = pack_bf16x4(make_float4(acc[0], acc[1], acc[2], acc[3]));
-            const uint2 hi = pack_bf16x4(make_float4(acc[4], acc[5], acc[6], acc[7]));
-            reinterpret_cast<uint4 *>(a.out)[row * LPG + j] = make_uint4(lo.x, lo.y, hi.x, hi.y);
-        } else {
-            float4 *o = reinterpret_cast<float4 *>(a.out) + (row * LPG + j) * 2;
-            o[0] = make_float4(acc[0], acc[1], acc[2], acc[3]);
-            o[1] = make_float4(acc[4], acc[5], acc[6], acc[7]);
-        }
+        const uint2 lo = pack_16x4<E>(make_float4(acc[0], acc[1], acc[2], acc[3]));
+        const uint2 hi = pack_16x4<E>(make_float4(acc[4], acc[5], acc[6], acc[7]));
+        reinterpret_cast<uint4 *>(a.out)[row * LPG + j] = make_uint4(lo.x, lo.y, hi.x, hi.y);
     }
 }
 
@@ -364,7 +358,7 @@ __global__ void __launch_bounds__(256) tmsda_fused_fwd8_kernel(const FusedArgs a
 // fixed-point accumulators with integer reductions (det_add4, msda_common.cuh) exactly as in msda_bwd_kernel, with the
 // bound max|attn| = 1 (the weights are softmax outputs here); every other gradient of this kernel is written once, in a
 // fixed order, so the whole backward is bit-identical run to run.
-template <bool BF16, bool HALF_ACC = false, bool GEN = false, bool DET = false>
+template <Elem E, bool HALF_ACC = false, bool GEN = false, bool DET = false>
 __global__ void __launch_bounds__(256, DEVIS_BWD_MIN_BLOCKS) tmsda_fused_bwd_kernel(const FusedArgs a)
 {
     static_assert(!(DET && HALF_ACC), "deterministic mode accumulates in fixed point");
@@ -391,17 +385,18 @@ __global__ void __launch_bounds__(256, DEVIS_BWD_MIN_BLOCKS) tmsda_fused_bwd_ker
     const size_t qrow = (size_t)outer * Lq + q, row = qrow * M + m;
 
     float4 gg = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (qlive)
-        gg = BF16 ? ldg_bf16x4(reinterpret_cast<const uint2 *>(a.grad_out) + row * LPG + j)
-                  : ldg_f4(reinterpret_cast<const float4 *>(a.grad_out) + row * LPG + j);
+    if (qlive) {
+        if constexpr (E != Elem::F32) gg = ldg_16x4<E>(reinterpret_cast<const uint2 *>(a.grad_out) + row * LPG + j);
+        else gg = ldg_f4(reinterpret_cast<const float4 *>(a.grad_out) + row * LPG + j);
+    }
 
-    constexpr unsigned kQuadBytes = BF16 ? 8u : 16u;
+    constexpr unsigned kQuadBytes = E != Elem::F32 ? 8u : 16u;
     const unsigned rowbytes = (unsigned)(M * LPG) * kQuadBytes;
     const char *vbase = reinterpret_cast<const char *>(a.value) + (size_t)(m * LPG + j) * kQuadBytes;
     asm volatile("" : "+l"(vbase));
-    static_assert(!HALF_ACC || BF16, "bf16 accumulation needs bf16 value");
+    static_assert(!HALF_ACC || E == Elem::BF16, "bf16 accumulation needs bf16 value");
     char *gvb = a.grad_value ? reinterpret_cast<char *>(a.grad_value) + (size_t)(m * LPG + j) * (HALF_ACC ? 8u : 16u) : nullptr;
-    constexpr unsigned kGvShift = (BF16 && !HALF_ACC) ? 1u : 0u;
+    constexpr unsigned kGvShift = (E != Elem::F32 && !HALF_ACC) ? 1u : 0u;
     // deterministic mode: 8-byte accumulators, channels of a (row, head) permuted as in det_add4 (lane j starts at word j)
     char *detb = DET ? reinterpret_cast<char *>(a.det.acc) + (size_t)(m * LPG) * 32u + (size_t)j * 8u : nullptr;
     const float det_sh = DET ? ldexpf(1.f, kDetFracBits - det_exponent(a.det.max_bits)) : 0.f;
@@ -439,11 +434,11 @@ __global__ void __launch_bounds__(256, DEVIS_BWD_MIN_BLOCKS) tmsda_fused_bwd_ker
                 float4 c;
                 X::fetch(buf, jj, g, off, c);
                 float4 v00, v01, v10, v11;
-                if (BF16) {
-                    v00 = ldg_bf16x4(reinterpret_cast<const uint2 *>(vbase + off.x));
-                    v01 = ldg_bf16x4(reinterpret_cast<const uint2 *>(vbase + off.y));
-                    v10 = ldg_bf16x4(reinterpret_cast<const uint2 *>(vbase + off.z));
-                    v11 = ldg_bf16x4(reinterpret_cast<const uint2 *>(vbase + off.w));
+                if constexpr (E != Elem::F32) {
+                    v00 = ldg_16x4<E>(reinterpret_cast<const uint2 *>(vbase + off.x));
+                    v01 = ldg_16x4<E>(reinterpret_cast<const uint2 *>(vbase + off.y));
+                    v10 = ldg_16x4<E>(reinterpret_cast<const uint2 *>(vbase + off.z));
+                    v11 = ldg_16x4<E>(reinterpret_cast<const uint2 *>(vbase + off.w));
                 } else {
                     v00 = ldg_f4(reinterpret_cast<const float4 *>(vbase + off.x));
                     v01 = ldg_f4(reinterpret_cast<const float4 *>(vbase + off.y));

@@ -16,7 +16,10 @@ from torch.autograd.function import once_differentiable
 from .. import _lib
 from .. import MultiScaleDeformableAttention as MSDA
 
-_DTYPES = {torch.float32: _lib.F32, torch.float64: _lib.F64, torch.bfloat16: _lib.BF16}
+# float16 value (what torch.autocast("cuda") hands the op by default) is served like bfloat16: 16-bit value, output and
+# grad_output, float32 locations, weights and gradients
+_DTYPES = {torch.float32: _lib.F32, torch.float64: _lib.F64, torch.bfloat16: _lib.BF16, torch.float16: _lib.F16}
+_16BIT = (torch.bfloat16, torch.float16)
 
 
 def _ptr(t):
@@ -24,7 +27,7 @@ def _ptr(t):
 
 
 def _aux(t, value):
-    want = torch.float32 if value.dtype == torch.bfloat16 else value.dtype
+    want = torch.float32 if value.dtype in _16BIT else value.dtype
     t = t if t.dtype == want else t.to(want)
     return t if t.is_contiguous() else t.contiguous()
 
@@ -88,7 +91,7 @@ class TemporalMSDeformAttnFunction(Function):
         gout = gout if gout.is_contiguous() else gout.contiguous()
         need_gv = ctx.needs_input_grad[0]
         half_acc = need_gv and MSDA.bf16_accumulate_enabled(value)
-        acc_dtype = torch.float32 if (value.dtype == torch.bfloat16 and not half_acc) else value.dtype
+        acc_dtype = torch.float32 if (value.dtype in _16BIT and not half_acc) else value.dtype
         gv = torch.empty(value.shape, dtype=acc_dtype, device=value.device) if need_gv else None
         glc, gac = torch.empty_like(lc), torch.empty_like(ac)
         glt = torch.empty_like(lt) if has_t else None
@@ -127,7 +130,7 @@ class TemporalMSDeformAttnFusedFunction(Function):
     Whole-clip temporal attention straight from the Linear outputs: the joint softmax over all taps and the sampling
     location arithmetic (encoder: ms_deform_attn.py:240-260, 437-452; decoder: :320-404, points or boxes, instance
     aware or not) happen inside the kernels, and the backward returns the gradients of the raw offsets and logits (and of
-    the reference points when they require grad).  value (T,S,M,32) fp32|bf16; ref (T,Lq,L,2|4); off_curr
+    the reference points when they require grad).  value (T,S,M,32) fp32|bf16|fp16; ref (T,Lq,L,2|4); off_curr
     (T,Lq,M,L,Pc,2); logit_curr (T,Lq,M,L*Pc); off_temporal (T,Lq,M,Wt*L,Pt,2); logit_temporal (T,Lq,M,Wt*L*Pt).
     temporal_ref_mode: _lib.TREF_LEVEL0 (encoder) | TREF_OWN | TREF_SAMPLED (decoder, instance aware).
     want_sampling: also return the sampling locations and softmax weights the kernel computed (non-differentiable
@@ -136,7 +139,7 @@ class TemporalMSDeformAttnFusedFunction(Function):
     @staticmethod
     def supported(value, reference_points, n_curr_points=4, n_temporal_points=4):
         """`value`: the projected value tensor (T,S,M,D) (or any tensor with its device, dtype and shape)"""
-        return (value.is_cuda and value.dtype in (torch.float32, torch.bfloat16) and value.shape[-1] == 32
+        return (value.is_cuda and value.dtype in (torch.float32,) + _16BIT and value.shape[-1] == 32
                 and n_curr_points % 4 == 0 and n_temporal_points % 4 == 0
                 and reference_points.shape[-1] in (2, 4) and value.numel() * value.element_size() < (1 << 31)
                 # deterministic mode: grad_value goes through fixed point inside the kernel; d/d(reference points) is a
@@ -148,7 +151,7 @@ class TemporalMSDeformAttnFusedFunction(Function):
                 temporal_ref_mode=_lib.TREF_LEVEL0, want_sampling=False):
         if not value.is_cuda:
             raise RuntimeError("Not implemented on the CPU")
-        if value.dtype not in (torch.float32, torch.bfloat16):
+        if value.dtype not in (torch.float32,) + _16BIT:
             raise RuntimeError(f'"temporal_ms_deform_attn_fused" not implemented for \'{value.dtype}\'')
         f32 = lambda t: (t if t.dtype == torch.float32 else t.float()).contiguous()
         value = value if value.is_contiguous() else value.contiguous()

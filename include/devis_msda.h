@@ -34,13 +34,15 @@
 extern "C" {
 #endif
 
-#define DEVIS_MSDA_ABI_VERSION 4
+#define DEVIS_MSDA_ABI_VERSION 5
 
 /* element types of value / output / grad_output */
 #define DEVIS_MSDA_F32 0  /* value, loc, weights, outputs and all gradients float            */
 #define DEVIS_MSDA_F64 1  /* everything double (the reference's gradcheck type, test.py:74)   */
 #define DEVIS_MSDA_BF16 2 /* extension: value/output/grad_output bf16; sampling locations,    */
                           /* attention weights and ALL gradients (incl. grad_value) float     */
+#define DEVIS_MSDA_F16 3  /* extension: value/output/grad_output IEEE half (torch.autocast's  */
+                          /* default); everything else float, exactly as for DEVIS_MSDA_BF16 */
 
 /* error codes */
 #define DEVIS_MSDA_OK 0
@@ -61,6 +63,8 @@ extern "C" {
                                            /* bf16 tensor like value, accumulated with packed bf16 reductions (every partial  */
                                            /* sum rounds to bf16, like PyTorch's bf16 atomicAdd scatters); halves the bytes   */
                                            /* the scatter moves.  Default (flag clear): float grad_value, float accumulation. */
+                                           /* With DEVIS_MSDA_F16: DEVIS_MSDA_ERR_UNSUPPORTED (fp16's range makes rounding    */
+                                           /* every partial sum unsafe).                                                      */
 
 int devis_msda_abi_version(void);
 const char *devis_msda_error_string(int code);
@@ -110,7 +114,7 @@ int devis_msda_forward(const void *value, const int64_t *spatial_shapes, const i
 /*
  * Backward.  Replaces ms_deform_attn_backward (vision.cpp:15).
  *   grad_output        (batch, num_query, num_heads*channels)
- *   grad_value         like value (float for DEVIS_MSDA_BF16)  -- zero-filled by this call, then accumulated
+ *   grad_value         like value (float for DEVIS_MSDA_BF16 / F16) -- zero-filled by this call, then accumulated
  *   grad_sampling_loc  like sampling_loc                        -- fully written
  *   grad_attn_weight   like attn_weight                         -- fully written
  * flags: DEVIS_MSDA_FLAG_*; the deterministic mode needs a workspace of
@@ -185,7 +189,7 @@ int devis_tmsda_backward(const void *value, const int64_t *spatial_shapes_host,
  *       out like devis_tmsda_forward's operands -- what TemporalMSDeformAttnDecoder.forward returns next to its output
  *       (:414, consumed by visualize_att_maps.py:162-165)
  *   grad_ref       optional (NULL = skip): d/d(ref), like ref; zero-filled by the call, accumulated with float atomics
- * value / output / grad_output: DEVIS_MSDA_F32 or DEVIS_MSDA_BF16; channels must be 32 and the point counts multiples of
+ * value / output / grad_output: DEVIS_MSDA_F32, DEVIS_MSDA_BF16 or DEVIS_MSDA_F16; channels must be 32 and the point counts multiples of
  * 4 (else DEVIS_MSDA_ERR_UNSUPPORTED and the caller uses devis_tmsda_forward on materialised operands).  The backward
  * writes d/d(off_*) and d/d(logit_*) directly; grad_value (float) is zero-filled by the call; flags:
  * DEVIS_MSDA_FLAG_NO_GRAD_VALUE, DEVIS_MSDA_FLAG_BF16_GRAD_VALUE, DEVIS_MSDA_FLAG_DETERMINISTIC (round 2: grad_value
