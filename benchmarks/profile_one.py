@@ -21,7 +21,7 @@ ap.add_argument("--tile", default="8x8")
 ap.add_argument("--threads", type=int, default=0)
 ap.add_argument("--qpg", type=int, default=0)
 ap.add_argument("--sigma", type=float, default=2.0)
-ap.add_argument("--bwd-mode", type=int, default=0, help="tuning key 6: 1 direct scatter, 2 windowed, 3 sorted")
+ap.add_argument("--bwd-mode", type=int, default=0, help="tuning key 6: 1 = the deterministic mode uses the direct 64-bit scatter instead of the sorted kernel")
 ap.add_argument("--margin", type=int, default=0)
 ap.add_argument("--min-level", type=int, default=0)
 a = ap.parse_args()

@@ -508,7 +508,7 @@ def test_fused_backward_without_park_against_float64_and_parked_run(knobs, name,
     nl, wt = len(c["shapes"]), c["n_frames"] - 1
     threads = c["threads"] or c["default_threads"]
     lq = sum(h * w for h, w in c["shapes"])
-    assert threads == (c["threads"] or (128 if lq >= 128 else 64))      # fused_grid's heuristic for this Lq
+    assert threads == (c["threads"] or (128 if lq >= 128 else 64))      # pick_shape's heuristic for this Lq
     assert _fused_bwd_smem(nl, wt, c["pc"], c["pt"], threads) > 48 * 1024
     assert _fused_bwd_smem(nl, wt, c["pc"], c["pt"], PARK_THREADS) <= 48 * 1024
     x, ref = _nopark_case(name, dtype_name)
