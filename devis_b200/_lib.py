@@ -41,6 +41,8 @@ SIGNATURES = {
     "devis_tmsda_fused_forward": (_i, [_vp] * 15 + [_i] * 12 + [_vp]),
     "devis_tmsda_fused_backward_workspace_bytes": (_sz, [_i] * 4 + [_u]),
     "devis_tmsda_fused_backward": (_i, [_vp] * 17 + [_i] * 12 + [_u, _vp, _sz, _vp]),
+    "devis_tmsda_fused_forward_ex": (_i, [_vp] * 16 + [_i] * 12 + [_vp]),
+    "devis_tmsda_fused_backward_ex": (_i, [_vp] * 18 + [_i] * 12 + [_u, _vp, _sz, _vp]),
     # include/devis_deform_conv.h
     "devis_dcn_im2col": (_i, [_vp] * 4 + [_i] * 15 + [_vp]),
     "devis_dcn_im2col_og": (_i, [_vp] * 4 + [_i] * 16 + [_vp]),

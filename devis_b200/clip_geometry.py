@@ -197,6 +197,10 @@ def from_reference_args(n_frames, input_spatial_shapes, input_level_start_index,
         if tlsi != tuple(j * frame_rows + st for j in range(wt) for st in lsi):
             raise RuntimeError("temporal level_start_index must be the per-frame start indices offset by one frame's rows "
                                "per temporal slot")
+    return _memoised(n_frames, shapes, lsi, table)
+
+
+def _memoised(n_frames, shapes, lsi, table):
     key = (n_frames, shapes, lsi, table)
     geom = _geom_cache.get(key)
     if geom is None:
@@ -205,3 +209,12 @@ def from_reference_args(n_frames, input_spatial_shapes, input_level_start_index,
         geom = ClipGeometry(shapes, n_frames, table, lsi)
         _geom_cache[key] = geom
     return geom
+
+
+def batch_geometry(batch, input_spatial_shapes, input_level_start_index):
+    """Geometry of MSDeformAttn's batched op for the whole-clip kernels: the batch of images is the frame axis and
+    there are no temporal slots (no frame table).  Host values read as in from_reference_args (memoised per tensor
+    object and version); the geometry is memoised by value."""
+    shapes = tuple(tuple(int(x) for x in r) for r in _host_list(input_spatial_shapes))
+    lsi = tuple(int(x) for x in _host_list(input_level_start_index))
+    return _memoised(int(batch), shapes, lsi, None)

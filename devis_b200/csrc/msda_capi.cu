@@ -138,6 +138,13 @@ void with_int(int v, F &&f)
     else with_int<Rest...>(v, f);
 }
 
+template <class F>
+void with_bool(bool v, F &&f)
+{
+    if (v) f(std::true_type{});
+    else f(std::false_type{});
+}
+
 // ROWB of the D = 32 kernels: with 8 heads the size of a value row is a compile-time immediate of the gathers, else 0
 template <Elem E, class F>
 void with_row_bytes(int M, F &&f)
@@ -720,6 +727,24 @@ int devis_tmsda_fused_forward(const void *value, const int64_t *spatial_shapes_h
                               int n_temporal_points, int t_window, int ref_dim, int temporal_ref_mode, int dtype,
                               void *stream)
 {
+    return devis_tmsda_fused_forward_ex(value, spatial_shapes_host, level_start_index_host, frame_table_host, ref,
+                                        off_curr, logit_curr, off_temporal, logit_temporal, output, loc_curr_out,
+                                        aw_curr_out, loc_temporal_out, aw_temporal_out, query_order, nullptr,
+                                        num_frames, spatial_size, num_heads, channels, num_levels, num_query,
+                                        n_curr_points, n_temporal_points, t_window, ref_dim, temporal_ref_mode, dtype,
+                                        stream);
+}
+
+int devis_tmsda_fused_forward_ex(const void *value, const int64_t *spatial_shapes_host,
+                                 const int64_t *level_start_index_host, const int32_t *frame_table_host,
+                                 const void *ref, const void *off_curr, const void *logit_curr,
+                                 const void *off_temporal, const void *logit_temporal, void *output,
+                                 void *loc_curr_out, void *aw_curr_out, void *loc_temporal_out, void *aw_temporal_out,
+                                 const int32_t *query_order, const uint8_t *padding_mask, int num_frames,
+                                 int spatial_size, int num_heads, int channels, int num_levels, int num_query,
+                                 int n_curr_points, int n_temporal_points, int t_window, int ref_dim,
+                                 int temporal_ref_mode, int dtype, void *stream)
+{
     FusedArgs a{};
     int rc = fill_fused(a, value, spatial_shapes_host, level_start_index_host, frame_table_host, ref, off_curr,
                         logit_curr, off_temporal, logit_temporal, query_order, num_frames, spatial_size, num_heads,
@@ -733,6 +758,7 @@ int devis_tmsda_fused_forward(const void *value, const int64_t *spatial_shapes_h
     a.aw_out[0] = reinterpret_cast<float *>(aw_curr_out);
     a.loc_out[1] = a.n_seg > 1 ? reinterpret_cast<float *>(loc_temporal_out) : nullptr;
     a.aw_out[1] = a.n_seg > 1 ? reinterpret_cast<float *>(aw_temporal_out) : nullptr;
+    a.mask = padding_mask;
     // dead corners skipped, virtual top-left addressing: signed 32-bit offsets, so value must stay below 2 GiB (the Python
     // side then uses the unfused op)
     if ((unsigned long long)num_frames * spatial_size * num_heads * channels * elem_size(dtype) >= (1ull << 31))
@@ -751,7 +777,9 @@ int devis_tmsda_fused_forward(const void *value, const int64_t *spatial_shapes_h
         with_elem(dtype, [&](auto e) {
             constexpr Elem E = decltype(e)::value;
             if constexpr (E != Elem::F32)
-                with_row_bytes<E>(num_heads, [&](auto rowb) { tmsda_fused_fwd8_kernel<E, rowb><<<grid, s.threads, smem, st>>>(a); });
+                with_row_bytes<E>(num_heads, [&](auto rowb) {
+                    with_bool(padding_mask != nullptr, [&](auto mk) { tmsda_fused_fwd8_kernel<E, rowb, mk><<<grid, s.threads, smem, st>>>(a); });
+                });
         });
         return check_launch(DEVIS_MSDA_KERNEL_FUSED_FWD);
     }
@@ -763,11 +791,13 @@ int devis_tmsda_fused_forward(const void *value, const int64_t *spatial_shapes_h
     with_elem(dtype, [&](auto e) {
         constexpr Elem E = decltype(e)::value;
         with_row_bytes<E>(num_heads, [&](auto rowb) {
-            if (general) {
-                tmsda_fused_fwd_kernel<E, 1, true, rowb><<<grid, s.threads, smem, st>>>(a);
-            } else if constexpr (E == Elem::F32) {
-                with_int<2, 1>(s.qpg, [&](auto q) { tmsda_fused_fwd_kernel<E, q, false, rowb><<<grid, s.threads, smem, st>>>(a); });
-            }
+            with_bool(padding_mask != nullptr, [&](auto mk) {
+                if (general) {
+                    tmsda_fused_fwd_kernel<E, 1, true, rowb, mk><<<grid, s.threads, smem, st>>>(a);
+                } else if constexpr (E == Elem::F32) {
+                    with_int<2, 1>(s.qpg, [&](auto q) { tmsda_fused_fwd_kernel<E, q, false, rowb, mk><<<grid, s.threads, smem, st>>>(a); });
+                }
+            });
         });
     });
     return check_launch(DEVIS_MSDA_KERNEL_FUSED_FWD);
@@ -790,6 +820,26 @@ int devis_tmsda_fused_backward(const void *value, const int64_t *spatial_shapes_
                                int channels, int num_levels, int num_query, int n_curr_points,
                                int n_temporal_points, int t_window, int ref_dim, int temporal_ref_mode, int dtype,
                                unsigned flags, void *workspace, size_t workspace_bytes, void *stream)
+{
+    return devis_tmsda_fused_backward_ex(value, spatial_shapes_host, level_start_index_host, frame_table_host, ref,
+                                         off_curr, logit_curr, off_temporal, logit_temporal, grad_output, grad_value,
+                                         grad_off_curr, grad_logit_curr, grad_off_temporal, grad_logit_temporal,
+                                         grad_ref, query_order, nullptr, num_frames, spatial_size, num_heads, channels,
+                                         num_levels, num_query, n_curr_points, n_temporal_points, t_window, ref_dim,
+                                         temporal_ref_mode, dtype, flags, workspace, workspace_bytes, stream);
+}
+
+int devis_tmsda_fused_backward_ex(const void *value, const int64_t *spatial_shapes_host,
+                                  const int64_t *level_start_index_host, const int32_t *frame_table_host,
+                                  const void *ref, const void *off_curr, const void *logit_curr,
+                                  const void *off_temporal, const void *logit_temporal, const void *grad_output,
+                                  void *grad_value, void *grad_off_curr, void *grad_logit_curr,
+                                  void *grad_off_temporal, void *grad_logit_temporal, void *grad_ref,
+                                  const int32_t *query_order, const uint8_t *padding_mask, int num_frames,
+                                  int spatial_size, int num_heads, int channels, int num_levels, int num_query,
+                                  int n_curr_points, int n_temporal_points, int t_window, int ref_dim,
+                                  int temporal_ref_mode, int dtype, unsigned flags, void *workspace,
+                                  size_t workspace_bytes, void *stream)
 {
     FusedArgs a{};
     int rc = fill_fused(a, value, spatial_shapes_host, level_start_index_host, frame_table_host, ref, off_curr,
@@ -824,6 +874,7 @@ int devis_tmsda_fused_backward(const void *value, const int64_t *spatial_shapes_
     a.grad_off[1] = reinterpret_cast<float *>(grad_off_temporal);
     a.grad_logit[1] = reinterpret_cast<float *>(grad_logit_temporal);
     a.grad_ref = reinterpret_cast<float *>(grad_ref);
+    a.mask = padding_mask;
     const LaunchShape s = pick_shape(num_query, kShapeBwd, 1);
     dim3 grid;
     if ((rc = lane_group_grid(a.d, s.threads / 8, s.qpg, grid))) return rc;
@@ -840,17 +891,16 @@ int devis_tmsda_fused_backward(const void *value, const int64_t *spatial_shapes_
     const bool general = ref_dim == 4 || (a.n_seg > 1 && temporal_ref_mode != 0) || grad_ref;
     with_elem(dtype, [&](auto e) {
         constexpr Elem E = decltype(e)::value;
-        auto launch = [&](auto gen) {
+        auto launch = [&](auto gen, auto mk) {
             if (det) {
-                tmsda_fused_bwd_kernel<E, false, gen, true><<<grid, s.threads, smem, st>>>(a);
+                tmsda_fused_bwd_kernel<E, false, gen, true, mk><<<grid, s.threads, smem, st>>>(a);
             } else if (half_acc) {
-                if constexpr (E == Elem::BF16) tmsda_fused_bwd_kernel<E, true, gen><<<grid, s.threads, smem, st>>>(a);
+                if constexpr (E == Elem::BF16) tmsda_fused_bwd_kernel<E, true, gen, false, mk><<<grid, s.threads, smem, st>>>(a);
             } else {
-                tmsda_fused_bwd_kernel<E, false, gen><<<grid, s.threads, smem, st>>>(a);
+                tmsda_fused_bwd_kernel<E, false, gen, false, mk><<<grid, s.threads, smem, st>>>(a);
             }
         };
-        if (general) launch(std::true_type{});
-        else launch(std::false_type{});
+        with_bool(general, [&](auto gen) { with_bool(padding_mask != nullptr, [&](auto mk) { launch(gen, mk); }); });
     });
     rc = check_launch(DEVIS_MSDA_KERNEL_FUSED_BWD);
     if (rc || !det) return rc;

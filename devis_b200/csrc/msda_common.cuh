@@ -181,6 +181,35 @@ __device__ __forceinline__ TapGeomV tap_geometry_v(float x, float y, const int4 
 }
 
 // ---------------------------------------------------------------------------------------------
+// Padding mask (MSDeformAttn's input_padding_mask): one byte per value row, nonzero = the row reads as zero, exactly as
+// value.masked_fill(mask[..., None], 0) before the op.  A masked corner is DROPPED, never multiplied by zero -- a masked
+// row may hold NaN or Inf, and 0 x NaN is NaN: it is not gathered, not scattered to, and its value counts as 0 in the
+// location and weight gradients.  Only the bytes of corners inside the map are read (rows frame*S + pixel, L1-resident).
+// ---------------------------------------------------------------------------------------------
+// tap_geometry_v's live bits without the masked corners
+__device__ __forceinline__ unsigned unmasked_live(const uint8_t *mask, int rowv, int W, unsigned live)
+{
+    const uint8_t *p = mask + (ptrdiff_t)rowv;
+    if ((live & 1u) && __ldg(p)) live &= ~1u;
+    if ((live & 2u) && __ldg(p + 1)) live &= ~2u;
+    if ((live & 4u) && __ldg(p + W)) live &= ~4u;
+    if ((live & 8u) && __ldg(p + W + 1)) live &= ~8u;
+    return live;
+}
+
+// per-corner bits of a TapGeom (bit0 TL, bit1 TR, bit2 BL, bit3 BR): the corner is inside the map and not masked
+__device__ __forceinline__ unsigned unmasked_corners(const uint8_t *mask, const TapGeom &t)
+{
+    const unsigned top = t.ok & 1u, bot = (t.ok >> 1) & 1u, left = (t.ok >> 2) & 1u, right = (t.ok >> 3) & 1u;
+    unsigned c = (top & left) | ((top & right) << 1) | ((bot & left) << 2) | ((bot & right) << 3);
+    if ((c & 1u) && __ldg(mask + t.rTL)) c &= ~1u;
+    if ((c & 2u) && __ldg(mask + t.rTR)) c &= ~2u;
+    if ((c & 4u) && __ldg(mask + t.rBL)) c &= ~4u;
+    if ((c & 8u) && __ldg(mask + t.rBR)) c &= ~8u;
+    return c;
+}
+
+// ---------------------------------------------------------------------------------------------
 // Tap exchange through shared memory.  A group of LPG lanes owns one (query, head); lane j prepares
 // tap k0+j and publishes a 32-byte record; then all lanes of the group walk the LPG records.
 // (Round-1 profile: doing this with __shfl_sync cost 6 L1-data-pipe wavefronts per tap -- shuffles

@@ -55,6 +55,7 @@ struct FusedArgs {
     float *grad_off[2];
     float *grad_logit[2];
     int park_iters;            // > 0: shared memory holds (weight, d/d weight) of that many exchanges per thread
+    const uint8_t *mask;       // padding mask (T, S), nonzero = the value row reads as zero (unmasked_live) [MASK]
 };
 
 // softmax statistics of one (query, head) row over both segments, computed by the LPG lanes of its group
@@ -193,7 +194,8 @@ __device__ __forceinline__ void raw_to_operands(const FusedArgs &a, int sg, cons
 #ifndef DEVIS_FUSED_FWD_TB
 #define DEVIS_FUSED_FWD_TB 2
 #endif
-template <Elem E, int QPG, bool GEN = false, int ROWB = 0>
+// MASK: a.mask is given; a masked corner's live bit is cleared, so its gather is never issued
+template <Elem E, int QPG, bool GEN = false, int ROWB = 0, bool MASK = false>
 __global__ void __launch_bounds__(256, DEVIS_FUSED_FWD_MIN_BLOCKS) tmsda_fused_fwd_kernel(const FusedArgs a)
 {
     constexpr int LPG = 8;
@@ -271,7 +273,8 @@ __global__ void __launch_bounds__(256, DEVIS_FUSED_FWD_MIN_BLOCKS) tmsda_fused_f
                 }
                 float *buf = xbuf + parity * Tap16x8::kWordsPerWarpBuf;
                 parity ^= 1;
-                const TapGeomV t = tap_geometry_v(x, y, sl, live);
+                TapGeomV t = tap_geometry_v(x, y, sl, live);
+                if (MASK) t.live = unmasked_live(a.mask, t.rowv, sl.y, t.live);
                 *reinterpret_cast<uint4 *>(buf + Tap16x8::word(j, g)) = make_tap16v(t, w, rowbytes);
                 __syncwarp();
                 consume_tap16v<E, ROWB, DEVIS_FUSED_FWD_TB>(buf, g, rowbytes, pitch_lo, pitch_hi, vbase, acc[i], v);
@@ -292,7 +295,7 @@ __global__ void __launch_bounds__(256, DEVIS_FUSED_FWD_MIN_BLOCKS) tmsda_fused_f
 // Four lanes per (query, head), 8 channels per lane (msda_fwd8v_kernel's shape): the forward of choice for 16-bit value
 // (bf16 or fp16), whose 64-byte rows cost 0.75 instead of 1.0 data-pipe cycles when 4 lanes fetch 16 bytes each.
 // 16-bit value only (the fp32 form of this shape loses to the eight-lane kernel); dead corners skipped, consume_tap16x4v
-template <Elem E, int ROWB>
+template <Elem E, int ROWB, bool MASK = false>
 __global__ void __launch_bounds__(256) tmsda_fused_fwd8_kernel(const FusedArgs a)
 {
     static_assert(E != Elem::F32, "16-bit value only");
@@ -339,7 +342,8 @@ __global__ void __launch_bounds__(256) tmsda_fused_fwd8_kernel(const FusedArgs a
             if (qlive) raw_to_operands<false>(a, sg, cur, sl, rmax, rinv, x, y, w);
             float *buf = xbuf + parity * Tap16::kWordsPerWarpBuf;
             parity ^= 1;
-            const TapGeomV t = tap_geometry_v(x, y, sl, qlive);
+            TapGeomV t = tap_geometry_v(x, y, sl, qlive);
+            if (MASK) t.live = unmasked_live(a.mask, t.rowv, sl.y, t.live);
             *reinterpret_cast<uint4 *>(buf + Tap16::word(j, g)) = make_tap16v(t, w, rowbytes);
             __syncwarp();
             consume_tap16x4v<E, ROWB>(buf, g, rowbytes, pitch, vbase, acc, v);
@@ -358,7 +362,10 @@ __global__ void __launch_bounds__(256) tmsda_fused_fwd8_kernel(const FusedArgs a
 // fixed-point accumulators with integer reductions (det_add4, msda_common.cuh) exactly as in msda_bwd_kernel, with the
 // bound max|attn| = 1 (the weights are softmax outputs here); every other gradient of this kernel is written once, in a
 // fixed order, so the whole backward is bit-identical run to run.
-template <Elem E, bool HALF_ACC = false, bool GEN = false, bool DET = false>
+// MASK: a.mask is given.  TapGeom's row / column bits cannot describe one masked corner, so the record carries four
+// per-corner bits (unmasked_corners) in bits 1-4 of the TL byte offset (value rows are >= 64 B; bit 0 is the sort tag of
+// msda_bwd_sort.cuh, unused here); a dropped corner reads as zero and scatters nothing -- by selection, not by a product.
+template <Elem E, bool HALF_ACC = false, bool GEN = false, bool DET = false, bool MASK = false>
 __global__ void __launch_bounds__(256, DEVIS_BWD_MIN_BLOCKS) tmsda_fused_bwd_kernel(const FusedArgs a)
 {
     static_assert(!(DET && HALF_ACC), "deterministic mode accumulates in fixed point");
@@ -424,7 +431,7 @@ __global__ void __launch_bounds__(256, DEVIS_BWD_MIN_BLOCKS) tmsda_fused_bwd_ker
             const TapGeom t = tap_geometry(x, y, sl, live);
             float *buf = xbuf + parity * X::kWordsPerWarpBuf;
             parity ^= 1;
-            X::publish(buf, j, g, t, w, rowbytes);
+            X::publish(buf, j, g, t, w, rowbytes, MASK ? unmasked_corners(a.mask, t) << 1 : 0u);
             __syncwarp();
 
             float dsum[LPG][4];
@@ -433,6 +440,11 @@ __global__ void __launch_bounds__(256, DEVIS_BWD_MIN_BLOCKS) tmsda_fused_bwd_ker
                 uint4 off;
                 float4 c;
                 X::fetch(buf, jj, g, off, c);
+                unsigned corners = 15u;
+                if (MASK) {
+                    corners = (off.x >> 1) & 15u;
+                    off.x &= ~30u;
+                }
                 float4 v00, v01, v10, v11;
                 if constexpr (E != Elem::F32) {
                     v00 = ldg_16x4<E>(reinterpret_cast<const uint2 *>(vbase + off.x));
@@ -444,6 +456,13 @@ __global__ void __launch_bounds__(256, DEVIS_BWD_MIN_BLOCKS) tmsda_fused_bwd_ker
                     v01 = ldg_f4(reinterpret_cast<const float4 *>(vbase + off.y));
                     v10 = ldg_f4(reinterpret_cast<const float4 *>(vbase + off.z));
                     v11 = ldg_f4(reinterpret_cast<const float4 *>(vbase + off.w));
+                }
+                if (MASK) {
+                    const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+                    if (!(corners & 1u)) v00 = z, c.x = 0.f;
+                    if (!(corners & 2u)) v01 = z, c.y = 0.f;
+                    if (!(corners & 4u)) v10 = z, c.z = 0.f;
+                    if (!(corners & 8u)) v11 = z, c.w = 0.f;
                 }
                 dsum[jj][0] = fmaf(v00.w, gg.w, fmaf(v00.z, gg.z, fmaf(v00.y, gg.y, v00.x * gg.x)));
                 dsum[jj][1] = fmaf(v01.w, gg.w, fmaf(v01.z, gg.z, fmaf(v01.y, gg.y, v01.x * gg.x)));

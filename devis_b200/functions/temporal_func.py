@@ -124,7 +124,7 @@ class TemporalMSDeformAttnFunction(Function):
 
 class TemporalMSDeformAttnFusedFunction(Function):
     """apply(value, ref, off_curr, logit_curr, off_temporal, logit_temporal, geometry, query_order=None,
-             temporal_ref_mode=TREF_LEVEL0, want_sampling=False) -> out (T, Lq, M*D)
+             temporal_ref_mode=TREF_LEVEL0, want_sampling=False, padding_mask=None) -> out (T, Lq, M*D)
                                                            | (out, loc_curr, aw_curr, loc_temporal, aw_temporal)
 
     Whole-clip temporal attention straight from the Linear outputs: the joint softmax over all taps and the sampling
@@ -134,7 +134,10 @@ class TemporalMSDeformAttnFusedFunction(Function):
     (T,Lq,M,L,Pc,2); logit_curr (T,Lq,M,L*Pc); off_temporal (T,Lq,M,Wt*L,Pt,2); logit_temporal (T,Lq,M,Wt*L*Pt).
     temporal_ref_mode: _lib.TREF_LEVEL0 (encoder) | TREF_OWN | TREF_SAMPLED (decoder, instance aware).
     want_sampling: also return the sampling locations and softmax weights the kernel computed (non-differentiable
-    by-products: what TemporalMSDeformAttnDecoder.forward hands to visualize_att_maps.py)."""
+    by-products: what TemporalMSDeformAttnDecoder.forward hands to visualize_att_maps.py).
+    padding_mask: optional CUDA bool (or uint8) tensor (T, S), True = padding.  Equivalent to
+    value.masked_fill(padding_mask[..., None], 0) before the op, NaN / Inf in masked rows included; no gradient.
+    MSDeformAttn passes its input_padding_mask here (its batch is the frame axis)."""
 
     @staticmethod
     def supported(value, reference_points, n_curr_points=4, n_temporal_points=4):
@@ -148,7 +151,7 @@ class TemporalMSDeformAttnFusedFunction(Function):
 
     @staticmethod
     def forward(ctx, value, ref, off_curr, logit_curr, off_temporal, logit_temporal, geometry, query_order=None,
-                temporal_ref_mode=_lib.TREF_LEVEL0, want_sampling=False):
+                temporal_ref_mode=_lib.TREF_LEVEL0, want_sampling=False, padding_mask=None):
         if not value.is_cuda:
             raise RuntimeError("Not implemented on the CPU")
         if value.dtype not in (torch.float32,) + _16BIT:
@@ -168,6 +171,12 @@ class TemporalMSDeformAttnFusedFunction(Function):
             raise RuntimeError("operands do not match the clip geometry")
         if tuple(ref.shape) != (t, lq, geometry.n_levels, ref_dim) or ref_dim not in (2, 4):
             raise RuntimeError(f"reference points {tuple(ref.shape)} must be (T, Lq, L, 2|4)")
+        if padding_mask is not None:
+            if tuple(padding_mask.shape) != (t, s) or padding_mask.dtype not in (torch.bool, torch.uint8) \
+                    or padding_mask.device != value.device:
+                raise RuntimeError(f"padding mask {tuple(padding_mask.shape)} {padding_mask.dtype} must be a bool tensor "
+                                   f"(T, S) = {(t, s)} on the device of value")
+            padding_mask = padding_mask.detach().contiguous()
         out = torch.empty((t, lq, m * d), dtype=value.dtype, device=value.device)
         samp = [None] * 4
         if want_sampling:
@@ -178,17 +187,17 @@ class TemporalMSDeformAttnFusedFunction(Function):
                 samp[3] = torch.empty((t, lq, m, geometry.t_window * geometry.n_levels, pt), dtype=torch.float32,
                                       device=value.device)
         with torch.cuda.device(value.device):
-            _lib.check(_lib.load().devis_tmsda_fused_forward(
+            _lib.check(_lib.load().devis_tmsda_fused_forward_ex(
                 _ptr(value), geometry.shapes_ptr, geometry.lsi_ptr, geometry.frames_ptr, _ptr(ref), _ptr(oc), _ptr(lc),
                 _ptr(ot), _ptr(lt), _ptr(out), _ptr(samp[0]), _ptr(samp[1]), _ptr(samp[2]), _ptr(samp[3]),
-                _ptr(query_order), t, s, m, d, geometry.n_levels, lq, pc, pt,
+                _ptr(query_order), _ptr(padding_mask), t, s, m, d, geometry.n_levels, lq, pc, pt,
                 geometry.t_window if has_t else 0, ref_dim, int(temporal_ref_mode), _DTYPES[value.dtype],
                 torch.cuda.current_stream().cuda_stream))
         ctx.geometry, ctx.has_t, ctx.tref = geometry, has_t, int(temporal_ref_mode)
         ctx.dims = (t, s, m, d, lq, pc, pt, ref_dim)
         ctx.in_dtypes = (off_curr.dtype, logit_curr.dtype, off_temporal.dtype if has_t else None,
                          logit_temporal.dtype if has_t else None, ref_in_dtype)
-        ctx.save_for_backward(value, ref, oc, lc, ot, lt, query_order)
+        ctx.save_for_backward(value, ref, oc, lc, ot, lt, query_order, padding_mask)
         if not want_sampling:
             return out
         extras = tuple(x for x in samp if x is not None)
@@ -199,7 +208,7 @@ class TemporalMSDeformAttnFusedFunction(Function):
     @staticmethod
     @once_differentiable
     def backward(ctx, grad_output, *_unused):
-        value, ref, oc, lc, ot, lt, query_order = ctx.saved_tensors
+        value, ref, oc, lc, ot, lt, query_order, padding_mask = ctx.saved_tensors
         geometry, has_t = ctx.geometry, ctx.has_t
         t, s, m, d, lq, pc, pt, ref_dim = ctx.dims
         gout = grad_output if grad_output.dtype == value.dtype else grad_output.to(value.dtype)
@@ -222,17 +231,18 @@ class TemporalMSDeformAttnFusedFunction(Function):
         with torch.cuda.device(value.device):
             ws_bytes = _lib.load().devis_tmsda_fused_backward_workspace_bytes(t, s, m, d, flags)
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=value.device) if ws_bytes else None
-            _lib.check(_lib.load().devis_tmsda_fused_backward(
+            _lib.check(_lib.load().devis_tmsda_fused_backward_ex(
                 _ptr(value), geometry.shapes_ptr, geometry.lsi_ptr, geometry.frames_ptr, _ptr(ref), _ptr(oc), _ptr(lc),
                 _ptr(ot), _ptr(lt), _ptr(gout), _ptr(gv), _ptr(goc), _ptr(glc), _ptr(got), _ptr(glt), _ptr(gref),
-                _ptr(query_order), t, s, m, d, geometry.n_levels, lq, pc, pt, geometry.t_window if has_t else 0,
+                _ptr(query_order), _ptr(padding_mask), t, s, m, d, geometry.n_levels, lq, pc, pt, geometry.t_window if has_t else 0,
                 ref_dim, ctx.tref, _DTYPES[value.dtype], flags, _ptr(ws), ws_bytes,
                 torch.cuda.current_stream().cuda_stream))
         doc, dlc, dot, dlt, dref = ctx.in_dtypes
         if gv is not None and gv.dtype != value.dtype:
             gv = gv.to(value.dtype)
         cast = lambda g, dt: g if (g is None or g.dtype == dt) else g.to(dt)
-        return gv, cast(gref, dref), cast(goc, doc), cast(glc, dlc), cast(got, dot), cast(glt, dlt), None, None, None, None
+        return (gv, cast(gref, dref), cast(goc, doc), cast(glc, dlc), cast(got, dot), cast(glt, dlt), None, None, None,
+                None, None)
 
 
 def temporal_ms_deform_attn(value, loc_curr, aw_curr, loc_temporal, aw_temporal, geometry, query_order=None):

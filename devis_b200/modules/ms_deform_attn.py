@@ -2,7 +2,8 @@
 (checkpoints load unchanged), call signatures and return values
 (/root/reference/src/models/ops/modules/ms_deform_attn.py), running on the sm_100a kernels.
 
-  MSDeformAttn                  ms_deform_attn.py:30-132   one op call, unchanged structure
+  MSDeformAttn                  ms_deform_attn.py:30-132   one op call; with fuse_prologue the softmax, the location
+                                                           arithmetic and the padding mask run inside the kernels
   TemporalMSDeformAttnBase      ms_deform_attn.py:137-285  projections + joint softmax
   TemporalMSDeformAttnEncoder   ms_deform_attn.py:417-464
   TemporalMSDeformAttnDecoder   ms_deform_attn.py:288-414
@@ -68,6 +69,11 @@ class MSDeformAttn(nn.Module):
         self.attention_weights = nn.Linear(d_model, n_heads * n_levels * n_points)
         self.value_proj = nn.Linear(d_model, d_model)
         self.output_proj = nn.Linear(d_model, d_model)
+        # encoder self-attention (Lq == S): walk the pixel-grid queries in 2-D tiles (cache locality only)
+        self.query_tile = (8, 8)
+        # let the kernels read the raw Linear outputs and the padding mask (TemporalMSDeformAttnFusedFunction with the
+        # batch as the frame axis): no softmax, location or masked_fill kernels and no copy of value, either way
+        self.fuse_prologue = True
         self._reset_parameters()
 
     def _reset_parameters(self):
@@ -82,15 +88,27 @@ class MSDeformAttn(nn.Module):
         xavier_uniform_(self.output_proj.weight.data)
         constant_(self.output_proj.bias.data, 0.)
 
+    def _fused_path(self, value, reference_points):
+        """whether forward() takes the fused-prologue kernels for this projected value (N,S,M,D).  float32 and bfloat16
+        only: float16 keeps the reference's dispatch (it raises), float64 and the shapes the fused kernels do not serve
+        (D != 32, P % 4 != 0, value >= 2 GiB, deterministic mode with learnable reference points) keep the unfused op."""
+        return (self.fuse_prologue and value.dtype in (torch.float32, torch.bfloat16) and value.shape[0] > 0
+                and TemporalMSDeformAttnFusedFunction.supported(value, reference_points, self.n_points, self.n_points))
+
     def forward(self, query, reference_points, input_flatten, input_spatial_shapes, input_level_start_index,
                 input_padding_mask=None):
         """query (N,Lq,C); reference_points (N,Lq,L,2|4); input_flatten (N,S,C); returns (out, None)."""
         n, lq, _ = query.shape
         s = input_flatten.shape[1]
         m, nl, p = self.n_heads, self.n_levels, self.n_points
+        value = self.value_proj(input_flatten)
+        # decided on the PROJECTED value (under autocast it is half precision while input_flatten is not)
+        heads = value.view(n, s, m, self.d_model // m)
+        if self._fused_path(heads, reference_points):
+            return self._forward_fused(query, reference_points, heads, input_spatial_shapes, input_level_start_index,
+                                       input_padding_mask)
         assert (input_spatial_shapes[:, 0] * input_spatial_shapes[:, 1]).sum() == s
 
-        value = self.value_proj(input_flatten)
         if input_padding_mask is not None:
             value = value.masked_fill(input_padding_mask[..., None], float(0))
         value = value.view(n, s, m, self.d_model // m)
@@ -107,6 +125,29 @@ class MSDeformAttn(nn.Module):
                 reference_points.shape[-1]))
         out = MSDeformAttnFunction.apply(value, input_spatial_shapes, input_level_start_index, loc, weights,
                                          self.im2col_step)
+        return self.output_proj(out), None
+
+    def _forward_fused(self, query, reference_points, value, input_spatial_shapes, input_level_start_index,
+                       input_padding_mask):
+        """One launch each way for the attention: the N images are the frames of a clip without temporal slots, the
+        softmax, `ref + off / (W, H)` (points, encoder form) or the box form (GEN) and the padding mask are evaluated in
+        the kernels.  Host values of the pyramid come from memoised reads: no device read-back the unfused path does
+        not make."""
+        n, lq, _ = query.shape
+        s = value.shape[1]
+        m, nl, p = self.n_heads, self.n_levels, self.n_points
+        geom = clip_geometry.batch_geometry(n, input_spatial_shapes, input_level_start_index)
+        assert sum(h * w for h, w in geom.shapes) == s
+        step = min(n, self.im2col_step)
+        if n % step != 0:
+            raise RuntimeError(f"batch({n}) must divide im2col_step({step})")
+        order = None
+        if self.query_tile and lq == s:
+            order = geom.tile_order(query.device, *self.query_tile)
+        out = TemporalMSDeformAttnFusedFunction.apply(
+            value, reference_points, self.sampling_offsets(query).view(n, lq, m, nl, p, 2),
+            self.attention_weights(query).view(n, lq, m, nl * p), None, None, geom, order, _lib.TREF_LEVEL0, False,
+            input_padding_mask)
         return self.output_proj(out), None
 
 

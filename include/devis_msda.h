@@ -221,6 +221,38 @@ int devis_tmsda_fused_backward(const void *value, const int64_t *spatial_shapes_
                                int n_temporal_points, int t_window, int ref_dim, int temporal_ref_mode, int dtype,
                                unsigned flags, void *workspace, size_t workspace_bytes, void *stream);
 
+/*
+ * The two calls above with an input padding mask.  devis_tmsda_fused_forward / _backward are these with
+ * padding_mask = NULL.
+ *   padding_mask   optional DEVICE uint8 (num_frames, spatial_size), one byte per value row; nonzero = the row is
+ *                  padding.  Exactly equivalent to value.masked_fill(padding_mask[..., None], 0) before the op -- even
+ *                  when a masked row holds NaN or Inf: a masked corner contributes nothing to the output, receives no
+ *                  grad_value and counts as a zero value in d/d(off_*), d/d(logit_*) and d/d(ref).  The mask is indexed
+ *                  by the frame a tap samples, so it also applies to the temporal slots.  NULL = no mask.
+ * This is what MSDeformAttn's input_padding_mask needs: its batch of N images is the frame axis (t_window = 0, no frame
+ * table), the encoder with points (ref_dim 2), the decoder with points or boxes.
+ */
+int devis_tmsda_fused_forward_ex(const void *value, const int64_t *spatial_shapes_host,
+                                 const int64_t *level_start_index_host, const int32_t *frame_table_host,
+                                 const void *ref, const void *off_curr, const void *logit_curr,
+                                 const void *off_temporal, const void *logit_temporal, void *output,
+                                 void *loc_curr_out, void *aw_curr_out, void *loc_temporal_out, void *aw_temporal_out,
+                                 const int32_t *query_order, const uint8_t *padding_mask, int num_frames,
+                                 int spatial_size, int num_heads, int channels, int num_levels, int num_query,
+                                 int n_curr_points, int n_temporal_points, int t_window, int ref_dim,
+                                 int temporal_ref_mode, int dtype, void *stream);
+int devis_tmsda_fused_backward_ex(const void *value, const int64_t *spatial_shapes_host,
+                                  const int64_t *level_start_index_host, const int32_t *frame_table_host,
+                                  const void *ref, const void *off_curr, const void *logit_curr,
+                                  const void *off_temporal, const void *logit_temporal, const void *grad_output,
+                                  void *grad_value, void *grad_off_curr, void *grad_logit_curr,
+                                  void *grad_off_temporal, void *grad_logit_temporal, void *grad_ref,
+                                  const int32_t *query_order, const uint8_t *padding_mask, int num_frames,
+                                  int spatial_size, int num_heads, int channels, int num_levels, int num_query,
+                                  int n_curr_points, int n_temporal_points, int t_window, int ref_dim,
+                                  int temporal_ref_mode, int dtype, unsigned flags, void *workspace,
+                                  size_t workspace_bytes, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
