@@ -28,6 +28,7 @@ import math
 import os
 import statistics
 import sys
+import time
 
 import torch
 import torch.nn.functional as F
@@ -354,6 +355,99 @@ def run(attn="both", iters=20, num_out=20, breakdown=True, height=360, width=640
     return out
 
 
+def _card():
+    """name and power limit of the device the numbers were taken on (part of every absolute number)"""
+    import subprocess
+    info = {"device": torch.cuda.get_device_name()}
+    try:
+        q = subprocess.run(["nvidia-smi", "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader",
+                            "-i", str(torch.cuda.current_device())], capture_output=True, text=True, timeout=60)
+        info["power_limit_and_max_sm_clock"] = q.stdout.strip()
+    except (OSError, subprocess.SubprocessError) as exc:
+        info["power_limit_and_max_sm_clock"] = "not read: %s" % exc
+    return info
+
+
+def run_compile(train=False, iters=10, rounds=3, height=360, width=640, tf32=False, n_matched=5):
+    """The model eager and with torch.compile (inductor, default mode) in one process, timed in alternating rounds of
+    `iters` calls each (CUDA events, median per round).  Compiled: the trunk (backbone, input projections, the whole
+    DeVIS transformer with our attention ops) and the mask head (our deformable convolutions); the box attention maps
+    (MultiScaleMHAttentionMap) and the post-processing stay eager -- inductor in torch 2.11 fails on the in-place
+    masked_fill_ of the attention-map einsum.  Inference: DeVISR50.forward; train: the training step of run_train
+    (forward + backward; clip_grad_norm and AdamW stay eager)."""
+    torch.manual_seed(0)
+    dev = torch.device("cuda")
+    torch.backends.cuda.matmul.allow_tf32 = bool(tf32)
+    torch.backends.cudnn.allow_tf32 = bool(tf32)
+    frames = torch.randn(6, 3, height, width, device=dev)
+    pad = torch.zeros(6, height, width, dtype=torch.bool, device=dev)
+    model = DeVISR50().to(dev)
+    head, trunk = model.mask_head, torch.compile(model.trunk)
+    compiled_head = torch.compile(head)
+
+    def use(compiled):
+        if compiled:
+            model.trunk, model.mask_head = trunk, compiled_head
+        else:
+            model.__dict__.pop("trunk", None)
+            model.mask_head = head
+    if train:
+        model.train()
+        for p in model.body.parameters():
+            p.requires_grad_(True)
+        params = [p for p in model.parameters() if p.requires_grad]
+        opt = torch.optim.AdamW(params, lr=1e-5, weight_decay=1e-4)
+
+        def make(flag):
+            def step():
+                use(flag)
+                opt.zero_grad(set_to_none=True)
+                model.training_loss(frames, pad, n_matched).backward()
+                torch.nn.utils.clip_grad_norm_(params, 0.1)
+                opt.step()
+            return step
+    else:
+        model.eval()
+
+        def make(flag):
+            def fwd():
+                use(flag)
+                model(frames, pad)
+            return fwd
+    eager, compiled = make(False), make(True)
+    t0 = time.perf_counter()
+    for _ in range(3):
+        compiled()                         # compilation + warm-up
+    torch.cuda.synchronize()
+    compile_s = time.perf_counter() - t0
+    for _ in range(3):
+        eager()
+    before = _lib.launch_count()
+    compiled()
+    torch.cuda.synchronize()
+    assert _lib.launch_count() > before, "the library's kernels did not run in the compiled model"
+
+    def timed(fn):
+        evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(iters)]
+        for a, b in evs:
+            a.record()
+            fn()
+            b.record()
+        torch.cuda.synchronize()
+        return statistics.median(a.elapsed_time(b) for a, b in evs)
+    per_round = {"eager": [], "compiled": []}
+    for _ in range(rounds):
+        per_round["eager"].append(round(timed(eager), 3))
+        per_round["compiled"].append(round(timed(compiled), 3))
+    med = {k: statistics.median(v) for k, v in per_round.items()}
+    return {"config": "DeVIS R50 %s, T=6, %dx%d, 60 queries, fp32 (TF32 %s), torch.compile(inductor) vs eager, %d "
+                      "alternating rounds x %d calls" % ("training step" if train else "inference", height, width,
+                                                         "on" if tf32 else "off", rounds, iters),
+            "ms_eager_median": round(med["eager"], 3), "ms_compiled_median": round(med["compiled"], 3),
+            "speedup": round(med["eager"] / med["compiled"], 3), "ms_per_round": per_round,
+            "compile_and_warmup_s": round(compile_s, 1), **_card()}
+
+
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
     ap.add_argument("--attn", default="both", choices=["ours", "reference", "both"])
@@ -364,6 +458,9 @@ if __name__ == "__main__":
     ap.add_argument("--train", action="store_true", help="time the training step (config 5) instead of inference (config 3)")
     ap.add_argument("--deterministic", action="store_true",
                     help="with --train --attn ours: check that two seeded training runs end bit-identical instead of timing")
+    ap.add_argument("--compile", action="store_true",
+                    help="time the whole model (inference, or with --train the training step) eager and under "
+                         "torch.compile in alternating rounds")
     a = ap.parse_args()
     if a.deterministic and not (a.train and a.attn == "ours"):
         ap.error("--deterministic needs --train --attn ours")
@@ -371,7 +468,9 @@ if __name__ == "__main__":
         os.environ.setdefault("CUBLAS_WORKSPACE_CONFIG", ":4096:8")    # before the first cuBLAS call
     res = {}
     for mode in (["off", "on"] if a.tf32 == "both" else [a.tf32]):
-        if a.deterministic:
+        if a.compile:
+            res["tf32_" + mode] = run_compile(a.train, max(4, a.iters // 2), tf32=mode == "on")
+        elif a.deterministic:
             res["tf32_" + mode] = run_train_determinism(tf32=mode == "on")
         elif a.train:
             res["tf32_" + mode] = run_train(a.attn, max(4, a.iters // 3), tf32=mode == "on")

@@ -6,6 +6,11 @@ current CUDA stream to the C-ABI library.
 
 ``import devis_b200.MultiScaleDeformableAttention as MSDA`` can replace
 ``import MultiScaleDeformableAttention as MSDA`` in functions/ms_deform_attn_func.py:18.
+
+The two functions are the torch.library custom ops ``devis::ms_deform_attn`` / ``devis::ms_deform_attn_backward``
+(the forward op carries the autograd formula of MSDeformAttnFunction), so torch.compile and torch.export trace the op
+as one node.  Every op of this package is tagged ``needs_exact_strides``: a compiled graph hands it its operands in the
+layout eager code would, which is what the contiguity checks below expect.
 """
 import torch
 
@@ -78,14 +83,26 @@ def _aux(t, value):
     return t if t.dtype == want else t.to(want)
 
 
-def ms_deform_attn_forward(value, spatial_shapes, level_start_index, sampling_loc, attn_weight, im2col_step):
-    """vision.cpp:14 / ms_deform_attn.h:20-39.  Returns (N, Lq, M*D) in value's dtype."""
+def _level_area(spatial_shapes):
+    """sum of H*W over the levels, from the memoised host copy (one synchronising read per tensor object)"""
+    from .clip_geometry import host_list
+    return sum(int(h) * int(w) for h, w in host_list(spatial_shapes))
+
+
+@torch.library.custom_op("devis::ms_deform_attn", mutates_args=(), tags=(torch.Tag.needs_exact_strides,))
+def _forward_op(value: torch.Tensor, spatial_shapes: torch.Tensor, level_start_index: torch.Tensor,
+                sampling_loc: torch.Tensor, attn_weight: torch.Tensor, im2col_step: int,
+                check_levels: bool) -> torch.Tensor:
+    """vision.cpp:14 / ms_deform_attn.h:20-39.  Returns (N, Lq, M*D) in value's dtype.  ``check_levels``: MSDeformAttn's
+    ``sum(H*W) == S`` assertion (ms_deform_attn.py:95), made here where the pyramid's host copy is read."""
     if not value.is_cuda:
         raise RuntimeError("Not implemented on the CPU")
     _check([("value", value), ("spatial_shapes", spatial_shapes), ("level_start_index", level_start_index),
             ("sampling_loc", sampling_loc), ("attn_weight", attn_weight)])
     code = _dtype_code(value)
     n, s, m, d = value.shape
+    if check_levels:
+        assert _level_area(spatial_shapes) == s
     nl = spatial_shapes.shape[0]
     lq, p = sampling_loc.shape[1], sampling_loc.shape[4]
     step = min(n, int(im2col_step)) if n > 0 else 1
@@ -103,11 +120,18 @@ def ms_deform_attn_forward(value, spatial_shapes, level_start_index, sampling_lo
     return out
 
 
-def ms_deform_attn_backward(value, spatial_shapes, level_start_index, sampling_loc, attn_weight, grad_output,
-                            im2col_step, need_grad_value=True):
-    """vision.cpp:15 / ms_deform_attn.h:41-61.  Returns [grad_value, grad_sampling_loc, grad_attn_weight].
-    ``need_grad_value=False`` (extension, used by the autograd Function when value is frozen) skips the scatter and
-    returns None in its place."""
+@_forward_op.register_fake
+def _(value, spatial_shapes, level_start_index, sampling_loc, attn_weight, im2col_step, check_levels):
+    n, _, m, d = value.shape
+    return value.new_empty((n, sampling_loc.shape[1], m * d))
+
+
+@torch.library.custom_op("devis::ms_deform_attn_backward", mutates_args=(), tags=(torch.Tag.needs_exact_strides,))
+def _backward_op(grad_output: torch.Tensor, value: torch.Tensor, spatial_shapes: torch.Tensor,
+                 level_start_index: torch.Tensor, sampling_loc: torch.Tensor, attn_weight: torch.Tensor,
+                 im2col_step: int, need_grad_value: bool) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """vision.cpp:15 / ms_deform_attn.h:41-61.  Returns (grad_value, grad_sampling_loc, grad_attn_weight);
+    grad_value is an empty tensor when ``need_grad_value`` is False (the scatter is skipped)."""
     if not value.is_cuda:
         raise RuntimeError("Not implemented on the CPU")
     _check([("value", value), ("spatial_shapes", spatial_shapes), ("level_start_index", level_start_index),
@@ -139,10 +163,53 @@ def ms_deform_attn_backward(value, spatial_shapes, level_start_index, sampling_l
             _ptr(value), _ptr(shapes), _ptr(lsi), _ptr(loc), _ptr(aw), _ptr(gout),
             _ptr(grad_value), _ptr(grad_loc), _ptr(grad_aw),
             n, s, m, d, nl, lq, p, max(int(im2col_step), 1), code, flags, _ptr(ws), ws_bytes, stream))
-    if grad_value is not None and grad_value.dtype != value.dtype:
+    if grad_value is None:
+        grad_value = value.new_empty(0)
+    elif grad_value.dtype != value.dtype:
         grad_value = grad_value.to(value.dtype)
     if grad_loc.dtype != sampling_loc.dtype:
         grad_loc = grad_loc.to(sampling_loc.dtype)
     if grad_aw.dtype != attn_weight.dtype:
         grad_aw = grad_aw.to(attn_weight.dtype)
-    return [grad_value, grad_loc, grad_aw]
+    return grad_value, grad_loc, grad_aw
+
+
+@_backward_op.register_fake
+def _(grad_output, value, spatial_shapes, level_start_index, sampling_loc, attn_weight, im2col_step, need_grad_value):
+    return (value.new_empty(value.shape if need_grad_value else (0,)), torch.empty_like(sampling_loc),
+            torch.empty_like(attn_weight))
+
+
+def _setup_context(ctx, inputs, output):
+    value, shapes, lsi, loc, aw, im2col_step, _ = inputs
+    ctx.im2col_step = im2col_step
+    ctx.save_for_backward(value, shapes, lsi, loc, aw)
+
+
+def _backward(ctx, grad_output):
+    """once differentiable, like the reference's Function (functions/ms_deform_attn_func.py:30-38)"""
+    value, shapes, lsi, loc, aw = ctx.saved_tensors
+    need_gv, need_loc, need_aw = ctx.needs_input_grad[0], ctx.needs_input_grad[3], ctx.needs_input_grad[4]
+    if not (need_gv or need_loc or need_aw):
+        return None, None, None, None, None, None, None
+    grad_value, grad_loc, grad_aw = _backward_op(grad_output.contiguous(), value, shapes, lsi, loc, aw,
+                                                 ctx.im2col_step, need_gv)
+    return (grad_value if need_gv else None), None, None, grad_loc, grad_aw, None, None
+
+
+_forward_op.register_autograd(_backward, setup_context=_setup_context)
+
+
+def ms_deform_attn_forward(value, spatial_shapes, level_start_index, sampling_loc, attn_weight, im2col_step):
+    """vision.cpp:14 / ms_deform_attn.h:20-39.  Returns (N, Lq, M*D) in value's dtype (op ``devis::ms_deform_attn``)."""
+    return _forward_op(value, spatial_shapes, level_start_index, sampling_loc, attn_weight, int(im2col_step), False)
+
+
+def ms_deform_attn_backward(value, spatial_shapes, level_start_index, sampling_loc, attn_weight, grad_output,
+                            im2col_step, need_grad_value=True):
+    """vision.cpp:15 / ms_deform_attn.h:41-61.  Returns [grad_value, grad_sampling_loc, grad_attn_weight].
+    ``need_grad_value=False`` (extension, used by the autograd formula when value is frozen) skips the scatter and
+    returns None in its place."""
+    grad_value, grad_loc, grad_aw = _backward_op(grad_output, value, spatial_shapes, level_start_index, sampling_loc,
+                                                 attn_weight, int(im2col_step), bool(need_grad_value))
+    return [grad_value if need_grad_value else None, grad_loc, grad_aw]

@@ -53,8 +53,22 @@ class ClipGeometry:
         self.lsi_ptr = self._lsi_np.ctypes.data_as(ctypes.c_void_p)
         self.frames_ptr = self._frames_np.ctypes.data_as(ctypes.c_void_p) if self.t_window else None
         self._orders = {}
+        self._op_args = None
 
     # ------------------------------------------------------------------------------------------
+    def op_args(self):
+        """(spatial_shapes (L,2), level_start_index (L,) as int64 CPU tensors with their host copies attached, the
+        frame offsets as a row-major (T, t_window) list of ints): how the ops (devis::tmsda*) receive this geometry.
+        The op body rebuilds the geometry from them (memoised by value) without a device read."""
+        if self._op_args is None:
+            shapes = attach_host_copy(torch.as_tensor(self._shapes_np), [list(r) for r in self.shapes])
+            lsi = attach_host_copy(torch.as_tensor(self._lsi_np), list(self.level_start_index))
+            offs = [f - t for t, row in enumerate(self.frame_table) for f in row] if self.t_window else []
+            self._op_args = (shapes, lsi, offs)
+            _geom_cache.setdefault((self.n_frames, tuple(tuple(r) for r in self.shapes), tuple(self.level_start_index),
+                                    tuple(tuple(r) for r in self.frame_table) if self.t_window else None), self)
+        return self._op_args
+
     def frame_table_tensor(self, device):
         """(T, t_window) int64 frame indices on `device`, uploaded once (the decoder's instance-aware gather of
         reference points indexes with it every layer; a fresh upload per call would also break CUDA-graph capture)"""
@@ -218,3 +232,20 @@ def batch_geometry(batch, input_spatial_shapes, input_level_start_index):
     shapes = tuple(tuple(int(x) for x in r) for r in _host_list(input_spatial_shapes))
     lsi = tuple(int(x) for x in _host_list(input_level_start_index))
     return _memoised(int(batch), shapes, lsi, None)
+
+
+def op_geometry(n_frames, spatial_shapes, level_start_index, temporal_spatial_shapes, temporal_level_start_index,
+                temporal_offsets, frame_offsets):
+    """The geometry inside the ops: from the current pyramid tensors, the optional temporal halves of the reference's
+    (current, temporal) pairs (validated as in from_reference_args) and the frame offsets -- T per-frame tensors of
+    t_window offsets or one (T, t_window) tensor (`temporal_offsets`), or the same numbers as a row-major list of ints
+    (`frame_offsets`); both empty for a clip without temporal slots (MSDeformAttn's batch)."""
+    if frame_offsets:
+        wt = len(frame_offsets) // n_frames
+        offs = [list(frame_offsets[t * wt:(t + 1) * wt]) for t in range(n_frames)]
+    elif temporal_offsets:
+        offs = temporal_offsets[0] if len(temporal_offsets) == 1 and temporal_offsets[0].dim() == 2 else temporal_offsets
+    else:
+        return batch_geometry(n_frames, spatial_shapes, level_start_index)
+    return from_reference_args(n_frames, (spatial_shapes, temporal_spatial_shapes),
+                               (level_start_index, temporal_level_start_index), offs)

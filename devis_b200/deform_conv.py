@@ -30,13 +30,19 @@ columns.  The lane-group fused kernels serve G > 1 when (Cin / G) % 4 == 0 (devi
 
 Supported: groups == 1, any offset_groups, float32 / float64 (half and bfloat16 are computed in float32 like
 torchvision's autocast wrapper does), CUDA only -- there is no CPU fallback.
+
+Each form is a ``torch.library`` custom op (``devis::deform_conv2d_{im2col,fused,igemm}`` and their ``*_backward``), so
+torch.compile and torch.export trace a layer as one node; the choice of form stays in ``deform_conv2d`` (traceable
+Python: grad mode, requires_grad, allow_tf32, the deterministic flag and the library's shape rules).  A forward op
+returns what its backward needs besides its inputs as extra outputs: the channels-last copy of the input (empty when the
+input is channels-last already, the backward then reads the input itself), the im2col form's columns, the fused form's
+packed weight -- exactly what the backward kept before.
 """
 
 import warnings
+from typing import Optional
 
 import torch
-from torch.autograd import Function
-from torch.autograd.function import once_differentiable
 from torch.nn.modules.utils import _pair
 
 from . import _lib
@@ -127,11 +133,23 @@ def set_fused(enabled):
     return old
 
 
+@torch.compiler.assume_constant_result
+def _library_fused_form(c, cout, kh, kw, offset_groups):
+    """the library's shape rule (a pure function of the ints): a constant to torch.compile, not a graph break"""
+    return int(_lib.load().devis_dcn_fused_form_og(c, cout, kh, kw, offset_groups, _lib.F32))
+
+
 def _fused_form(c, cout, kh, kw, dtype, offset_groups=1):
     """bit 0: fused forward kernel serves the layer, bit 1: fused data-backward kernel does (devis_dcn_fused_form_og)"""
     if not _FUSED or dtype != torch.float32:
         return 0
-    return int(_lib.load().devis_dcn_fused_form_og(c, cout, kh, kw, offset_groups, _lib.F32))
+    return _library_fused_form(int(c), int(cout), int(kh), int(kw), int(offset_groups))
+
+
+@torch.compiler.assume_constant_result
+def _packed_weight_elems(c, cout, kh, kw, offset_groups):
+    """floats of the fused kernels' weight layout for the layer (the library's rule; a constant to torch.compile)"""
+    return int(_lib.load().devis_dcn_packed_weight_elems_og(c, cout, kh, kw, offset_groups))
 
 
 def _offset_groups(offset, kh, kw):
@@ -155,170 +173,326 @@ def _packed_weight(weight, offset_groups=1):
     return packed
 
 
-class FusedDeformConv2dFunction(Function):
-    """apply(input, offset, weight, bias, mask, stride, padding, dilation) -> (N, Cout, Ho, Wo), fused kernels"""
-
-    @staticmethod
-    def forward(ctx, input, offset, weight, bias, mask, stride, padding, dilation):
-        n, c, h, w = input.shape
-        cout, _, kh, kw = weight.shape
-        (sh, sw), (ph, pw), (dh, dw) = stride, padding, dilation
-        ho, wo = _out_size(h, kh, sh, ph, dh), _out_size(w, kw, sw, pw, dw)
-        x = input.permute(0, 2, 3, 1)
-        x = x if x.is_contiguous() else x.contiguous()
-        offset = offset if offset.is_contiguous() else offset.contiguous()
-        if mask is not None:
-            mask = mask if mask.is_contiguous() else mask.contiguous()
-        if bias is not None:
-            bias = bias if bias.is_contiguous() else bias.contiguous()
-        og = _offset_groups(offset, kh, kw)
-        packed = _packed_weight(weight) if og == 1 else _packed_weight(weight, og)   # G = 1: the hook's original signature
-        out = torch.empty((n, ho, wo, cout), dtype=input.dtype, device=input.device)
-        dims = (n, h, w, c, ho, wo, kh, kw, sh, sw, ph, pw, dh, dw)
-        with torch.cuda.device(input.device):
-            _lib.check(_lib.load().devis_dcn_fused_forward_og(_ptr(x), _ptr(offset), _ptr(mask), _ptr(packed), _ptr(bias),
-                                                              _ptr(out), *dims, og, cout,
-                                                              torch.cuda.current_stream().cuda_stream))
-        ctx.dims, ctx.og, ctx.cout, ctx.has_bias = dims, og, cout, bias is not None
-        ctx.form = _fused_form(c, cout, kh, kw, input.dtype, og)
-        ctx.weight = weight.detach() if not ctx.form & 2 else None    # only the GEMM route of the backward reads it
-        ctx.save_for_backward(x, offset, mask, packed)
-        return out.permute(0, 3, 1, 2)
-
-    @staticmethod
-    @once_differentiable
-    def backward(ctx, grad_out):
-        x, offset, mask, packed = ctx.saved_tensors
-        n, h, w, c, ho, wo, kh, kw = ctx.dims[:8]
-        cout, k, og = ctx.cout, kh * kw, ctx.og
-        g = grad_out.permute(0, 2, 3, 1)
-        g = g if g.is_contiguous() else g.contiguous()                    # (N, Ho, Wo, Cout)
-        need_in, need_off, need_w, need_b, need_m = ctx.needs_input_grad[:5]
-        grad_w = grad_b = grad_in = grad_off = grad_m = None
-        lib = _lib.load()
-        stream = torch.cuda.current_stream().cuda_stream
-        with torch.cuda.device(x.device):
-            if need_in or need_off or (need_m and mask is not None):
-                flags = _grad_input_flags(x.dtype) if need_in else 0
-                gx = torch.empty_like(x) if need_in else None
-                grad_off = torch.empty_like(offset)
-                grad_m = torch.empty_like(mask) if mask is not None else None
-                if ctx.form & 2:
-                    per = _data_chunk(n, h, w, c, flags, n)
-                    ws, ws_bytes = _workspace(lib, per, h, w, c, flags, x.device)
-                    for n0 in range(0, n, per):
-                        n1 = min(n, n0 + per)
-                        _lib.check(lib.devis_dcn_fused_backward_og(
-                            _ptr(x[n0:n1]), _ptr(offset[n0:n1]), _ptr(mask[n0:n1]) if mask is not None else None,
-                            _ptr(packed), _ptr(g[n0:n1]), _ptr(gx[n0:n1]) if need_in else None, _ptr(grad_off[n0:n1]),
-                            _ptr(grad_m[n0:n1]) if mask is not None else None, n1 - n0, *ctx.dims[1:], og, cout, flags,
-                            _ptr(ws), ws_bytes, stream))
-                else:
-                    # wider layers: column gradient by GEMM (a bounded chunk of the batch at a time) + scatter kernel
-                    w2 = ctx.weight.permute(0, 2, 3, 1).reshape(cout, k * c)
-                    per = _data_chunk(n, h, w, c, flags, _COLS_CHUNK_BYTES // max(1, ho * wo * k * c * 4))
-                    ws, ws_bytes = _workspace(lib, per, h, w, c, flags, x.device)
-                    g2 = g.view(n * ho * wo, cout)
-                    for n0 in range(0, n, per):
-                        n1 = min(n, n0 + per)
-                        grad_cols = g2[n0 * ho * wo:n1 * ho * wo] @ w2
-                        _lib.check(lib.devis_dcn_col2im_og(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
-                                                           _ptr(mask[n0:n1]) if mask is not None else None, _ptr(grad_cols),
-                                                           _ptr(gx[n0:n1]) if need_in else None, _ptr(grad_off[n0:n1]),
-                                                           _ptr(grad_m[n0:n1]) if mask is not None else None, n1 - n0,
-                                                           *ctx.dims[1:], og, _DTYPES[x.dtype], flags, _ptr(ws), ws_bytes,
-                                                           stream))
-                grad_in = gx.permute(0, 3, 1, 2) if need_in else None
-            if need_w and og == 1 and x.dtype == torch.float32 and not torch.are_deterministic_algorithms_enabled() \
-                    and lib.devis_dcn_wgrad_supported(c, cout, kh, kw, _DTYPES[x.dtype]):
-                # narrow layers: gather + contraction with grad_out in one kernel, no column matrix (dcn_wgrad_kernel,
-                # one offset group only).  Its cross-block float atomics are order-dependent: under
-                # torch.use_deterministic_algorithms the GEMM route below, deterministic like torchvision's, is taken.
-                gw3 = torch.empty((cout, k, c), dtype=x.dtype, device=x.device)
-                _lib.check(lib.devis_dcn_weight_grad(_ptr(x), _ptr(offset), _ptr(mask), _ptr(g), _ptr(gw3), *ctx.dims,
-                                                     cout, stream))
-                grad_w = gw3.view(cout, kh, kw, c).permute(0, 3, 1, 2)
-            elif need_w:
-                # cols^T x grad_out from columns recomputed a bounded chunk of the batch at a time
-                per = max(1, min(n, _COLS_CHUNK_BYTES // max(1, ho * wo * k * c * 4)))
-                cols = torch.empty((per * ho * wo, k * c), dtype=x.dtype, device=x.device)
-                gw2 = torch.zeros((cout, k * c), dtype=x.dtype, device=x.device)
-                g2 = g.view(n * ho * wo, cout)
-                for n0 in range(0, n, per):
-                    n1 = min(n, n0 + per)
-                    rows = (n1 - n0) * ho * wo
-                    _lib.check(lib.devis_dcn_im2col_og(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
-                                                       _ptr(mask[n0:n1]) if mask is not None else None, _ptr(cols),
-                                                       n1 - n0, *ctx.dims[1:], og, _DTYPES[x.dtype], stream))
-                    gw2 += _wgrad(g2[n0 * ho * wo:n1 * ho * wo], cols[:rows])
-                grad_w = gw2.view(cout, kh, kw, c).permute(0, 3, 1, 2)
-        if need_b and ctx.has_bias:
-            grad_b = g.sum((0, 1, 2))
-        return grad_in, grad_off, grad_w, grad_b, grad_m, None, None, None
+OptTensor = Optional[torch.Tensor]
 
 
-class DeformConv2dFunction(Function):
-    """apply(input, offset, weight, bias, mask, stride, padding, dilation) -> (N, Cout, Ho, Wo)"""
+def _nhwc(input):
+    """(input read channels-last, the copy to keep for the backward): an empty tensor when no copy was made (the
+    backward then permutes the input again, which costs nothing)"""
+    x = input.permute(0, 2, 3, 1)
+    if x.is_contiguous():
+        return x, input.new_empty(0)
+    x = x.contiguous()
+    return x, x
 
-    @staticmethod
-    def forward(ctx, input, offset, weight, bias, mask, stride, padding, dilation):
-        n, c, h, w = input.shape
-        cout, _, kh, kw = weight.shape
-        (sh, sw), (ph, pw), (dh, dw) = stride, padding, dilation
-        ho, wo = _out_size(h, kh, sh, ph, dh), _out_size(w, kw, sw, pw, dw)
-        x = input.permute(0, 2, 3, 1)
-        x = x if x.is_contiguous() else x.contiguous()                    # (N, H, W, C)
-        offset = offset if offset.is_contiguous() else offset.contiguous()
-        if mask is not None:
-            mask = mask if mask.is_contiguous() else mask.contiguous()
-        k, og = kh * kw, _offset_groups(offset, kh, kw)
-        cols = torch.empty((n * ho * wo, k * c), dtype=input.dtype, device=input.device)
-        dims = (n, h, w, c, ho, wo, kh, kw, sh, sw, ph, pw, dh, dw)
-        with torch.cuda.device(input.device):
-            _lib.check(_lib.load().devis_dcn_im2col_og(_ptr(x), _ptr(offset), _ptr(mask), _ptr(cols), *dims, og,
-                                                       _DTYPES[input.dtype], torch.cuda.current_stream().cuda_stream))
-        w2 = weight.permute(0, 2, 3, 1).reshape(cout, k * c)              # columns are [k][ci]
-        out = torch.addmm(bias, cols, w2.t()) if bias is not None else cols @ w2.t()
-        ctx.dims, ctx.og = dims, og
-        ctx.has_bias = bias is not None
-        ctx.save_for_backward(x, offset, mask, cols, w2)
-        return out.view(n, ho, wo, cout).permute(0, 3, 1, 2)
 
-    @staticmethod
-    @once_differentiable
-    def backward(ctx, grad_out):
-        x, offset, mask, cols, w2 = ctx.saved_tensors
-        n, h, w, c, ho, wo, kh, kw = ctx.dims[:8]
-        cout = w2.shape[0]
-        g2 = grad_out.permute(0, 2, 3, 1).reshape(n * ho * wo, cout)
-        need_in, need_off, need_w, need_b, need_m = ctx.needs_input_grad[:5]
-        grad_w = grad_b = grad_in = grad_off = grad_m = None
-        if need_w:
-            grad_w = _wgrad(g2, cols).view(cout, kh, kw, c).permute(0, 3, 1, 2)
-        if need_b and ctx.has_bias:
-            grad_b = g2.sum(0)
+def _saved_nhwc(input, x_copy):
+    return x_copy if x_copy.dim() == 4 else input.permute(0, 2, 3, 1)
+
+
+def _contig(t):
+    return t if t is None or t.is_contiguous() else t.contiguous()
+
+
+def _fake_forward(input, offset, weight, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w):
+    """(NCHW view of a channels-last output, the channels-last input copy or an empty tensor) as the forms return them"""
+    n, c, h, w = input.shape
+    cout, _, kh, kw = weight.shape
+    ho, wo = _out_size(h, kh, stride_h, pad_h, dil_h), _out_size(w, kw, stride_w, pad_w, dil_w)
+    out = input.new_empty((n, ho, wo, cout)).permute(0, 3, 1, 2)
+    x_copy = input.new_empty(0) if input.permute(0, 2, 3, 1).is_contiguous() else input.new_empty((n, h, w, c))
+    return out, x_copy
+
+
+def _fake_backward(input, offset, weight, bias, mask, need_in, need_off, need_w, need_b, need_m):
+    """gradients as the backward ops return them: grad_input and grad_weight are NCHW views of channels-last buffers,
+    an empty tensor stands for one that is not computed (the offset and mask gradients come with the data backward)"""
+    n, c, h, w = input.shape
+    cout, _, kh, kw = weight.shape
+    empty = lambda: input.new_empty(0)
+    data = need_in or need_off or (need_m and mask is not None)
+    like = lambda t: torch.empty_like(t, memory_format=torch.contiguous_format)
+    grad_in = input.new_empty((n, h, w, c)).permute(0, 3, 1, 2) if need_in else empty()
+    grad_off = like(offset) if data else empty()
+    grad_w = input.new_empty((cout, kh, kw, c)).permute(0, 3, 1, 2) if need_w else empty()
+    grad_b = input.new_empty((cout,)) if need_b and bias is not None else empty()
+    grad_m = like(mask) if data and mask is not None else empty()
+    return grad_in, grad_off, grad_w, grad_b, grad_m
+
+
+def _needs(ctx):
+    """(need_in, need_off, need_w, need_b, need_m)"""
+    return tuple(ctx.needs_input_grad[:5])
+
+
+def _autograd_result(grads, n_args):
+    """backward-op results -> autograd's: None for the empty placeholders and for the non-tensor arguments"""
+    return tuple(None if g.numel() == 0 and g.dim() == 1 else g for g in grads) + (None,) * n_args
+
+
+# ------------------------------------------------------------------------------------------------------------------------
+# fused form: gather and contraction in one kernel
+# ------------------------------------------------------------------------------------------------------------------------
+@torch.library.custom_op("devis::deform_conv2d_fused", mutates_args=(), tags=(torch.Tag.needs_exact_strides,))
+def _fused_op(input: torch.Tensor, offset: torch.Tensor, weight: torch.Tensor, bias: OptTensor, mask: OptTensor,
+              stride_h: int, stride_w: int, pad_h: int, pad_w: int, dil_h: int, dil_w: int,
+              packed_elems: int) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """(out (N, Cout, Ho, Wo), channels-last input copy or empty, packed weight of ``packed_elems`` floats: the
+    library's size for the layer, _packed_weight_elems)"""
+    if not input.is_cuda:
+        raise RuntimeError("deform_conv2d: not implemented on the CPU (no fallback in this library)")
+    n, c, h, w = input.shape
+    cout, _, kh, kw = weight.shape
+    sh, sw, ph, pw, dh, dw = stride_h, stride_w, pad_h, pad_w, dil_h, dil_w
+    ho, wo = _out_size(h, kh, sh, ph, dh), _out_size(w, kw, sw, pw, dw)
+    x, x_copy = _nhwc(input)
+    offset, mask, bias = _contig(offset), _contig(mask), _contig(bias)
+    og = _offset_groups(offset, kh, kw)
+    packed = _packed_weight(weight) if og == 1 else _packed_weight(weight, og)   # G = 1: the hook's original signature
+    if packed.numel() != packed_elems:
+        raise RuntimeError(f"deform_conv2d: packed weight has {packed.numel()} elements, expected {packed_elems}")
+    out = torch.empty((n, ho, wo, cout), dtype=input.dtype, device=input.device)
+    dims = (n, h, w, c, ho, wo, kh, kw, sh, sw, ph, pw, dh, dw)
+    with torch.cuda.device(input.device):
+        _lib.check(_lib.load().devis_dcn_fused_forward_og(_ptr(x), _ptr(offset), _ptr(mask), _ptr(packed), _ptr(bias),
+                                                          _ptr(out), *dims, og, cout,
+                                                          torch.cuda.current_stream().cuda_stream))
+    return out.permute(0, 3, 1, 2), x_copy, packed
+
+
+@_fused_op.register_fake
+def _(input, offset, weight, bias, mask, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w, packed_elems):
+    out, x_copy = _fake_forward(input, offset, weight, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w)
+    return out, x_copy, input.new_empty((packed_elems,), dtype=torch.float32)
+
+
+@torch.library.custom_op("devis::deform_conv2d_fused_backward", mutates_args=(), tags=(torch.Tag.needs_exact_strides,))
+def _fused_backward_op(grad_out: torch.Tensor, input: torch.Tensor, x_copy: torch.Tensor, offset: torch.Tensor,
+                       weight: torch.Tensor, bias: OptTensor, mask: OptTensor, packed: torch.Tensor, stride_h: int,
+                       stride_w: int, pad_h: int, pad_w: int, dil_h: int, dil_w: int, form: int, need_in: bool,
+                       need_off: bool, need_w: bool, need_b: bool,
+                       need_m: bool) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """(grad_input, grad_offset, grad_weight, grad_bias, grad_mask); ``form``: the forward's _fused_form"""
+    x = _saved_nhwc(input, x_copy)
+    offset, mask = _contig(offset), _contig(mask)
+    n, h, w, c = x.shape
+    cout, _, kh, kw = weight.shape
+    sh, sw, ph, pw, dh, dw = stride_h, stride_w, pad_h, pad_w, dil_h, dil_w
+    ho, wo = _out_size(h, kh, sh, ph, dh), _out_size(w, kw, sw, pw, dw)
+    dims = (n, h, w, c, ho, wo, kh, kw, sh, sw, ph, pw, dh, dw)
+    k, og = kh * kw, _offset_groups(offset, kh, kw)
+    g = grad_out.permute(0, 2, 3, 1)
+    g = g if g.is_contiguous() else g.contiguous()                    # (N, Ho, Wo, Cout)
+    grad_w = grad_b = grad_in = grad_off = grad_m = None
+    lib = _lib.load()
+    stream = torch.cuda.current_stream().cuda_stream
+    with torch.cuda.device(x.device):
         if need_in or need_off or (need_m and mask is not None):
-            grad_cols = g2 @ w2
             flags = _grad_input_flags(x.dtype) if need_in else 0
-            gx = torch.empty_like(x) if need_in else None
+            gx = torch.empty_like(x, memory_format=torch.contiguous_format) if need_in else None
             grad_off = torch.empty_like(offset)
             grad_m = torch.empty_like(mask) if mask is not None else None
-            lib = _lib.load()
-            with torch.cuda.device(x.device):
-                stream = torch.cuda.current_stream().cuda_stream
+            if form & 2:
                 per = _data_chunk(n, h, w, c, flags, n)
                 ws, ws_bytes = _workspace(lib, per, h, w, c, flags, x.device)
                 for n0 in range(0, n, per):
                     n1 = min(n, n0 + per)
+                    _lib.check(lib.devis_dcn_fused_backward_og(
+                        _ptr(x[n0:n1]), _ptr(offset[n0:n1]), _ptr(mask[n0:n1]) if mask is not None else None,
+                        _ptr(packed), _ptr(g[n0:n1]), _ptr(gx[n0:n1]) if need_in else None, _ptr(grad_off[n0:n1]),
+                        _ptr(grad_m[n0:n1]) if mask is not None else None, n1 - n0, *dims[1:], og, cout, flags,
+                        _ptr(ws), ws_bytes, stream))
+            else:
+                # wider layers: column gradient by GEMM (a bounded chunk of the batch at a time) + scatter kernel
+                w2 = weight.detach().permute(0, 2, 3, 1).reshape(cout, k * c)
+                per = _data_chunk(n, h, w, c, flags, _COLS_CHUNK_BYTES // max(1, ho * wo * k * c * 4))
+                ws, ws_bytes = _workspace(lib, per, h, w, c, flags, x.device)
+                g2 = g.view(n * ho * wo, cout)
+                for n0 in range(0, n, per):
+                    n1 = min(n, n0 + per)
+                    grad_cols = g2[n0 * ho * wo:n1 * ho * wo] @ w2
                     _lib.check(lib.devis_dcn_col2im_og(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
-                                                       _ptr(mask[n0:n1]) if mask is not None else None,
-                                                       _ptr(grad_cols[n0 * ho * wo:n1 * ho * wo]),
+                                                       _ptr(mask[n0:n1]) if mask is not None else None, _ptr(grad_cols),
                                                        _ptr(gx[n0:n1]) if need_in else None, _ptr(grad_off[n0:n1]),
                                                        _ptr(grad_m[n0:n1]) if mask is not None else None, n1 - n0,
-                                                       *ctx.dims[1:], ctx.og, _DTYPES[x.dtype], flags, _ptr(ws),
-                                                       ws_bytes, stream))
+                                                       *dims[1:], og, _DTYPES[x.dtype], flags, _ptr(ws), ws_bytes,
+                                                       stream))
             grad_in = gx.permute(0, 3, 1, 2) if need_in else None
-        return grad_in, grad_off, grad_w, grad_b, grad_m, None, None, None
+        if need_w and og == 1 and x.dtype == torch.float32 and not torch.are_deterministic_algorithms_enabled() \
+                and lib.devis_dcn_wgrad_supported(c, cout, kh, kw, _DTYPES[x.dtype]):
+            # narrow layers: gather + contraction with grad_out in one kernel, no column matrix (dcn_wgrad_kernel,
+            # one offset group only).  Its cross-block float atomics are order-dependent: under
+            # torch.use_deterministic_algorithms the GEMM route below, deterministic like torchvision's, is taken.
+            gw3 = torch.empty((cout, k, c), dtype=x.dtype, device=x.device)
+            _lib.check(lib.devis_dcn_weight_grad(_ptr(x), _ptr(offset), _ptr(mask), _ptr(g), _ptr(gw3), *dims,
+                                                 cout, stream))
+            grad_w = gw3.view(cout, kh, kw, c).permute(0, 3, 1, 2)
+        elif need_w:
+            # cols^T x grad_out from columns recomputed a bounded chunk of the batch at a time
+            per = max(1, min(n, _COLS_CHUNK_BYTES // max(1, ho * wo * k * c * 4)))
+            cols = torch.empty((per * ho * wo, k * c), dtype=x.dtype, device=x.device)
+            gw2 = torch.zeros((cout, k * c), dtype=x.dtype, device=x.device)
+            g2 = g.view(n * ho * wo, cout)
+            for n0 in range(0, n, per):
+                n1 = min(n, n0 + per)
+                rows = (n1 - n0) * ho * wo
+                _lib.check(lib.devis_dcn_im2col_og(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
+                                                   _ptr(mask[n0:n1]) if mask is not None else None, _ptr(cols),
+                                                   n1 - n0, *dims[1:], og, _DTYPES[x.dtype], stream))
+                gw2 += _wgrad(g2[n0 * ho * wo:n1 * ho * wo], cols[:rows])
+            grad_w = gw2.view(cout, kh, kw, c).permute(0, 3, 1, 2)
+    if need_b and bias is not None:
+        grad_b = g.sum((0, 1, 2))
+    return tuple(x.new_empty(0) if t is None else t for t in (grad_in, grad_off, grad_w, grad_b, grad_m))
+
+
+@_fused_backward_op.register_fake
+def _(grad_out, input, x_copy, offset, weight, bias, mask, packed, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w,
+      form, need_in, need_off, need_w, need_b, need_m):
+    return _fake_backward(input, offset, weight, bias, mask, need_in, need_off, need_w, need_b, need_m)
+
+
+def _fused_setup_context(ctx, inputs, output):
+    input, offset, weight, bias, mask, *geometry, _ = inputs
+    _, x_copy, packed = output
+    cout, c, kh, kw = weight.shape
+    ctx.geometry = geometry
+    ctx.form = _fused_form(c, cout, kh, kw, input.dtype, _offset_groups(offset, kh, kw))
+    ctx.mark_non_differentiable(x_copy, packed)
+    ctx.save_for_backward(input, x_copy, offset, weight, bias, mask, packed)
+
+
+def _fused_backward(ctx, grad_out, *_unused):
+    input, x_copy, offset, weight, bias, mask, packed = ctx.saved_tensors
+    return _autograd_result(_fused_backward_op(grad_out, input, x_copy, offset, weight, bias, mask, packed,
+                                               *ctx.geometry, ctx.form, *_needs(ctx)), 7)
+
+
+_fused_op.register_autograd(_fused_backward, setup_context=_fused_setup_context)
+
+
+class FusedDeformConv2dFunction:
+    """apply(input, offset, weight, bias, mask, stride, padding, dilation) -> (N, Cout, Ho, Wo), fused kernels
+    (op ``devis::deform_conv2d_fused``, once differentiable)"""
+
+    @staticmethod
+    def apply(input, offset, weight, bias, mask, stride, padding, dilation):
+        cout, c, kh, kw = weight.shape
+        elems = _packed_weight_elems(int(c), int(cout), int(kh), int(kw), int(_offset_groups(offset, kh, kw)))
+        return _fused_op(input, offset, weight, bias, mask, *stride, *padding, *dilation, elems)[0]
+
+
+# ------------------------------------------------------------------------------------------------------------------------
+# im2col form: column matrix + cuBLAS GEMM
+# ------------------------------------------------------------------------------------------------------------------------
+@torch.library.custom_op("devis::deform_conv2d_im2col", mutates_args=(), tags=(torch.Tag.needs_exact_strides,))
+def _im2col_op(input: torch.Tensor, offset: torch.Tensor, weight: torch.Tensor, bias: OptTensor, mask: OptTensor,
+               stride_h: int, stride_w: int, pad_h: int, pad_w: int, dil_h: int,
+               dil_w: int) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """(out (N, Cout, Ho, Wo), channels-last input copy or empty, columns (N*Ho*Wo, K*Cin))"""
+    if not input.is_cuda:
+        raise RuntimeError("deform_conv2d: not implemented on the CPU (no fallback in this library)")
+    n, c, h, w = input.shape
+    cout, _, kh, kw = weight.shape
+    sh, sw, ph, pw, dh, dw = stride_h, stride_w, pad_h, pad_w, dil_h, dil_w
+    ho, wo = _out_size(h, kh, sh, ph, dh), _out_size(w, kw, sw, pw, dw)
+    x, x_copy = _nhwc(input)                                          # (N, H, W, C)
+    offset, mask = _contig(offset), _contig(mask)
+    k, og = kh * kw, _offset_groups(offset, kh, kw)
+    cols = torch.empty((n * ho * wo, k * c), dtype=input.dtype, device=input.device)
+    dims = (n, h, w, c, ho, wo, kh, kw, sh, sw, ph, pw, dh, dw)
+    with torch.cuda.device(input.device):
+        _lib.check(_lib.load().devis_dcn_im2col_og(_ptr(x), _ptr(offset), _ptr(mask), _ptr(cols), *dims, og,
+                                                   _DTYPES[input.dtype], torch.cuda.current_stream().cuda_stream))
+    w2 = weight.permute(0, 2, 3, 1).reshape(cout, k * c)              # columns are [k][ci]
+    out = torch.addmm(bias, cols, w2.t()) if bias is not None else cols @ w2.t()
+    return out.view(n, ho, wo, cout).permute(0, 3, 1, 2), x_copy, cols
+
+
+@_im2col_op.register_fake
+def _(input, offset, weight, bias, mask, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w):
+    out, x_copy = _fake_forward(input, offset, weight, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w)
+    n, _, ho, wo = out.shape
+    cout, c, kh, kw = weight.shape
+    return out, x_copy, input.new_empty((n * ho * wo, kh * kw * c))
+
+
+@torch.library.custom_op("devis::deform_conv2d_im2col_backward", mutates_args=(), tags=(torch.Tag.needs_exact_strides,))
+def _im2col_backward_op(grad_out: torch.Tensor, input: torch.Tensor, x_copy: torch.Tensor, offset: torch.Tensor,
+                        weight: torch.Tensor, bias: OptTensor, mask: OptTensor, cols: torch.Tensor, stride_h: int,
+                        stride_w: int, pad_h: int, pad_w: int, dil_h: int, dil_w: int, need_in: bool, need_off: bool,
+                        need_w: bool, need_b: bool,
+                        need_m: bool) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """(grad_input, grad_offset, grad_weight, grad_bias, grad_mask) from the forward's columns"""
+    x = _saved_nhwc(input, x_copy)
+    offset, mask = _contig(offset), _contig(mask)
+    n, h, w, c = x.shape
+    cout, _, kh, kw = weight.shape
+    sh, sw, ph, pw, dh, dw = stride_h, stride_w, pad_h, pad_w, dil_h, dil_w
+    ho, wo = _out_size(h, kh, sh, ph, dh), _out_size(w, kw, sw, pw, dw)
+    dims = (n, h, w, c, ho, wo, kh, kw, sh, sw, ph, pw, dh, dw)
+    og = _offset_groups(offset, kh, kw)
+    w2 = weight.detach().permute(0, 2, 3, 1).reshape(cout, kh * kw * c)
+    g2 = grad_out.permute(0, 2, 3, 1).reshape(n * ho * wo, cout)
+    grad_w = grad_b = grad_in = grad_off = grad_m = None
+    if need_w:
+        grad_w = _wgrad(g2, cols).view(cout, kh, kw, c).permute(0, 3, 1, 2)
+    if need_b and bias is not None:
+        grad_b = g2.sum(0)
+    if need_in or need_off or (need_m and mask is not None):
+        grad_cols = g2 @ w2
+        flags = _grad_input_flags(x.dtype) if need_in else 0
+        gx = torch.empty_like(x, memory_format=torch.contiguous_format) if need_in else None
+        grad_off = torch.empty_like(offset)
+        grad_m = torch.empty_like(mask) if mask is not None else None
+        lib = _lib.load()
+        with torch.cuda.device(x.device):
+            stream = torch.cuda.current_stream().cuda_stream
+            per = _data_chunk(n, h, w, c, flags, n)
+            ws, ws_bytes = _workspace(lib, per, h, w, c, flags, x.device)
+            for n0 in range(0, n, per):
+                n1 = min(n, n0 + per)
+                _lib.check(lib.devis_dcn_col2im_og(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
+                                                   _ptr(mask[n0:n1]) if mask is not None else None,
+                                                   _ptr(grad_cols[n0 * ho * wo:n1 * ho * wo]),
+                                                   _ptr(gx[n0:n1]) if need_in else None, _ptr(grad_off[n0:n1]),
+                                                   _ptr(grad_m[n0:n1]) if mask is not None else None, n1 - n0,
+                                                   *dims[1:], og, _DTYPES[x.dtype], flags, _ptr(ws),
+                                                   ws_bytes, stream))
+        grad_in = gx.permute(0, 3, 1, 2) if need_in else None
+    return tuple(x.new_empty(0) if t is None else t for t in (grad_in, grad_off, grad_w, grad_b, grad_m))
+
+
+@_im2col_backward_op.register_fake
+def _(grad_out, input, x_copy, offset, weight, bias, mask, cols, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w,
+      need_in, need_off, need_w, need_b, need_m):
+    return _fake_backward(input, offset, weight, bias, mask, need_in, need_off, need_w, need_b, need_m)
+
+
+def _im2col_setup_context(ctx, inputs, output):
+    input, offset, weight, bias, mask, *geometry = inputs
+    _, x_copy, cols = output
+    ctx.geometry = geometry
+    ctx.mark_non_differentiable(x_copy, cols)
+    ctx.save_for_backward(input, x_copy, offset, weight, bias, mask, cols)
+
+
+def _im2col_backward(ctx, grad_out, *_unused):
+    input, x_copy, offset, weight, bias, mask, cols = ctx.saved_tensors
+    return _autograd_result(_im2col_backward_op(grad_out, input, x_copy, offset, weight, bias, mask, cols,
+                                                *ctx.geometry, *_needs(ctx)), 6)
+
+
+_im2col_op.register_autograd(_im2col_backward, setup_context=_im2col_setup_context)
+
+
+class DeformConv2dFunction:
+    """apply(input, offset, weight, bias, mask, stride, padding, dilation) -> (N, Cout, Ho, Wo)
+    (op ``devis::deform_conv2d_im2col``, once differentiable)"""
+
+    @staticmethod
+    def apply(input, offset, weight, bias, mask, stride, padding, dilation):
+        return _im2col_op(input, offset, weight, bias, mask, *stride, *padding, *dilation)[0]
 
 
 _TENSOR_CORE = True
@@ -331,98 +505,145 @@ def set_tensor_core(enabled):
     return old
 
 
-def _igemm_supported(c, cout, kh, kw, dtype):
-    if not _TENSOR_CORE or dtype != torch.float32:
-        return False
+@torch.compiler.assume_constant_result
+def _library_igemm_supported(c, cout, kh, kw):
     return bool(_lib.load().devis_dcn_igemm_supported(c, cout, kh, kw, _lib.F32))
 
 
-class IGemmDeformConv2dFunction(Function):
+def _igemm_supported(c, cout, kh, kw, dtype):
+    if not _TENSOR_CORE or dtype != torch.float32:
+        return False
+    return _library_igemm_supported(int(c), int(cout), int(kh), int(kw))
+
+
+@torch.library.custom_op("devis::deform_conv2d_igemm", mutates_args=(), tags=(torch.Tag.needs_exact_strides,))
+def _igemm_op(input: torch.Tensor, offset: torch.Tensor, weight: torch.Tensor, bias: OptTensor, mask: OptTensor,
+              stride_h: int, stride_w: int, pad_h: int, pad_w: int, dil_h: int,
+              dil_w: int) -> tuple[torch.Tensor, torch.Tensor]:
+    """(out (N, Cout, Ho, Wo), channels-last input copy or empty).  Precision: torch.backends.cuda.matmul.allow_tf32
+    as it is when the op runs"""
+    if not input.is_cuda:
+        raise RuntimeError("deform_conv2d: not implemented on the CPU (no fallback in this library)")
+    n, c, h, w = input.shape
+    cout, _, kh, kw = weight.shape
+    sh, sw, ph, pw, dh, dw = stride_h, stride_w, pad_h, pad_w, dil_h, dil_w
+    ho, wo = _out_size(h, kh, sh, ph, dh), _out_size(w, kw, sw, pw, dw)
+    x, x_copy = _nhwc(input)
+    offset, mask, bias = _contig(offset), _contig(mask), _contig(bias)
+    lib = _lib.load()
+    wd = weight.detach()
+    wd = wd if wd.is_contiguous() else wd.contiguous()
+    packed = torch.empty(int(lib.devis_dcn_igemm_packed_weight_elems(c, cout, kh, kw)), dtype=torch.float32,
+                         device=input.device)
+    out = torch.empty((n, ho, wo, cout), dtype=input.dtype, device=input.device)
+    dims = (n, h, w, c, ho, wo, kh, kw, sh, sw, ph, pw, dh, dw)
+    precision = _lib.DCN_PRECISION_TF32 if torch.backends.cuda.matmul.allow_tf32 else _lib.DCN_PRECISION_3XTF32
+    with torch.cuda.device(input.device):
+        stream = torch.cuda.current_stream().cuda_stream
+        _lib.check(lib.devis_dcn_igemm_pack_weight(_ptr(wd), _ptr(packed), c, cout, kh, kw, stream))
+        _lib.check(lib.devis_dcn_igemm_forward(_ptr(x), _ptr(offset), _ptr(mask), _ptr(packed), _ptr(bias), _ptr(out),
+                                               *dims, cout, precision, stream))
+    return out.permute(0, 3, 1, 2), x_copy
+
+
+@_igemm_op.register_fake
+def _(input, offset, weight, bias, mask, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w):
+    return _fake_forward(input, offset, weight, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w)
+
+
+@torch.library.custom_op("devis::deform_conv2d_igemm_backward", mutates_args=(), tags=(torch.Tag.needs_exact_strides,))
+def _igemm_backward_op(grad_out: torch.Tensor, input: torch.Tensor, x_copy: torch.Tensor, offset: torch.Tensor,
+                       weight: torch.Tensor, bias: OptTensor, mask: OptTensor, stride_h: int, stride_w: int, pad_h: int,
+                       pad_w: int, dil_h: int, dil_w: int, need_in: bool, need_off: bool, need_w: bool, need_b: bool,
+                       need_m: bool) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """(grad_input, grad_offset, grad_weight, grad_bias, grad_mask): the im2col form's backward with the columns
+    recomputed in bounded chunks"""
+    x = _saved_nhwc(input, x_copy)
+    offset, mask = _contig(offset), _contig(mask)
+    n, h, w, c = x.shape
+    cout, _, kh, kw = weight.shape
+    sh, sw, ph, pw, dh, dw = stride_h, stride_w, pad_h, pad_w, dil_h, dil_w
+    ho, wo = _out_size(h, kh, sh, ph, dh), _out_size(w, kw, sw, pw, dw)
+    dims = (n, h, w, c, ho, wo, kh, kw, sh, sw, ph, pw, dh, dw)
+    k = kh * kw
+    weight = weight.detach()
+    weight = weight if weight.is_contiguous() else weight.contiguous()
+    g2 = grad_out.permute(0, 2, 3, 1).reshape(n * ho * wo, cout)
+    g2 = g2 if g2.is_contiguous() else g2.contiguous()
+    w2 = weight.permute(0, 2, 3, 1).reshape(cout, k * c)
+    grad_w = grad_b = grad_in = grad_off = grad_m = None
+    lib = _lib.load()
+    with torch.cuda.device(x.device):
+        stream = torch.cuda.current_stream().cuda_stream
+        if need_w:
+            per = max(1, min(n, _COLS_CHUNK_BYTES // max(1, ho * wo * k * c * 4)))
+            cols = torch.empty((per * ho * wo, k * c), dtype=x.dtype, device=x.device)
+            gw2 = torch.zeros((cout, k * c), dtype=x.dtype, device=x.device)
+            for n0 in range(0, n, per):
+                n1 = min(n, n0 + per)
+                rows = (n1 - n0) * ho * wo
+                _lib.check(lib.devis_dcn_im2col(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
+                                                _ptr(mask[n0:n1]) if mask is not None else None, _ptr(cols),
+                                                n1 - n0, *dims[1:], _DTYPES[x.dtype], stream))
+                gw2 += _wgrad(g2[n0 * ho * wo:n1 * ho * wo], cols[:rows])
+            del cols
+            grad_w = gw2.view(cout, kh, kw, c).permute(0, 3, 1, 2)
+        if need_b and bias is not None:
+            grad_b = g2.sum(0)
+        if need_in or need_off or (need_m and mask is not None):
+            flags = _grad_input_flags(x.dtype) if need_in else 0
+            gx = torch.empty_like(x, memory_format=torch.contiguous_format) if need_in else None
+            grad_off = torch.empty_like(offset)
+            grad_m = torch.empty_like(mask) if mask is not None else None
+            per = _data_chunk(n, h, w, c, flags, _COLS_CHUNK_BYTES // max(1, ho * wo * k * c * 4))
+            ws, ws_bytes = _workspace(lib, per, h, w, c, flags, x.device)
+            for n0 in range(0, n, per):
+                n1 = min(n, n0 + per)
+                grad_cols = g2[n0 * ho * wo:n1 * ho * wo] @ w2
+                _lib.check(lib.devis_dcn_col2im_ex(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
+                                                   _ptr(mask[n0:n1]) if mask is not None else None, _ptr(grad_cols),
+                                                   _ptr(gx[n0:n1]) if need_in else None, _ptr(grad_off[n0:n1]),
+                                                   _ptr(grad_m[n0:n1]) if mask is not None else None, n1 - n0,
+                                                   *dims[1:], _DTYPES[x.dtype], flags, _ptr(ws), ws_bytes,
+                                                   stream))
+            grad_in = gx.permute(0, 3, 1, 2) if need_in else None
+    return tuple(x.new_empty(0) if t is None else t for t in (grad_in, grad_off, grad_w, grad_b, grad_m))
+
+
+@_igemm_backward_op.register_fake
+def _(grad_out, input, x_copy, offset, weight, bias, mask, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w, need_in,
+      need_off, need_w, need_b, need_m):
+    return _fake_backward(input, offset, weight, bias, mask, need_in, need_off, need_w, need_b, need_m)
+
+
+def _igemm_setup_context(ctx, inputs, output):
+    input, offset, weight, bias, mask, *geometry = inputs
+    ctx.geometry = geometry
+    ctx.mark_non_differentiable(output[1])
+    ctx.save_for_backward(input, output[1], offset, weight, bias, mask)
+
+
+def _igemm_backward(ctx, grad_out, *_unused):
+    input, x_copy, offset, weight, bias, mask = ctx.saved_tensors
+    return _autograd_result(_igemm_backward_op(grad_out, input, x_copy, offset, weight, bias, mask, *ctx.geometry,
+                                               *_needs(ctx)), 6)
+
+
+_igemm_op.register_autograd(_igemm_backward, setup_context=_igemm_setup_context)
+
+
+class IGemmDeformConv2dFunction:
     """apply(input, offset, weight, bias, mask, stride, padding, dilation) -> (N, Cout, Ho, Wo)
 
     Forward of the wide mask-head layers as an implicit GEMM on the tensor cores (devis_dcn_igemm_forward, tcgen05 /
     TMEM): no column matrix is written or kept.  One offset group only.  Precision follows ``torch.backends.cuda.matmul.allow_tf32`` exactly as
     torchvision's ``addmm`` would: off (the default) -> 3xTF32, fp32-grade; on -> one TF32 pass.  The backward is the
     im2col form's (cuBLAS GEMMs + devis_dcn_col2im), with the columns RECOMPUTED for the weight gradient, so nothing of
-    column size lives between forward and backward."""
+    column size lives between forward and backward.  Op ``devis::deform_conv2d_igemm``, once differentiable."""
 
     @staticmethod
-    def forward(ctx, input, offset, weight, bias, mask, stride, padding, dilation):
-        n, c, h, w = input.shape
-        cout, _, kh, kw = weight.shape
-        (sh, sw), (ph, pw), (dh, dw) = stride, padding, dilation
-        ho, wo = _out_size(h, kh, sh, ph, dh), _out_size(w, kw, sw, pw, dw)
-        x = input.permute(0, 2, 3, 1)
-        x = x if x.is_contiguous() else x.contiguous()
-        offset = offset if offset.is_contiguous() else offset.contiguous()
-        if mask is not None:
-            mask = mask if mask.is_contiguous() else mask.contiguous()
-        if bias is not None:
-            bias = bias if bias.is_contiguous() else bias.contiguous()
-        lib = _lib.load()
-        wd = weight.detach()
-        wd = wd if wd.is_contiguous() else wd.contiguous()
-        packed = torch.empty(int(lib.devis_dcn_igemm_packed_weight_elems(c, cout, kh, kw)), dtype=torch.float32,
-                             device=input.device)
-        out = torch.empty((n, ho, wo, cout), dtype=input.dtype, device=input.device)
-        dims = (n, h, w, c, ho, wo, kh, kw, sh, sw, ph, pw, dh, dw)
-        precision = _lib.DCN_PRECISION_TF32 if torch.backends.cuda.matmul.allow_tf32 else _lib.DCN_PRECISION_3XTF32
-        with torch.cuda.device(input.device):
-            stream = torch.cuda.current_stream().cuda_stream
-            _lib.check(lib.devis_dcn_igemm_pack_weight(_ptr(wd), _ptr(packed), c, cout, kh, kw, stream))
-            _lib.check(lib.devis_dcn_igemm_forward(_ptr(x), _ptr(offset), _ptr(mask), _ptr(packed), _ptr(bias), _ptr(out),
-                                                   *dims, cout, precision, stream))
-        ctx.dims, ctx.has_bias = dims, bias is not None
-        ctx.save_for_backward(x, offset, mask, wd)
-        return out.permute(0, 3, 1, 2)
-
-    @staticmethod
-    @once_differentiable
-    def backward(ctx, grad_out):
-        x, offset, mask, weight = ctx.saved_tensors
-        n, h, w, c, ho, wo, kh, kw = ctx.dims[:8]
-        cout, k = weight.shape[0], kh * kw
-        g2 = grad_out.permute(0, 2, 3, 1).reshape(n * ho * wo, cout)
-        g2 = g2 if g2.is_contiguous() else g2.contiguous()
-        w2 = weight.permute(0, 2, 3, 1).reshape(cout, k * c)
-        need_in, need_off, need_w, need_b, need_m = ctx.needs_input_grad[:5]
-        grad_w = grad_b = grad_in = grad_off = grad_m = None
-        lib = _lib.load()
-        with torch.cuda.device(x.device):
-            stream = torch.cuda.current_stream().cuda_stream
-            if need_w:
-                per = max(1, min(n, _COLS_CHUNK_BYTES // max(1, ho * wo * k * c * 4)))
-                cols = torch.empty((per * ho * wo, k * c), dtype=x.dtype, device=x.device)
-                gw2 = torch.zeros((cout, k * c), dtype=x.dtype, device=x.device)
-                for n0 in range(0, n, per):
-                    n1 = min(n, n0 + per)
-                    rows = (n1 - n0) * ho * wo
-                    _lib.check(lib.devis_dcn_im2col(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
-                                                    _ptr(mask[n0:n1]) if mask is not None else None, _ptr(cols),
-                                                    n1 - n0, *ctx.dims[1:], _DTYPES[x.dtype], stream))
-                    gw2 += _wgrad(g2[n0 * ho * wo:n1 * ho * wo], cols[:rows])
-                del cols
-                grad_w = gw2.view(cout, kh, kw, c).permute(0, 3, 1, 2)
-            if need_b and ctx.has_bias:
-                grad_b = g2.sum(0)
-            if need_in or need_off or (need_m and mask is not None):
-                flags = _grad_input_flags(x.dtype) if need_in else 0
-                gx = torch.empty_like(x) if need_in else None
-                grad_off = torch.empty_like(offset)
-                grad_m = torch.empty_like(mask) if mask is not None else None
-                per = _data_chunk(n, h, w, c, flags, _COLS_CHUNK_BYTES // max(1, ho * wo * k * c * 4))
-                ws, ws_bytes = _workspace(lib, per, h, w, c, flags, x.device)
-                for n0 in range(0, n, per):
-                    n1 = min(n, n0 + per)
-                    grad_cols = g2[n0 * ho * wo:n1 * ho * wo] @ w2
-                    _lib.check(lib.devis_dcn_col2im_ex(_ptr(x[n0:n1]), _ptr(offset[n0:n1]),
-                                                       _ptr(mask[n0:n1]) if mask is not None else None, _ptr(grad_cols),
-                                                       _ptr(gx[n0:n1]) if need_in else None, _ptr(grad_off[n0:n1]),
-                                                       _ptr(grad_m[n0:n1]) if mask is not None else None, n1 - n0,
-                                                       *ctx.dims[1:], _DTYPES[x.dtype], flags, _ptr(ws), ws_bytes,
-                                                       stream))
-                grad_in = gx.permute(0, 3, 1, 2) if need_in else None
-        return grad_in, grad_off, grad_w, grad_b, grad_m, None, None, None
+    def apply(input, offset, weight, bias, mask, stride, padding, dilation):
+        return _igemm_op(input, offset, weight, bias, mask, *stride, *padding, *dilation)[0]
 
 
 def deform_conv2d(input, offset, weight, bias=None, stride=(1, 1), padding=(0, 0), dilation=(1, 1), mask=None):
@@ -461,7 +682,9 @@ def deform_conv2d(input, offset, weight, bias=None, stride=(1, 1), padding=(0, 0
     same = lambda t: None if t is None else (t if t.dtype == input.dtype else t.to(input.dtype))
     # fused forward when the layer is served; when gradients are needed only if its data backward is fused as well
     # (otherwise the im2col form, which keeps its columns for the backward, is the faster training path)
-    form = _fused_form(c, cout, kh, kw, input.dtype, og) if n > 0 else 0
+    # (the layer's channel counts are read from the weight: a parameter, static for torch.compile even when the input
+    # shapes are dynamic; c == cin_g was checked above)
+    form = _fused_form(cin_g, cout, kh, kw, input.dtype, og) if n > 0 else 0
     needs_grad = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (input, offset, weight, bias, mask))
     fn = FusedDeformConv2dFunction if form & 1 and (form & 2 or not needs_grad) else DeformConv2dFunction
     # Forward on the tensor cores (tcgen05 implicit GEMM) for the layers with enough contraction to pay for it: everything
@@ -470,8 +693,8 @@ def deform_conv2d(input, offset, weight, bias=None, stride=(1, 1), padding=(0, 0
     # 16 -> 4 623 against 246 us stay where they are).  With gradients the 72 -> 32 layer keeps the im2col form: its backward
     # reuses the forward's columns, which is 270 us faster there than recomputing them (at 560 MB of columns for 60 instances).
     # The tensor-core forward serves one offset group only.
-    if og == 1 and n > 0 and _igemm_supported(c, cout, kh, kw, input.dtype) and \
-            (not form & 1 or (c * kh * kw >= 576 and cout >= 32 and not form & 2 and not needs_grad)):
+    if og == 1 and n > 0 and _igemm_supported(cin_g, cout, kh, kw, input.dtype) and \
+            (not form & 1 or (cin_g * kh * kw >= 576 and cout >= 32 and not form & 2 and not needs_grad)):
         fn = IGemmDeformConv2dFunction
     out = fn.apply(input, same(offset), same(weight), same(bias), same(mask), stride, padding, dilation)
     return out if out.dtype == out_dtype else out.to(out_dtype)

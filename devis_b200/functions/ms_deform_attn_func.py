@@ -7,28 +7,15 @@ grad_attn_weight, None)``.  The arithmetic runs in the sm_100a kernels behind th
 (The reference file also holds ``ms_deform_attn_core_pytorch``; that is the oracle and lives in
 oracle/msda_torch.py -- the product package has no PyTorch implementation of the op.)
 """
-from torch.autograd import Function
-from torch.autograd.function import once_differentiable
-
 from .. import MultiScaleDeformableAttention as MSDA
 
 
-class MSDeformAttnFunction(Function):
-    @staticmethod
-    def forward(ctx, value, value_spatial_shapes, value_level_start_index, sampling_locations,
-                attention_weights, im2col_step):
-        ctx.im2col_step = im2col_step
-        output = MSDA.ms_deform_attn_forward(value, value_spatial_shapes, value_level_start_index,
-                                             sampling_locations, attention_weights, im2col_step)
-        ctx.save_for_backward(value, value_spatial_shapes, value_level_start_index, sampling_locations,
-                              attention_weights)
-        return output
+class MSDeformAttnFunction:
+    """Entry point of the op ``devis::ms_deform_attn`` (MultiScaleDeformableAttention._forward_op), whose registered
+    autograd formula is this contract; torch.compile and torch.export trace it as one node."""
 
     @staticmethod
-    @once_differentiable
-    def backward(ctx, grad_output):
-        value, shapes, lsi, loc, aw = ctx.saved_tensors
-        grad_value, grad_loc, grad_aw = MSDA.ms_deform_attn_backward(
-            value, shapes, lsi, loc, aw, grad_output.contiguous(), ctx.im2col_step,
-            need_grad_value=ctx.needs_input_grad[0])
-        return grad_value, None, None, grad_loc, grad_aw, None
+    def apply(value, value_spatial_shapes, value_level_start_index, sampling_locations, attention_weights,
+              im2col_step):
+        return MSDA._forward_op(value, value_spatial_shapes, value_level_start_index, sampling_locations,
+                                attention_weights, int(im2col_step), False)

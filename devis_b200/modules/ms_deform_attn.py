@@ -13,6 +13,10 @@ over the T frames in Python and issues two op calls and one gather copy of ``val
 the whole clip is one ``TemporalMSDeformAttnFunction`` call that reads ``value`` in place, and with
 ``fuse_prologue`` (default, encoder and decoder) the kernels also take over the joint softmax and the location
 arithmetic (``TemporalMSDeformAttnFusedFunction``), reading the Linear outputs directly.
+
+The modules call the custom ops (torch.ops.devis.*) with the pyramid tensors and the frame offsets themselves; the op
+bodies read their host copies and validate them.  What is left here is traceable Python -- shapes, flags, the choice
+of the fused path -- so torch.compile(fullgraph=True) and torch.export trace these modules without a graph break.
 """
 import math
 import warnings
@@ -22,8 +26,10 @@ import torch.nn.functional as F
 from torch import nn
 from torch.nn.init import constant_, xavier_uniform_
 
-from .. import _lib, clip_geometry
-from ..functions import MSDeformAttnFunction, TemporalMSDeformAttnFusedFunction, temporal_ms_deform_attn
+from .. import MultiScaleDeformableAttention as MSDA
+from .. import _lib
+from ..functions import TemporalMSDeformAttnFusedFunction
+from ..functions import temporal_func
 
 
 def _is_power_of_2(n):
@@ -49,6 +55,53 @@ def _ray_bias(n_heads, n_slots, n_points):
 def _wh(spatial_shapes, dtype):
     """(L,2) offset normaliser in (W, H) order (ms_deform_attn.py:113-114)."""
     return torch.stack([spatial_shapes[..., 1], spatial_shapes[..., 0]], -1).to(dtype)
+
+
+def _pair_halves(arg):
+    """the reference's (current, temporal) pair of shape / start-index tensors -> (current, temporal or None)"""
+    if isinstance(arg, (tuple, list)):
+        return arg[0], (arg[1] if len(arg) > 1 else None)
+    return arg, None
+
+
+def _offset_args(temporal_offsets):
+    """the per-frame temporal offsets as the ops take them: (tensors, ints) -- T tensors (the reference's form, passed
+    through so that their memoised host copy is reused) or one (T, t_window) tensor; python lists (what the trunk
+    passes) as a row-major list of ints, which a compiled graph keeps as constants"""
+    if isinstance(temporal_offsets, torch.Tensor):
+        return [temporal_offsets], []
+    if all(isinstance(o, torch.Tensor) for o in temporal_offsets):
+        return list(temporal_offsets), []
+    return [], [int(o) for row in temporal_offsets for o in row]
+
+
+_FRAME_INDEX = {}
+
+
+def _frame_index(temporal_offsets, n_frames, device):
+    """(T, t_window) int64 frame indices on `device` from the per-frame offsets, by tensor ops (no host read)"""
+    tensors, ints = _offset_args(temporal_offsets)
+    if ints:
+        wt = len(ints) // n_frames
+        rows = tuple(tuple(t + o for o in ints[t * wt:(t + 1) * wt]) for t in range(n_frames))
+        if torch.compiler.is_compiling():         # a constant of the graph
+            return torch.tensor(rows, dtype=torch.long, device=device)
+        # eager: uploaded once per table and device (a fresh upload per call would also break CUDA-graph capture)
+        key = (rows, str(device))
+        if key not in _FRAME_INDEX:
+            if len(_FRAME_INDEX) > 64:
+                _FRAME_INDEX.clear()
+            _FRAME_INDEX[key] = torch.tensor(rows, dtype=torch.long, device=device)
+        return _FRAME_INDEX[key]
+    if len(tensors) == 1 and tensors[0].dim() == 2:
+        table = tensors[0]
+    else:
+        table = torch.stack([o.reshape(-1) for o in tensors])
+    return table.to(device=device, dtype=torch.long) + torch.arange(n_frames, device=device)[:, None]
+
+
+def _tile(query_tile):
+    return tuple(query_tile) if query_tile else (0, 0)
 
 
 def _check_head_dim(d_model, n_heads):
@@ -107,7 +160,6 @@ class MSDeformAttn(nn.Module):
         if self._fused_path(heads, reference_points):
             return self._forward_fused(query, reference_points, heads, input_spatial_shapes, input_level_start_index,
                                        input_padding_mask)
-        assert (input_spatial_shapes[:, 0] * input_spatial_shapes[:, 1]).sum() == s
 
         if input_padding_mask is not None:
             value = value.masked_fill(input_padding_mask[..., None], float(0))
@@ -123,31 +175,27 @@ class MSDeformAttn(nn.Module):
         else:
             raise ValueError("Last dim of reference_points must be 2 or 4, but get {} instead.".format(
                 reference_points.shape[-1]))
-        out = MSDeformAttnFunction.apply(value, input_spatial_shapes, input_level_start_index, loc, weights,
-                                         self.im2col_step)
+        # (the op asserts sum(H*W) == S on the pyramid's host copy)
+        out = MSDA._forward_op(value, input_spatial_shapes, input_level_start_index, loc, weights, self.im2col_step,
+                               True)
         return self.output_proj(out), None
 
     def _forward_fused(self, query, reference_points, value, input_spatial_shapes, input_level_start_index,
                        input_padding_mask):
         """One launch each way for the attention: the N images are the frames of a clip without temporal slots, the
         softmax, `ref + off / (W, H)` (points, encoder form) or the box form (GEN) and the padding mask are evaluated in
-        the kernels.  Host values of the pyramid come from memoised reads: no device read-back the unfused path does
-        not make."""
+        the kernels.  Host values of the pyramid come from memoised reads inside the op: no device read-back the unfused
+        path does not make."""
         n, lq, _ = query.shape
-        s = value.shape[1]
         m, nl, p = self.n_heads, self.n_levels, self.n_points
-        geom = clip_geometry.batch_geometry(n, input_spatial_shapes, input_level_start_index)
-        assert sum(h * w for h, w in geom.shapes) == s
         step = min(n, self.im2col_step)
         if n % step != 0:
             raise RuntimeError(f"batch({n}) must divide im2col_step({step})")
-        order = None
-        if self.query_tile and lq == s:
-            order = geom.tile_order(query.device, *self.query_tile)
-        out = TemporalMSDeformAttnFusedFunction.apply(
+        out = temporal_func._fused_op(
             value, reference_points, self.sampling_offsets(query).view(n, lq, m, nl, p, 2),
-            self.attention_weights(query).view(n, lq, m, nl * p), None, None, geom, order, _lib.TREF_LEVEL0, False,
-            input_padding_mask)
+            self.attention_weights(query).view(n, lq, m, nl * p), None, None, input_spatial_shapes,
+            input_level_start_index, None, None, [], [], None, *_tile(self.query_tile), _lib.TREF_LEVEL0, False,
+            input_padding_mask, True)[0]
         return self.output_proj(out), None
 
 
@@ -206,10 +254,6 @@ class TemporalMSDeformAttnBase(nn.Module):
         aw_t = joint[..., nl * pc:].reshape(t, lq, m, wt * nl, pt)
         return value, off_c, off_t, aw_c, aw_t
 
-    def _geometry(self, n_frames, input_spatial_shapes, input_level_start_index, temporal_offsets):
-        return clip_geometry.from_reference_args(n_frames, input_spatial_shapes, input_level_start_index,
-                                                 temporal_offsets)
-
     def forward(self, query, reference_points, input_flatten, input_spatial_shapes, input_level_start_index,
                 temporal_offsets):
         raise NotImplementedError
@@ -221,25 +265,24 @@ class TemporalMSDeformAttnEncoder(TemporalMSDeformAttnBase):
         """query (T,S,C); reference_points (T,S,L,2); input_flatten (T,S,C); input_spatial_shapes /
         input_level_start_index: (current, temporal) pairs; temporal_offsets: T tensors of t_window frame
         offsets.  Returns (out (T,S,C), None) -- ms_deform_attn.py:419-464."""
-        cur_shapes = input_spatial_shapes[0]
-        n_frames = input_flatten.shape[0]
+        cur_shapes, t_shapes = _pair_halves(input_spatial_shapes)
+        cur_lsi, t_lsi = _pair_halves(input_level_start_index)
+        offs, ints = _offset_args(temporal_offsets)
         assert reference_points.shape[-1] == 2
-        geom = self._geometry(n_frames, input_spatial_shapes, input_level_start_index, temporal_offsets)
-        order = None
-        if self.query_tile and query.shape[1] == geom.spatial_size:
-            order = geom.tile_order(query.device, *self.query_tile)
+        tile = _tile(self.query_tile)
 
         t, lq, _ = query.shape
         m, nl, wt, pc, pt = self.n_heads, self.n_levels, self.t_window, self.n_curr_points, self.n_temporal_points
         value = self.value_proj(input_flatten).view(t, input_flatten.shape[1], m, self.d_model // m)
         # decided on the PROJECTED value (under autocast it is half precision while input_flatten is not)
         if self.fuse_prologue and TemporalMSDeformAttnFusedFunction.supported(value, reference_points, pc, pt):
-            out = TemporalMSDeformAttnFusedFunction.apply(
+            out = temporal_func._fused_op(
                 value, reference_points,
                 self.sampling_offsets(query).view(t, lq, m, nl, pc, 2),
                 self.attention_weights(query).view(t, lq, m, nl * pc),
                 self.temporal_sampling_offsets(query).view(t, lq, m, wt * nl, pt, 2),
-                self.temporal_attention_weights(query).view(t, lq, m, wt * nl * pt), geom, order)
+                self.temporal_attention_weights(query).view(t, lq, m, wt * nl * pt), cur_shapes, cur_lsi, t_shapes,
+                t_lsi, offs, ints, None, *tile, _lib.TREF_LEVEL0, False, None, False)[0]
             return self.output_proj(out), None
 
         _, off_c, off_t, aw_c, aw_t = self._compute_deformable_attention(query, None)
@@ -250,7 +293,8 @@ class TemporalMSDeformAttnEncoder(TemporalMSDeformAttnBase):
         loc_t = reference_points[:, :, 0][:, :, None, None, None, :] \
             + off_t / wh.repeat(self.t_window, 1)[None, None, None, :, None, :]
 
-        out = temporal_ms_deform_attn(value, loc_c, aw_c, loc_t, aw_t, geom, order)
+        out = temporal_func._tmsda_op(value, loc_c, aw_c, loc_t, aw_t, cur_shapes, cur_lsi, t_shapes, t_lsi, offs, ints, None,
+                                      *tile)
         return self.output_proj(out), None
 
 
@@ -266,13 +310,14 @@ class TemporalMSDeformAttnDecoder(TemporalMSDeformAttnBase):
         """query (1,T*q,C); reference_points (1,T*q,L,2|4) or (T,q,L,2|4); input_flatten (T,S,C).  Returns the
         reference's 5-tuple (ms_deform_attn.py:414): out (1,T*q,C), T current location tensors
         (1,q,M,L,Pc,2), T temporal location tensors (1,q,M,Wt*L,Pt,2), current and temporal weights."""
-        cur_shapes = input_spatial_shapes[0]
+        cur_shapes, t_shapes = _pair_halves(input_spatial_shapes)
+        cur_lsi, t_lsi = _pair_halves(input_level_start_index)
+        offs, ints = _offset_args(temporal_offsets)
         n_frames = input_flatten.shape[0]
         q = query.shape[1] // n_frames
         query = query.reshape(n_frames, q, query.shape[-1])
         if reference_points.shape[0] != n_frames:
             reference_points = reference_points.reshape((n_frames, q) + tuple(reference_points.shape[-2:]))
-        geom = self._geometry(n_frames, input_spatial_shapes, input_level_start_index, temporal_offsets)
         m, nl, wt, pc, pt = self.n_heads, self.n_levels, self.t_window, self.n_curr_points, self.n_temporal_points
         value = self.value_proj(input_flatten).view(n_frames, input_flatten.shape[1], m, self.d_model // m)
         if reference_points.shape[-1] not in (2, 4):
@@ -282,13 +327,14 @@ class TemporalMSDeformAttnDecoder(TemporalMSDeformAttnBase):
         if self.fuse_prologue and TemporalMSDeformAttnFusedFunction.supported(value, reference_points, pc, pt):
             # one launch each way: softmax, `ref + off / (W, H)` or the box form, the instance-aware reference lookup and
             # the 5-tuple's locations / weights (by-products, not differentiable) all happen in the kernels
-            out, loc_c, aw_c, loc_t, aw_t = TemporalMSDeformAttnFusedFunction.apply(
+            out, loc_c, aw_c, loc_t, aw_t = temporal_func._fused_op(
                 value, reference_points,
                 self.sampling_offsets(query).view(n_frames, q, m, nl, pc, 2),
                 self.attention_weights(query).view(n_frames, q, m, nl * pc),
                 self.temporal_sampling_offsets(query).view(n_frames, q, m, wt * nl, pt, 2),
-                self.temporal_attention_weights(query).view(n_frames, q, m, wt * nl * pt), geom, None,
-                _lib.TREF_SAMPLED if self.dec_instance_aware_att else _lib.TREF_OWN, True)
+                self.temporal_attention_weights(query).view(n_frames, q, m, wt * nl * pt), cur_shapes, cur_lsi,
+                t_shapes, t_lsi, offs, ints, None, 0, 0, _lib.TREF_SAMPLED if self.dec_instance_aware_att else _lib.TREF_OWN,
+                True, None, False)
             out = self.output_proj(out.flatten(0, 1)[None])
             return (out, [loc_c[t][None] for t in range(n_frames)], [loc_t[t][None] for t in range(n_frames)],
                     aw_c, aw_t)
@@ -298,7 +344,7 @@ class TemporalMSDeformAttnDecoder(TemporalMSDeformAttnBase):
         # reference point each temporal (slot, level) starts from: the same query's own reference in the
         # sampled frame when instance-aware (:342-344), else its frame-t reference repeated (:346-347)
         if self.dec_instance_aware_att:
-            table = geom.frame_table_tensor(query.device)                                      # (T, Wt)
+            table = _frame_index(temporal_offsets, n_frames, query.device)                     # (T, Wt)
             ref_t = reference_points[table].permute(0, 2, 1, 3, 4).flatten(2, 3)                 # (T,q,Wt*L,.)
         else:
             ref_t = reference_points.repeat(1, 1, self.t_window, 1)
@@ -312,7 +358,8 @@ class TemporalMSDeformAttnDecoder(TemporalMSDeformAttnBase):
                 + (off_c / self.n_curr_points) * reference_points[:, :, None, :, None, 2:] * 0.5
             loc_t = ref_t[:, :, None, :, None, :2] + (off_t / self.n_temporal_points) * ref_t[:, :, None, :, None, 2:] * 0.5
 
-        out = temporal_ms_deform_attn(value, loc_c, aw_c, loc_t, aw_t, geom, None)
+        out = temporal_func._tmsda_op(value, loc_c, aw_c, loc_t, aw_t, cur_shapes, cur_lsi, t_shapes, t_lsi, offs, ints, None,
+                                      0, 0)
         out = self.output_proj(out.flatten(0, 1)[None])
         return (out, [loc_c[t][None] for t in range(n_frames)], [loc_t[t][None] for t in range(n_frames)],
                 aw_c, aw_t)
